@@ -3,6 +3,7 @@
 on the complex scene, 1920x1080, 64 spp (BASELINE.json configs[2]) at N = 1/2/4/8 B200, tile-sharded.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # own arm (CUDA)
+    python bench.py ... --dump-outputs DIR                         # + the last timed step's frame and counters as .npy
     python bench.py --impl reference [...]                         # the CPU port of the reference (oracle/, OpenMP)
     torchrun --nproc-per-node N ... bench.py --gpus N ...          # N > 1, one rank per GPU over NCCL
 
@@ -65,6 +66,16 @@ def ncu_dram_bytes():
 def flop_per_query(n_spheres, n_lights):
     """SURVEY.md 8d: 20 FLOP per ray-sphere test x N, + hit point/normal 15 + 25 per light + bounce/TBN/fold 70."""
     return 20 * n_spheres + 15 + 25 * n_lights + 70
+
+
+def dump_outputs(out_dir, image, stats):
+    """--dump-outputs: the frame and counters one timed step returned to its caller, whole (25 MB), so that two builds
+    can be compared output for output.  Step i renders with seed i, so equal arguments give equal inputs.
+      image.npy  float32 [H, W, 3], the resolved frame
+      stats.npy  float64 [8], the path kernel's uint64 counter block (exact: every count is far below 2**53)"""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "image.npy"), image.detach().cpu().numpy().astype(np.float32, copy=False))
+    np.save(os.path.join(out_dir, "stats.npy"), stats.detach().cpu().numpy().astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -354,8 +365,14 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the per-shape table and the sustained run")
     ap.add_argument("--flush-mib", type=int, default=256, help="size of the L2 flush between timed steps (diagnostic; 0 = none)")
     ap.add_argument("--debug-ranks", action="store_true", help="every rank prints its own per-step times to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's frame and counters to DIR/image.npy and DIR/stats.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the CUDA arm only")
         return run_reference_arm(args)
     args.warmup = max(args.warmup, 3)
     if args.mode == "auto":
@@ -416,7 +433,8 @@ def main():
     def one_step(i, ev_i, kev_i):
         """One step of the benchmark: [L2 flush, untimed] [event] the frame [event] [counters].  The warm-up steps run this
         very function, so nothing in the timed region is a first use (the first `counters += r.stats` alone loads a
-        torch kernel module: 15 ms of idle GPU after which the next two frames of every rank ran 3-5 % slow)."""
+        torch kernel module: 15 ms of idle GPU after which the next two frames of every rank ran 3-5 % slow).
+        -> (image, stats): what the renderer hands its caller (the [H,W,3] float32 frame on rank 0, None elsewhere)."""
         nonlocal launches, counters
         # L2 flush between the timed steps (untimed: outside the step's event pair).  The K steps are bracketed by a
         # barrier + synchronize on both sides, not individually: inside, the frame protocol itself keeps the ranks together
@@ -424,8 +442,10 @@ def main():
             flush.zero_()
         ev_i[0].record()
         # the step, with the dominant kernel bracketed separately for the roofline
+        image = None
         if fused:
-            r.render_fused(cam, W, H, spp, DEPTH, THRESHOLD, seed=i, fov=FOV, mode=args.mode, kernel_events=kev_i, in_kernel=in_kernel)
+            image, _ = r.render_fused(cam, W, H, spp, DEPTH, THRESHOLD, seed=i, fov=FOV, mode=args.mode, kernel_events=kev_i,
+                                      in_kernel=in_kernel)
             launches += r.launches
         else:
             r._ensure(W, H)
@@ -449,8 +469,11 @@ def main():
                 if rank == 0:
                     r.scene.resolve(r.accum, W, H, spp, r.image, nat.F32)
                     launches += 1
+            if rank == 0:
+                image = r.image
         ev_i[1].record()
         counters += r.stats
+        return image, r.stats
 
     mk_ev = lambda: (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))      # noqa: E731
     for i in range(args.warmup):
@@ -466,9 +489,11 @@ def main():
     launches = 0
     barrier()
     for i in range(args.steps):
-        one_step(i, ev[i], kev[i])
+        last = one_step(i, ev[i], kev[i])
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     step_ms = [a.elapsed_time(b) for a, b in ev]
     kern_ms = [a.elapsed_time(b) for a, b in kev]
     if args.debug_ranks:
