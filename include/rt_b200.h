@@ -167,11 +167,11 @@ typedef struct rt_path_params {
     double mirror_threshold;/* material.reflective > threshold mirrors: 0.9 complex (:349), 0 chandelier (:481) */
     uint64_t seed;
     int32_t accumulate;
-    int32_t schedule;       /* bit 0: 0 = lock-step warps (default), 1 = per-lane path regeneration; bit 1 (value 2):
-                               diagnostic, switch off the camera-ray candidate lists of the FP32 lock-step kernel;
-                               bit 2 (value 4): diagnostic, small scenes use the shared-memory sphere loop instead of
-                               the parameter-block one.  Same image in every combination of bits 0-1; bit 2 changes
-                               the selection key (3 instead of 6 index bits), i.e. near-ties of the FP32 build */
+    int32_t schedule;       /* 0 = default.  Bit 1 (value 2): diagnostic, switch off the camera-ray candidate lists of
+                               the FP32 parameter-block kernel (same image); bit 2 (value 4): diagnostic, small scenes
+                               use the shared-memory sphere loop instead of the parameter-block one, which changes the
+                               selection key (3 instead of 6 index bits), i.e. near-ties of the FP32 build.  Any other
+                               bit (bit 0 included) is rejected with RT_ERR_INVALID */
     int32_t ksplit;         /* lanes sharing one pixel's samples: -1 = automatic (keeps >= 64 waves of CTAs in the grid),
                                0 or 1 = one thread per pixel, 2..32 = that power of two.  Same image either way. */
     int32_t reserved_;

@@ -3,7 +3,6 @@
 #include <atomic>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <limits>
 #include <new>
@@ -278,8 +277,7 @@ static int upload_scene(rt_scene *sc, const rt_scene_desc *s, cudaStream_t st) {
     CU(cudaEventRecord(sc->staged, st));
     {   // small scenes: the path kernel takes the FP32 pair array through its parameter block (kMode 3)
         const int n_pad = (s->n + 7) & ~7;
-        static const bool off = std::getenv("RT_B200_NO_PKC") != nullptr;      // A/B switch for measurements
-        sc->pkc_ok = !off && n_pad > 0 && n_pad <= RT_PKC_MAX && s->nL <= RT_LPKC_MAX;
+        sc->pkc_ok = n_pad > 0 && n_pad <= RT_PKC_MAX && s->nL <= RT_LPKC_MAX;
         std::memset(&sc->pkc, 0, sizeof sc->pkc);
         if (sc->pkc_ok) {
             // blob layout (pack_scene): sph[n_pad] pk[n_pad] mat[n] col[n] g_vec g_col [nG] p_pos p_col [nP] l_pos l_col [nL] lpk
@@ -607,8 +605,7 @@ static int render_whitted_t(rt_scene *sc, const SceneDev<T> &view, const rt_whit
     // FP32 reductions in no fixed order, so only for integer-valued background / miss colours (sums then exact).  Every
     // counter slot has its own tile list, so frames in flight on different streams do not share one
     unsigned *sched2 = nullptr, *heavy = nullptr;
-    static const bool no_split = std::getenv("RT_B200_NO_SPLIT") != nullptr;       // A/B switch for measurements
-    if (sizeof(T) == 4 && !no_split && p->s1 - p->s0 >= 4 && p->s1 - p->s0 <= 4096) {
+    if (sizeof(T) == 4 && p->s1 - p->s0 >= 4 && p->s1 - p->s0 <= 4096) {
         bool ints = true;
         for (int k = 0; k < 3; ++k) {
             const double a = p->miss[k], b = (double)view.bg[k];
@@ -656,6 +653,8 @@ struct ExplicitRays { const double *rays; const int32_t *ids; int depth0; };
 template <typename T>
 static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_path_params *p, void *accum, uint64_t *stats,
                          cudaStream_t st, const rt_path_sink *sink = nullptr, const ExplicitRays *xr = nullptr) {
+    // bit 1: no camera-ray candidate lists, bit 2: no parameter-block kernel (include/rt_b200.h)
+    if (p->schedule & ~6) return fail(RT_ERR_INVALID, "unknown schedule bits");
     PathDev<T> pp;
     std::memset(&pp, 0, sizeof pp);
     if (xr) { pp.rays = xr->rays; pp.ray_ids = xr->ids; pp.depth0 = xr->depth0; }
@@ -671,7 +670,6 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
     for (uint32_t r = 0; r < 10; ++r) { pp.rk[2 * r] = pp.k0 + r * 0x9E3779B9u; pp.rk[2 * r + 1] = pp.k1 + r * 0xBB67AE85u; }
     pp.accumulate = p->accumulate;
     pp.int_fold = sc->int_colours && (p->s1 - p->s0) <= 65536;
-    pp.regenerate = (p->schedule & 1) != 0;
     pp.primary_cull = (p->schedule & 2) == 0;
     pp.sink = RT_SINK_ACCUM; pp.tile_step = 1; pp.world = 1; pp.spp_total = p->s1 - p->s0;
     pp.col_step = 1; pp.col_first = 0; pp.seg_w = p->W;
@@ -758,8 +756,7 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
             // instead of a coarse one (brute-force scenes; with a hierarchy the units are short already)
             int lk2 = lk + 2 < 5 ? lk + 2 : 5;
             while (lk2 > lk && (ns >> lk2) < 2) --lk2;
-            static const bool no_fine = std::getenv("RT_B200_NO_FINE_TAIL") != nullptr;      // A/B switch for measurements
-            if (view.bvh.nodes == 0 && lk2 > lk && !no_fine) {
+            if (view.bvh.nodes == 0 && lk2 > lk) {
                 pp.ksplit2_log2 = lk2;
                 pp.fine_pixels = (int)(3LL * 32 * sms * (32 >> lk) / 2);
             }
@@ -777,10 +774,9 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
     pp.tile_step = sink->tile_step; pp.y0 = sink->tile_first * 8;
     }
     {   // table fold (parameter-block kernel only): worth its per-CTA build (n * 768 entries) from ~4 M pixel-samples up
-        static const bool no_tab = std::getenv("RT_B200_NO_FOLD_TAB") != nullptr;              // A/B switch for measurements
         const int step = pp.tile_step > 1 ? pp.tile_step : 1;
         const long long work = (long long)pp.seg_w * ((pp.y1 - pp.y0 + step - 1) / step) * (p->s1 - p->s0);
-        pp.fold_tab = !no_tab && pp.int_fold && sc->byte_colours && !xr && work >= (4LL << 20);
+        pp.fold_tab = pp.int_fold && sc->byte_colours && !xr && work >= (4LL << 20);
     }
     if (!sc->sched_dev) return fail(RT_ERR_INVALID, "scene has no scheduler counters (upload failed?)");
     unsigned *sched = sc->sched_dev + 4 * (sc->sched_next.fetch_add(1u) % RT_SCHED_SLOTS);      // {next unit, warps done, CTAs resolved, -}
@@ -875,42 +871,9 @@ RT_EXPORT int rt_peer_free(int device, void *ptr_dev) {
     CU(cudaFree(ptr_dev));
     return RT_OK;
 }
-// A flag write that needs no SM: the driver's stream memory operation (cuStreamWriteValue32, default flags = a system
-// fence before the write), fetched through the runtime so that libcuda is not linked.  A release LAUNCH queued behind a
-// copy cannot start while another stream's persistent kernel holds every SM; the memory operation can.
-typedef int (*rt_write_value32_fn)(cudaStream_t, unsigned long long, unsigned int, unsigned int);
-static rt_write_value32_fn stream_write_value32() {
-    static rt_write_value32_fn fn = []() -> rt_write_value32_fn {
-        // opt-in (RT_B200_MEMOPS=1): bit-identical frames in every protocol variant at 2 GPUs, but no measurable gain
-        // there (the release is off the critical path once the frame-on-host event no longer waits for it) and not
-        // exercised at 8 GPUs, so the release stays a one-warp kernel by default
-        if (!std::getenv("RT_B200_MEMOPS")) return nullptr;
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
-        if (cudaGetDriverEntryPoint("cuStreamWriteValue32", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        return reinterpret_cast<rt_write_value32_fn>(p);
-    }();
-    return fn;
-}
-
 RT_EXPORT int rt_peer_signal(int device, uint32_t *const *flag_ptrs, int32_t n, uint32_t epoch, void *stream) {
     if (!flag_ptrs || n < 1 || n > 32) return fail(RT_ERR_INVALID, "bad arguments");
     CU(cudaSetDevice(device));
-    for (int i = 0; i < n; ++i) if (!flag_ptrs[i]) return fail(RT_ERR_INVALID, "NULL flag pointer");
-    if (rt_write_value32_fn wr = stream_write_value32()) {
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        if (cudaStreamIsCapturing(S(stream), &cap) == cudaSuccess && cap == cudaStreamCaptureStatusNone) {
-            int done = 0;
-            for (; done < n; ++done)
-                if (wr(S(stream), (unsigned long long)(uintptr_t)flag_ptrs[done], epoch, 0u) != 0) break;
-            if (done == n) return RT_OK;
-            if (done > 0) return fail(RT_ERR_CUDA, "cuStreamWriteValue32 failed part-way through a signal");
-            // first write refused (address kind not supported by this driver): the kernel below does the job
-        }
-    }
     PeerFlagTable tab;
     std::memset(&tab, 0, sizeof tab);
     for (int i = 0; i < n; ++i) {

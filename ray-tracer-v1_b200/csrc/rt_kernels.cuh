@@ -2,8 +2,8 @@
 // double, without FMA contraction, in rt_f64.cu) and their launchers.
 //
 //   whitted_kernel   Algorithm A frame: camera ray -> nearestSphereIntersect -> terminalRGB, spp accumulation
-//   path_kernel      Algorithm B frame: TraditionalRenderer.render, persistent per-pixel threads that regenerate
-//                    the next sample as soon as a path ends, so every loop trip of a warp is one nearest-hit query
+//   path_kernel      Algorithm B frame: TraditionalRenderer.render, persistent warps whose per-pixel lanes trace one
+//                    sample together, one nearest-hit query per loop trip, and fold it once the longest path has ended
 //   trace_rays_kernel / sphere_disc_kernel   batched Ray.nearestSphereIntersect / sphereDiscriminant
 //   env_reset_kernel / env_step_kernel       batched RayTracerEnv
 //   resolve_kernel   sums -> float32 image
@@ -116,21 +116,6 @@ RT_DEV void flush_stats(unsigned long long *stats, int slot, unsigned long long 
 #endif
 #ifndef RT_PATH_MIN_BLOCKS_PKC
 #define RT_PATH_MIN_BLOCKS_PKC 4   /* kMode 3 needs 72 registers unconstrained: 4 CTAs/SM at 64 measured 2.2 % faster (no spills) */
-#endif
-#ifndef RT_SBASE_OPAQUE
-#define RT_SBASE_OPAQUE 0   /* A/B (negative): base kept in a register saves the 3 uniform instructions per winner fetch, measured SLOWER: 16.60 vs 16.45 ms */
-#endif
-#ifndef RT_DEFER_FOLD
-#define RT_DEFER_FOLD 1        /* lock-step schedule: fold once per sample and warp (A/B: see DESIGN.md) */
-#endif
-#ifndef RT_PHILOX_RK
-#define RT_PHILOX_RK 1         /* Philox round keys from the parameter block instead of two IADD per round */
-#endif
-#ifndef RT_PRIMARY_CULL
-#define RT_PRIMARY_CULL 1      /* camera rays: warp-coherent candidate list instead of the full sphere loop */
-#endif
-#ifndef RT_SKIP_LAST_BOUNCE
-#define RT_SKIP_LAST_BOUNCE 1  /* no bounce direction for the ray that is never traced */
 #endif
 #define RT_MODE_DECL constexpr bool kShared = kMode != 2; constexpr bool kBvh = kMode == 1 || kMode == 2
 
@@ -317,12 +302,6 @@ __global__ void __launch_bounds__(256, RT_WHITTED_MIN_BLOCKS) whitted_heavy_kern
 // ------------------------------------------------------------------ epoch flags in peer memory (rt_path_sink::sync)
 // wait: system-scope acquire loads until the flag has reached the epoch (wrap-safe compare); gives up after
 // timeout_cycles and reports instead of hanging.  post: system-scope release store; the caller has fenced.
-// 1: a warp asks for its NEXT work unit before it traces the current one (the counter's latency is never waited for);
-// 0: when it is done.  Prefetching means that when the counter runs out every warp still owns TWO units, so the drain
-// of a launch is twice as long; with 8 warps per scheduler the ~1 us of the atomic is hidden anyway.
-#ifndef RT_PREFETCH_UNIT
-#define RT_PREFETCH_UNIT 0
-#endif
 #ifdef RT_TRACE_WARPS
 RT_DEV unsigned long long rt_globaltimer() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
 #endif
@@ -369,15 +348,12 @@ template <typename T> RT_DEV V3<T> path_camera_ray(const PathDev<T> &pp, int x, 
     return d;
 }
 
-// One thread per pixel, looping over its samples; 8x4-pixel warps.  Two schedules:
-//   kRegen = false  lock-step: the warp traces sample s of all its 32 pixels together, one nearest-hit query per
-//                   trip, until every lane's path has ended, then folds and starts sample s+1 together.  Everything
-//                   outside the sphere loop (camera ray, Philox, fold) runs once per sample at full lane occupancy.
-//   kRegen = true   path regeneration: a lane starts its next sample the trip after its path ends.  No idle lanes in
-//                   the sphere loop, but lanes drift out of phase, so the per-sample code runs on a few lanes every
-//                   trip.  Pays off only when early termination is common and the per-sample code is short.
+// One thread per pixel, looping over its samples; 8x4-pixel warps in lock-step: the warp traces sample s of all its
+// 32 pixels together, one nearest-hit query per trip, until every lane's path has ended, then folds and starts sample
+// s+1 together.  Everything outside the sphere loop (camera ray, Philox, fold) runs once per sample at full lane
+// occupancy.
 // kIntFold: integer fold through the div255 table (all leaf colours integer-valued), else the double-division fold.
-template <typename T, int kMode, bool kIntFold, bool kRegen>
+template <typename T, int kMode, bool kIntFold>
 __global__ void __launch_bounds__(256, (sizeof(T) == 4 ? (kMode == 3 ? RT_PATH_MIN_BLOCKS_PKC : RT_PATH_MIN_BLOCKS) : 1))
 path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned long long *stats,
             const __grid_constant__ typename std::conditional<kMode == 3, PkConst, PkNone>::type pkc) {
@@ -398,9 +374,6 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
         __shared__ __align__(16) double s_div255[256];
         float4 *const s_sph = s_all, *const s_hit = s_all + RT_PKC_MAX, *const s_col = s_all + 2 * RT_PKC_MAX, *const s_cw = s_all + 3 * RT_PKC_MAX;
         s_base = (unsigned)__cvta_generic_to_shared(s_all);
-#if RT_SBASE_OPAQUE
-        asm volatile("" : "+r"(s_base));       // keep the base in a register: not re-derived from SR_CgaCtaId at every use
-#endif
         const int n_pad = (sc.n + 7) & ~7;
         const float *pkf = reinterpret_cast<const float *>(sc.pk);       // pair j: cx0 cx1 cy0 cy1 | cz0 cz1 w0 w1
         for (int i = threadIdx.x; i < n_pad; i += blockDim.x) {
@@ -423,7 +396,7 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
         S.lb.nL = sc.nL; S.lb.l_pos = sc.l_pos; S.lb.l_col = sc.l_col; S.lb.l_index = sc.l_index; S.lb.lpk = sc.lpk;
         S.la.nG = 0; S.la.nP = 0;
         __syncthreads();
-        if constexpr (kIntFold && !kRegen && !M<T>::exact) {
+        if constexpr (kIntFold && !M<T>::exact) {
             if (pp.fold_tab) {
                 // fold table: entry [sphere][channel][tot] = int(albedo * (tot / 255.0)), the very product the fold evaluates
                 // (fold_path_int), computed once per CTA -- four entries per 32-bit store
@@ -481,8 +454,9 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     // counter, so the scene staging, the div255 table and the statistics flush are paid once per CTA instead of once
     // per tile, the load balances at warp granularity, and the eight warps of a CTA drift apart freely (no barrier
     // inside the loop).  The first units are static (CTA c, warp w -> unit 8c + w); the counter hands out the rest.
-    // A warp asks for its next unit when it has finished the current one (RT_PREFETCH_UNIT: asking before tracing hid the
-    // counter's latency but left every warp with two units in hand when the counter ran out -- twice the drain).
+    // A warp asks for its next unit when it has finished the current one: asking before tracing would hide the
+    // counter's latency (hidden anyway by 8 warps per scheduler) but leave every warp with two units in hand when the
+    // counter runs out -- twice the drain.
     // pp.sched = {next, done}: the last warp of the launch to finish resets both, so no memset precedes a launch.
     const unsigned n_coarse = (unsigned)(pp.gx * pp.gy) << 3, n_units = n_coarse + ((unsigned)(pp.gx2 * pp.gy2) << 3);
     const unsigned first_dyn = (unsigned)gridDim.x << 3;
@@ -491,10 +465,6 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     unsigned long long rt_trace_last = 0, rt_trace_unit = 0;
 #endif
     for (unsigned unit = ((unsigned)blockIdx.x << 3) + (unsigned)w_; unit < n_units;) {
-    unsigned nxt = 0;
-#if RT_PREFETCH_UNIT
-    if (lane_ == 0) nxt = first_dyn + atomicAdd(pp.sched, 1u);
-#endif
     RT_ASSERT(unit < n_units);
 #ifdef RT_TRACE_WARPS
     rt_trace_last = rt_globaltimer(); rt_trace_unit = unit;
@@ -524,7 +494,7 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     // primary rays of this warp tile: spheres its cone of camera rays can touch (cone_candidates, rt_trace.cuh)
     unsigned long long cand = ~0ull;
     bool first_trip = false;                          // warp-uniform: every live lane is about to trace its camera ray
-    if constexpr (kMode == 3 && !kRegen && RT_PRIMARY_CULL) if (pp.primary_cull) {
+    if constexpr (kMode == 3) if (pp.primary_cull) {
         const int bw = 1 << pw_sh, bh = 1 << ph_sh;   // the warp's pixel block
         const int x0 = xs;
         const int y0 = ys;
@@ -544,13 +514,12 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     } else {
         int s = pp.s0 + sub, depth = 0;
         bool alive = has_pixel && s < pp.s1;          // lane has a path in flight
-        bool more = alive;                            // lane still has samples to do (regen schedule)
         V3<T> O = cam, D = mk<T>(T(0), T(0), T(-1));
         // colour at the end of the path: miss / depth limit give Colour(2,2,5), an emissive hit its own colour.  Lives
-        // across trips (reset per sample): in the lock-step schedule the fold waits for the warp's longest path.
+        // across trips (reset per sample): the fold waits for the warp's longest path.
         int leaf0 = 2, leaf1 = 2, leaf2 = 5;
         double lf0 = 2.0, lf1 = 2.0, lf2 = 5.0;
-        bool pend = false;                            // lane traced a sample whose fold is still due (lock-step)
+        bool pend = false;                            // lane traced a sample whose fold is still due
         auto start_sample = [&](int smp) {
             depth = 0; O = cam;
             leaf0 = 2; leaf1 = 2; leaf2 = 5; lf0 = 2.0; lf1 = 2.0; lf2 = 5.0; pend = true;
@@ -565,9 +534,9 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                 }
             }
             rng.begin(pixel, (uint32_t)smp, pp.k0, pp.k1);
-            if constexpr (kMode == 3 && !kRegen && RT_PRIMARY_CULL) if (pp.primary_cull) n_tests += (unsigned)__popcll(cand);
+            if constexpr (kMode == 3) if (pp.primary_cull) n_tests += (unsigned)__popcll(cand);
             uint32_t wa, wb;
-            if (RT_PHILOX_RK) rng.pair_rk(0u, wa, wb, pp.rk); else rng.pair(0u, wa, wb);
+            rng.pair_rk(0u, wa, wb, pp.rk);
             D = path_camera_ray<T>(pp, x, y, u01<T>(wa), u01<T>(wb));
             n_rays++;                                 // trace_ray_traditional call count, chandelier.py:432
         };
@@ -576,15 +545,15 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
         if (alive) start_sample(s);
         first_trip = true;
         for (;;) {
-            const bool primary_trip = first_trip;     // this trip traces the camera rays of a sample (lock-step only)
+            const bool primary_trip = first_trip;     // this trip traces the camera rays of a sample
             first_trip = false;
             bool ended = false;
             int i = -1;
             if constexpr (kMode == 3) {
                 // the selection runs on the CONVERGED warp (its pair votes take the full mask): a lane without a path in
                 // flight goes through the arithmetic on its stale ray and votes "no"; its result is never read
-                if (!kRegen && RT_PRIMARY_CULL && primary_trip && pp.primary_cull) i = select_candidates(S.g.sv.cw, cand, S.g.sv.key_mask6, O, D);
-                else i = brute_select_pkc<!kRegen>(pkc, S.g.sv.n_padded, S.g.sv.key_mask6, O, D, alive);   // regen: lanes leave the loop one by one
+                if (primary_trip && pp.primary_cull) i = select_candidates(S.g.sv.cw, cand, S.g.sv.key_mask6, O, D);
+                else i = brute_select_pkc<true>(pkc, S.g.sv.n_padded, S.g.sv.key_mask6, O, D, alive);
             }
             if (alive) {
                 // ---- one call of trace_ray_traditional below the depth limit: a nearest-hit query
@@ -596,9 +565,8 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                 if constexpr (kMode == 3) {
                     // one LDS.128 for the winner's (centre, r) -- shared by the robust distance and the normal -- and one
                     // for its (1/r, reflective, emissive) record
-                    // sphere tests: the lock-step kernel counts the camera rays' candidates once per sample (start_sample)
-                    // and derives the full-scene queries at the end of the launch (no counter update per trip)
-                    if constexpr (kRegen) n_tests += (unsigned)S.g.sv.n;
+                    // sphere tests: the kernel counts the camera rays' candidates once per sample (start_sample) and
+                    // derives the full-scene queries at the end of the launch (no counter update per trip)
                     if (i >= 0) {
                         float4 w, hr;
                         lds_v4x2<16 * RT_PKC_MAX>(s_base + 16u * (unsigned)i, w, hr);      // (centre, r) and (1/r, reflective, emissive)
@@ -637,7 +605,7 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                         ended = depth >= pp.max_bounces;                             // ... returns (2,2,5) at once
                         // the bounce ray of the deepest level is never traced (counter-based RNG: skipping its
                         // draw changes nothing), so its direction is not computed either
-                        if (!RT_SKIP_LAST_BOUNCE || !ended) {
+                        if (!ended) {
                             const bool mirror = m.x > pp.mirror_threshold;
                             T r1 = T(0), r2 = T(0);
                             // (measured: letting mirror lanes fill the two-slot Philox cache at even depths, so that they
@@ -645,7 +613,7 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                             // LOSES 3.5 % on the chandelier, where most surfaces mirror and the rounds would run for nobody)
                             if (!mirror) {
                                 uint32_t wa, wb;
-                                if (RT_PHILOX_RK) rng.pair_rk((uint32_t)depth, wa, wb, pp.rk); else rng.pair((uint32_t)depth, wa, wb);
+                                rng.pair_rk((uint32_t)depth, wa, wb, pp.rk);
                                 r1 = u01<T>(wa); r2 = u01<T>(wb);
                             }
                             D = bounce_direction<T>(D, h.n, mirror, r1, r2);
@@ -654,54 +622,27 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                     }
                 }
             }
-            if (RT_DEFER_FOLD && !kRegen) {
-                // lock-step: a lane whose path ends early only parks its leaf; the whole warp folds together once
-                // the sample's longest path has ended (one full-occupancy fold instead of several sparse ones)
-                if (ended) alive = false;             // (ended is only ever set by a live lane)
-                if (__any_sync(0xffffffffu, alive)) continue;
-                if (pend) {
-                    pend = false;
-                    if constexpr (kIntFold) {
-                        int c[3] = {leaf0, leaf1, leaf2};
-                        fold_path_int<T, kMode == 3>(S.g, st, depth, div255, c, fold_from, s_base + 32u * RT_PKC_MAX,
-                                                     (kMode == 3 && pp.fold_tab) ? (unsigned)__cvta_generic_to_shared(smem) : 0u);
-                        a0 += (unsigned)c[0]; a1 += (unsigned)c[1]; a2 += (unsigned)c[2];
-                    } else {
-                        double c[3] = {lf0, lf1, lf2};
-                        fold_path<T, kMode == 3>(S.g, st, depth, c, fold_from);
-                        a0 += c[0]; a1 += c[1]; a2 += c[2];
-                    }
-                }
-                s += kk;
-                if (s - sub >= pp.s1) break;
-                if (has_pixel && s < pp.s1) { alive = true; start_sample(s); }
-                first_trip = true;
-                continue;
-            }
-            if (alive && ended) {
-                alive = false;
+            // a lane whose path ends early only parks its leaf; the whole warp folds together once the sample's longest
+            // path has ended (one full-occupancy fold instead of several sparse ones)
+            if (ended) alive = false;                 // (ended is only ever set by a live lane)
+            if (__any_sync(0xffffffffu, alive)) continue;
+            if (pend) {
+                pend = false;
                 if constexpr (kIntFold) {
                     int c[3] = {leaf0, leaf1, leaf2};
-                    fold_path_int<T, kMode == 3>(S.g, st, depth, div255, c, fold_from, s_base + 32u * RT_PKC_MAX);
+                    fold_path_int<T, kMode == 3>(S.g, st, depth, div255, c, fold_from, s_base + 32u * RT_PKC_MAX,
+                                                 (kMode == 3 && pp.fold_tab) ? (unsigned)__cvta_generic_to_shared(smem) : 0u);
                     a0 += (unsigned)c[0]; a1 += (unsigned)c[1]; a2 += (unsigned)c[2];
                 } else {
                     double c[3] = {lf0, lf1, lf2};
                     fold_path<T, kMode == 3>(S.g, st, depth, c, fold_from);
                     a0 += c[0]; a1 += c[1]; a2 += c[2];
                 }
-                if constexpr (kRegen) {
-                    if ((s += kk) < pp.s1) { alive = true; start_sample(s); } else more = false;
-                }
             }
-            if constexpr (kRegen) {
-                if (!more) break;
-            } else {
-                if (__any_sync(0xffffffffu, alive)) continue;      // wait for the warp's longest path
-                s += kk;
-                if (s - sub >= pp.s1) break;                       // s - sub is warp-uniform in this schedule
-                if (has_pixel && s < pp.s1) { alive = true; start_sample(s); }
-                first_trip = true;
-            }
+            s += kk;
+            if (s - sub >= pp.s1) break;              // s - sub is warp-uniform
+            if (has_pixel && s < pp.s1) { alive = true; start_sample(s); }
+            first_trip = true;
         }
     }
     if constexpr (kIntFold) {                        // the k lanes of a pixel are adjacent: butterfly sum
@@ -743,9 +684,8 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
             accum[o] = out;
         }
     }
-#if !RT_PREFETCH_UNIT
+    unsigned nxt = 0;
     if (lane_ == 0) nxt = first_dyn + atomicAdd(pp.sched, 1u);
-#endif
     unit = __shfl_sync(0xffffffffu, nxt, 0);
     }   // work units of this warp
 #ifdef RT_TRACE_WARPS
@@ -814,11 +754,11 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
         flush_stats(stats, STAT_SMALL, n_small);
         flush_stats(stats, STAT_QUERIES, n_query);
         unsigned long long tests = n_tests;
-        if constexpr (kMode == 3 && !kRegen) {
+        if constexpr (kMode == 3) {
             // every query but the camera rays' (when those walk their candidate lists) tests the whole scene; a camera
             // ray is a trace call that no hit caused: n_rays - (n_inter - n_light)
             unsigned n_prim = 0u;
-            if (RT_PRIMARY_CULL && pp.primary_cull) n_prim = n_rays - (n_inter - n_light);
+            if (pp.primary_cull) n_prim = n_rays - (n_inter - n_light);
             tests += (unsigned long long)(n_query - min(n_prim, n_query)) * (unsigned)sc.n;
         }
         flush_stats(stats, STAT_SPHERE_TESTS, tests);
@@ -1291,15 +1231,8 @@ template <typename T> RT_DEV double env_lighting_reward(const Geo<T> &g, const E
 // 18 stores), then the CTA copies the block of rows to HBM as consecutive 16-byte stores -- the per-thread rows would
 // be 72-byte strided 4-byte stores, 18 partial sectors per warp instruction.
 #ifndef RT_ENV_BLOCK
-#define RT_ENV_BLOCK 64         /* envs per CTA.  65,536 envs = 1,024 CTAs = 6.9 per SM: 1 % imbalance (128: 3.46 per SM, 15 %) */
+#define RT_ENV_BLOCK 64         /* envs (one thread each) per CTA.  65,536 envs = 1,024 CTAs = 6.9 per SM: 1 % imbalance (128: 3.46 per SM, 15 %) */
 #endif
-// Envs per warp.  The step is latency-bound, not issue-bound (65,536 envs are 3.5 full warps per scheduler, issue slots
-// 27 % busy, and every divergent branch of a warp runs one after the other), so a warp carries RT_ENV_LANES envs in its
-// low lanes and leaves the others idle: more warps per scheduler to hide latency, fewer distinct paths per warp.
-#ifndef RT_ENV_LANES
-#define RT_ENV_LANES 32
-#endif
-#define RT_ENV_THREADS (RT_ENV_BLOCK / RT_ENV_LANES * 32)
 // register budget of the step kernel: left to itself ptxas settles on 80 registers and spills 64 bytes; the launch
 // never has more than 14 warps per SM to place (65,536 episodes / 148 SMs), so registers are free
 #ifndef RT_ENV_REGS
@@ -1311,9 +1244,9 @@ RT_DEV void env_flush_obs(const float *rows, float *obs, int B) {
     const int n = min(RT_ENV_BLOCK, B - base) * 18;                      // floats of this CTA's rows
     float *dst = obs + (size_t)base * 18;                                // 64 * 72 bytes per CTA: 16-byte aligned
     const int n4 = (((uintptr_t)obs & 15u) == 0) ? n >> 2 : 0;
-    for (int j = threadIdx.x; j < n4; j += RT_ENV_THREADS)
+    for (int j = threadIdx.x; j < n4; j += RT_ENV_BLOCK)
         reinterpret_cast<float4 *>(dst)[j] = reinterpret_cast<const float4 *>(rows)[j];
-    for (int j = 4 * n4 + threadIdx.x; j < n; j += RT_ENV_THREADS) dst[j] = rows[j];
+    for (int j = 4 * n4 + threadIdx.x; j < n; j += RT_ENV_BLOCK) dst[j] = rows[j];
 }
 
 // reset of one episode (RL/ray_tracer_env.py:254-293, _get_initial_ray :121-142): camera ray through pixel (px, py),
@@ -1407,11 +1340,11 @@ __global__ void __maxnreg__(RT_ENV_REGS) env_step_kernel(SceneDev<T> sc, EnvDev<
     __shared__ __align__(16) float s_rows[RT_ENV_BLOCK * 18];
     Staged<T> S;
     stage_scene<T, kShared>(sc, smem, S);
-    const int slot = RT_ENV_LANES == 32 ? (int)threadIdx.x : (int)(threadIdx.x >> 5) * RT_ENV_LANES + (int)(threadIdx.x & 31u);
+    const int slot = (int)threadIdx.x;
     const int b = blockIdx.x * RT_ENV_BLOCK + slot;
     float *row = s_rows + 18 * slot;
     Counters ct = {0u, 0u, 0u, 0u};
-    if ((RT_ENV_LANES == 32 || (threadIdx.x & 31u) < RT_ENV_LANES) && b < e.B) {
+    if (b < e.B) {
         const unsigned live = __activemask();       // the lanes of this warp that carry an episode (converged here)
         EnvReg<T> st = env_load<T>(e, b);
         RT_ASSERT(st.idx >= -1 && st.idx < sc.n && st.bounce >= 0);
@@ -1646,37 +1579,33 @@ cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, void *accum
     int mode = mode_for(sc, extra);
     // small brute-force FP32 scenes: sphere pairs through the parameter block (kMode 3)
     if (mode == 0 && sizeof(T) == 4 && pkc && ((sc.n + 7) & ~7) <= RT_PKC_MAX && sc.nL <= RT_LPKC_MAX) mode = 3;
-    if (mode != 3 || !pp.int_fold || pp.regenerate) ppl.fold_tab = 0;
+    if (mode != 3 || !pp.int_fold) ppl.fold_tab = 0;
     // kMode 3 uses static shared arrays; its dynamic part is the fold table [n][3][256] bytes
     const size_t sm = mode == 3 ? (ppl.fold_tab ? (size_t)sc.n * 768 : 0) : (mode != 2 ? smem_for(sc) : 0) + extra;
     cudaError_t e = cudaSuccess;
-#define RT_PATH_CASE(M_, F_, R_)                                                                                   \
-    { e = allow_smem(path_kernel<T, M_, F_, R_>, sm); if (e != cudaSuccess) return e;                              \
-      grid.x = persistent_ctas(path_kernel<T, M_, F_, R_>, sm, tiles_total);                                       \
+#define RT_PATH_CASE(M_, F_)                                                                                       \
+    { e = allow_smem(path_kernel<T, M_, F_>, sm); if (e != cudaSuccess) return e;                                  \
+      grid.x = persistent_ctas(path_kernel<T, M_, F_>, sm, tiles_total);                                           \
       if (pp.max_ctas > 0 && grid.x > (unsigned)pp.max_ctas) grid.x = (unsigned)pp.max_ctas;                        \
-      path_kernel<T, M_, F_, R_><<<grid, block, sm, st>>>(sc, ppl, (v4 *)accum, stats, PkNone()); }
+      path_kernel<T, M_, F_><<<grid, block, sm, st>>>(sc, ppl, (v4 *)accum, stats, PkNone()); }
     if (mode == 3) {
         if constexpr (sizeof(T) == 4) {
-#define RT_PATH_CASE3(F_, R_)                                                                                      \
-    { e = allow_smem(path_kernel<T, 3, F_, R_>, sm ? sm + 8192 : 0); /* + the static arrays: opt in above 48 KB in all */ \
+#define RT_PATH_CASE3(F_)                                                                                          \
+    { e = allow_smem(path_kernel<T, 3, F_>, sm ? sm + 8192 : 0); /* + the static arrays: opt in above 48 KB in all */ \
       if (e != cudaSuccess) return e;                                                                              \
-      grid.x = persistent_ctas(path_kernel<T, 3, F_, R_>, sm, tiles_total);                                        \
+      grid.x = persistent_ctas(path_kernel<T, 3, F_>, sm, tiles_total);                                            \
       if (pp.max_ctas > 0 && grid.x > (unsigned)pp.max_ctas) grid.x = (unsigned)pp.max_ctas;                        \
-      path_kernel<T, 3, F_, R_><<<grid, block, sm, st>>>(sc, ppl, (v4 *)accum, stats, *pkc); }
-            if (pp.int_fold) { if (pp.regenerate) RT_PATH_CASE3(true, true) else RT_PATH_CASE3(true, false) }
-            else { if (pp.regenerate) RT_PATH_CASE3(false, true) else RT_PATH_CASE3(false, false) }
+      path_kernel<T, 3, F_><<<grid, block, sm, st>>>(sc, ppl, (v4 *)accum, stats, *pkc); }
+            if (pp.int_fold) RT_PATH_CASE3(true) else RT_PATH_CASE3(false)
 #undef RT_PATH_CASE3
         }
         return cudaGetLastError();
     }
-    const int variant = mode * 4 + (pp.int_fold ? 2 : 0) + (pp.regenerate ? 1 : 0);
+    const int variant = mode * 2 + (pp.int_fold ? 1 : 0);
     switch (variant) {
-        case 0: RT_PATH_CASE(0, false, false) break;   case 1: RT_PATH_CASE(0, false, true) break;
-        case 2: RT_PATH_CASE(0, true, false) break;    case 3: RT_PATH_CASE(0, true, true) break;
-        case 4: RT_PATH_CASE(1, false, false) break;   case 5: RT_PATH_CASE(1, false, true) break;
-        case 6: RT_PATH_CASE(1, true, false) break;    case 7: RT_PATH_CASE(1, true, true) break;
-        case 8: RT_PATH_CASE(2, false, false) break;   case 9: RT_PATH_CASE(2, false, true) break;
-        case 10: RT_PATH_CASE(2, true, false) break;   default: RT_PATH_CASE(2, true, true) break;
+        case 0: RT_PATH_CASE(0, false) break;   case 1: RT_PATH_CASE(0, true) break;
+        case 2: RT_PATH_CASE(1, false) break;   case 3: RT_PATH_CASE(1, true) break;
+        case 4: RT_PATH_CASE(2, false) break;   default: RT_PATH_CASE(2, true) break;
     }
 #undef RT_PATH_CASE
     return cudaGetLastError();
@@ -1769,7 +1698,7 @@ cudaError_t launch_env_step(const SceneDev<T> &sc, const EnvDev<T> &e, const flo
                             uint8_t *terminated, uint8_t *truncated, int *reason, R *info, float *final_obs, int *pixels_out,
                             uint64_t seed, unsigned long long *stats, cudaStream_t st) {
     if (e.B <= 0) return cudaSuccess;
-    const int block = RT_ENV_THREADS, grid = (e.B + RT_ENV_BLOCK - 1) / RT_ENV_BLOCK;
+    const int block = RT_ENV_BLOCK, grid = (e.B + RT_ENV_BLOCK - 1) / RT_ENV_BLOCK;
     const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
     const size_t rows = RT_ENV_BLOCK * 18 * sizeof(float);                 // static shared rows on top of the staged scene
     const int mode = mode_for(sc, rows);

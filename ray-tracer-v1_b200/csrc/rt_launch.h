@@ -43,8 +43,7 @@ template <typename T> struct PathDev {
     int int_fold;                // every leaf colour is an integer in [0, 65535]: integer fold + uint32 accumulators
     int fold_tab;                // kMode 3, int_fold, every colour <= 255: the fold reads int(albedo * (tot / 255.0)) from a
                                  // per-CTA byte table [sphere][channel][tot] in dynamic shared memory (n * 768 bytes)
-    int regenerate;              // 1: path-regeneration schedule, 0: lock-step schedule (rt_kernels.cuh)
-    int primary_cull;            // 1: camera rays use the warp tile's candidate list (FP32 lock-step kMode 3)
+    int primary_cull;            // 1: camera rays use the warp tile's candidate list (FP32 kMode 3)
     // fused multi-GPU sinks (rt_path_sink, include/rt_b200.h); sink == 0: accum only
     int ksplit_log2;             // 2^ksplit_log2 lanes share a pixel and split its samples (integer fold only)
     int sink, tile_step, world, spp_total;

@@ -200,16 +200,13 @@ RT_DEV int brute_select_pk(const float4 *pk, int n_padded, int key_mask, V3<floa
 // fully unrolled so that every LDCU.128 has an immediate constant-bank address, and the sphere operands of FFMA2 /
 // FADD2 are uniform registers.  Groups at or beyond n_padded are skipped by a uniform branch.
 //
-// RT_VOTE_SKIP: the second half of a pair's test -- sign merge, MUFU.SQRT, t, key, running minimum: 10 of its 27 issue
+// Vote skip: the second half of a pair's test -- sign merge, MUFU.SQRT, t, key, running minimum: 10 of its 27 issue
 // cycles -- only matters if SOME lane can hit one of the two spheres, i.e. has tca >= 0 and disc >= 0 (the conditions
 // the sign merge folds into the square root).  For the small spheres of a scene that is rare even for 32 incoherent
 // bounce rays (complex scene: 2-24 % of the warp trips per pair, tools/sim/cull_sim.py), so one warp vote on the sign
 // bits of (tca | disc) skips it for the whole warp; a skipped pair would have produced two NaN keys, so the winner,
 // ties included, is unchanged and frames stay bit-identical.  The first RT_PKC_ALWAYS_PAIRS pairs (the wall spheres
 // of every reference scene, hit by some lane in ~100 % of the trips) are finished unconditionally.
-#ifndef RT_VOTE_SKIP
-#define RT_VOTE_SKIP 1
-#endif
 #ifndef RT_PKC_ALWAYS_PAIRS
 #define RT_PKC_ALWAYS_PAIRS 3
 #endif
@@ -252,7 +249,7 @@ RT_DEV int brute_select_pkc(const PkConst &pkc, int n_padded, int key_mask6, V3<
             }
             const bool always = base / 2 + j0 < RT_PKC_ALWAYS_PAIRS;
             bool some = true;
-            if (RT_VOTE_SKIP && kWarp && !always) some = __any_sync(0xffffffffu, x >= 0 && live);
+            if (kWarp && !always) some = __any_sync(0xffffffffu, x >= 0 && live);
             if (__builtin_expect(some, always)) {
 #pragma unroll
                 for (int v = 0; v < RT_VOTE_PAIRS; ++v) {

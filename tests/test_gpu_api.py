@@ -430,3 +430,15 @@ def test_step_auto_equals_step_plus_masked_reset(rt, precision, flavour):
          0.0 if exact else {"rl": 7.5e-3, "fb": 1.5e-3}[flavour])
     assert finished > B                              # every env restarted at least once inside the fused launches
     fused.close(); graph.close(); plain.close()
+
+
+def test_unknown_schedule_bits_are_rejected(rt):
+    """rt_path_params.schedule knows bits 1 and 2 only; any other bit is an error, not a silent default render."""
+    from ray_tracer_v1_b200 import _native as nat
+    z, fs = load_golden("path_chandelier_48x27")
+    sc = nat.DeviceScene(fs)
+    for schedule in (1, 8):
+        p = sc.path_params(z["cam"], 16, 16, 1, int(z["max_bounces"]), float(z["mirror_threshold"]), schedule=schedule)
+        with pytest.raises(nat.NativeLibraryError, match="unknown schedule bits"):
+            sc.render_path_host(p, nat.F32)
+    sc.close()

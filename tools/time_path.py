@@ -1,5 +1,6 @@
 #!/usr/bin/env python
-"""Device-time the path kernel alone (CUDA events) for schedule / scene / spp variants.  Development aid."""
+"""Device-time the path kernel alone (CUDA events) for scene / spp / ksplit variants and the diagnostic schedule bits
+(rt_path_params.schedule: 2 = no camera-ray candidate lists, 4 = no parameter-block kernel).  Development aid."""
 import argparse
 import os
 import sys
@@ -22,7 +23,7 @@ def main():
     ap.add_argument("--h", type=int, default=1080)
     ap.add_argument("--lbvh", action="store_true")
     ap.add_argument("--ksplit", type=int, default=-1, help="-1 auto, 0 off, k = lanes per pixel")
-    ap.add_argument("--schedules", default="0,1")
+    ap.add_argument("--schedules", default="0", help="comma-separated schedule values, e.g. 0,2,4")
     ap.add_argument("--no-stats", action="store_true", help="launch without the statistics counters")
     ap.add_argument("--save", default=None, help="write the last accumulation buffer to this .npy")
     args = ap.parse_args()
