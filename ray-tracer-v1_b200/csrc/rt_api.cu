@@ -5,6 +5,7 @@
 #include <cstdio>
 #include <cstring>
 #include <limits>
+#include <mutex>
 #include <new>
 #include <string>
 #include <vector>
@@ -353,15 +354,24 @@ RT_EXPORT int rt_device_count(int *count) {
     return RT_OK;
 }
 
+// cudaDeviceGetAttribute, asked once per (device, attribute): the clock rate is a slow query.  Failures are not cached.
+static cudaError_t device_attr(int dev, cudaDeviceAttr attr, int *value) {
+    struct Entry { int dev; cudaDeviceAttr attr; int value; };
+    static std::mutex mu;
+    static std::vector<Entry> cache;
+    std::lock_guard<std::mutex> lock(mu);
+    for (const Entry &c : cache)
+        if (c.dev == dev && c.attr == attr) { *value = c.value; return cudaSuccess; }
+    const cudaError_t e = cudaDeviceGetAttribute(value, attr, dev);
+    if (e == cudaSuccess) cache.push_back(Entry{dev, attr, *value});
+    return e;
+}
+
 RT_EXPORT int rt_device_props(int device, int64_t *props6, size_t *total_mem) {
     cudaDeviceProp p;
     CU(cudaGetDeviceProperties(&p, device));
-    static int khz_cache[64] = {0};        // cudaDevAttrClockRate is a slow query: once per device
-    int khz = device >= 0 && device < 64 ? khz_cache[device] : 0;
-    if (khz == 0) {
-        CU(cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, device));
-        if (device >= 0 && device < 64) khz_cache[device] = khz;
-    }
+    int khz = 0;
+    CU(device_attr(device, cudaDevAttrClockRate, &khz));
     if (props6) {
         props6[0] = p.multiProcessorCount; props6[1] = p.major; props6[2] = p.minor; props6[3] = khz;
         props6[4] = p.l2CacheSize; props6[5] = (int64_t)p.sharedMemPerBlockOptin;
@@ -650,6 +660,93 @@ RT_EXPORT int rt_render_whitted(rt_scene *scene, int precision, const rt_whitted
 // ------------------------------------------------------------------ Algorithm B frame
 struct ExplicitRays { const double *rays; const int32_t *ids; int depth0; };
 
+// chandelier.py:412-415: aspect = W/H; half_height = tan(radians(fov)/2); half_width = half_height*aspect
+template <typename T> static void path_camera(PathDev<T> &pp, const rt_path_params *p) {
+    for (int k = 0; k < 3; ++k) pp.cam[k] = (T)p->cam[k];
+    pp.W = p->W; pp.H = p->H;
+    const double aspect = (double)p->W / (double)p->H;
+    const double half_h = std::tan((p->fov_deg * (M_PI / 180.0)) / 2), half_w = half_h * aspect;
+    pp.aspect = (T)aspect; pp.half_w = (T)half_w; pp.half_h = (T)half_h;
+    pp.inv_W = (T)(1.0 / (double)p->W); pp.inv_H = (T)(1.0 / (double)p->H);
+}
+
+// Cuts one path-kernel launch into work units: sets the band (y0, tile_step, col_*, seg_w), the sample split, both tile
+// grids and fold_tab of pp (which holds W, y1 and int_fold of the request) and returns the kernel variant and its dynamic
+// shared memory.  Every rank of a frame plans from the same numbers, so the launches of a frame tile it exactly.
+template <typename T>
+static PathLaunch plan_path_launch(PathDev<T> &pp, const SceneDev<T> &sc, const rt_path_params *p, const rt_path_sink *sink,
+                                   bool xr, bool byte_colours, bool allow_pkc, int sms) {
+    const int ns = p->s1 - p->s0;
+    const bool image = sink && sink->mode == RT_SINK_IMAGE;
+    long long pixels = 0;
+    // interleave: the 2-D interleave (rt_path_sink::col_split), one column segment of every stripe; false when a segment
+    // does not hold whole work units of both tile grids (32 / 16 / 8 / 4 pixels wide for 1-2 / 4 / 8-16 / 32 lanes per pixel)
+    auto plan = [&](bool interleave) {
+        pp.col_step = 1; pp.col_first = 0; pp.seg_w = p->W; pp.tile_step = 1; pp.y0 = p->y0;
+        if (interleave) {
+            pp.col_step = sink->tile_step; pp.col_first = sink->tile_first; pp.seg_w = p->W / sink->tile_step; pp.y0 = 0;
+        } else if (image) {                                     // every tile_step-th 8-row stripe from tile_first
+            pp.tile_step = sink->tile_step; pp.y0 = sink->tile_first * 8;
+        }
+        const int rows = pp.y1 - pp.y0, step = pp.tile_step;
+        const int owned = ((rows + 7) / 8 + step - 1) / step;             // 8-row stripes of this launch
+        pixels = (long long)pp.seg_w * ((rows + step - 1) / step);
+        // sample split (automatic): k lanes per pixel so that a lane keeps about 8 samples -- measured best at 8, 16, 32
+        // and 64 samples per launch (k = 1, 2, 4, 8: tighter camera-ray cones against per-unit overhead) -- and, for small
+        // frames, more lanes per pixel until there are ~4 warp tiles per resident warp (every lane keeps >= 2 samples)
+        int lk = 0;
+        pp.ksplit2_log2 = 0;
+        if (pp.int_fold && p->ksplit != 0 && !xr) {
+            if (p->ksplit > 0) { while ((1 << (lk + 1)) <= p->ksplit && lk < 5) ++lk; }
+            else {
+                const long long want = 4LL * 32 * sms;             // warp tiles: 4 per resident warp (32 warps per SM)
+                // with a hierarchy the lanes of a pixel traverse together: coherence wins, 8 lanes per pixel whenever a
+                // lane keeps >= 2 samples (1e3-1e5-sphere scenes: 11.3 / 48.5 / 222 ms per 16 spp against 12.5 / 51.9 / 227)
+                const int per_lane = sc.bvh.nodes > 0 ? 2 : 8;
+                while (lk < 3 && (ns >> (lk + 1)) >= per_lane) ++lk;
+                while (lk < 5 && (pixels << lk) / 32 < want && (ns >> (lk + 1)) >= 2) ++lk;
+                // the LAST work units of the launch are finer (more lanes per pixel, every lane still keeps >= 2 samples),
+                // so that the drain of the launch is a fine unit long instead of a coarse one (brute-force scenes; with a
+                // hierarchy the units are short already)
+                int lk2 = lk + 2 < 5 ? lk + 2 : 5;
+                while (lk2 > lk && (ns >> lk2) < 2) --lk2;
+                if (sc.bvh.nodes == 0 && lk2 > lk) pp.ksplit2_log2 = lk2;
+            }
+        }
+        pp.ksplit_log2 = lk;
+        const int lk2 = pp.ksplit2_log2 > lk ? pp.ksplit2_log2 : lk, pw = unit_pw_log2(lk), pw2 = unit_pw_log2(lk2);
+        const int ctw = 4 << pw, cth = 2 << ((5 - lk) - pw), ctw2 = 4 << pw2, cth2 = 2 << ((5 - lk2) - pw2);
+        // coarse tile grid: stripes of 8 rows (8 / cth CTA rows each); without interleaving the last stripe may be cut short
+        pp.gx = (pp.seg_w + ctw - 1) / ctw;
+        pp.gy = step > 1 ? owned * (8 / cth) : (rows + cth - 1) / cth;
+        pp.gx2 = pp.gy2 = pp.stripe2 = 0;
+        if (lk2 > lk) {
+            // fine grid over the last owned stripes (see path_kernel): 1.5 coarse units' worth of pixels per resident
+            // warp, whole 8-row stripes, at most half of them
+            int fs = (int)((3LL * 32 * sms * (32 >> lk) / 2 + 8LL * pp.seg_w - 1) / (8LL * pp.seg_w));
+            if (fs > owned / 2) fs = owned / 2;
+            if (fs >= 1) {
+                const int sb = owned - fs, rows_a = sb * 8;             // (tile_step == 1: rows of the coarse part)
+                pp.stripe2 = sb;
+                pp.gy = step > 1 ? sb * (8 / cth) : (rows_a + cth - 1) / cth;
+                pp.gx2 = (pp.seg_w + ctw2 - 1) / ctw2;
+                pp.gy2 = step > 1 ? fs * (8 / cth2) : (rows - rows_a + cth2 - 1) / cth2;
+            }
+        }
+        return !interleave || (pp.seg_w % ctw == 0 && pp.seg_w % ctw2 == 0);
+    };
+    if (!plan(image && sink->col_split && sink->tile_step > 1)) plan(false);
+    const size_t extra = 256 * sizeof(double);                  // div255 table of the integer fold
+    PathLaunch pl;
+    pl.mode = mode_for(sc, extra);
+    if (pl.mode == 0 && allow_pkc) pl.mode = 3;   // small brute-force FP32 scenes: sphere pairs through the parameter block
+    // table fold (kMode 3 only): worth its per-CTA build (n * 768 entries) from ~4 M pixel-samples up
+    pp.fold_tab = pl.mode == 3 && pp.int_fold && byte_colours && pixels * ns >= (4LL << 20);
+    // kMode 3 uses static shared arrays; its dynamic part is the fold table [n][3][256] bytes
+    pl.smem = pl.mode == 3 ? (pp.fold_tab ? (size_t)sc.n * 768 : 0) : (pl.mode != 2 ? smem_for(sc) : 0) + extra;
+    return pl;
+}
+
 template <typename T>
 static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_path_params *p, void *accum, uint64_t *stats,
                          cudaStream_t st, const rt_path_sink *sink = nullptr, const ExplicitRays *xr = nullptr) {
@@ -658,35 +755,25 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
     PathDev<T> pp;
     std::memset(&pp, 0, sizeof pp);
     if (xr) { pp.rays = xr->rays; pp.ray_ids = xr->ids; pp.depth0 = xr->depth0; }
-    pp.cam[0] = (T)p->cam[0]; pp.cam[1] = (T)p->cam[1]; pp.cam[2] = (T)p->cam[2];
-    pp.W = p->W; pp.H = p->H; pp.y0 = p->y0; pp.y1 = p->y1; pp.s0 = p->s0; pp.s1 = p->s1; pp.max_bounces = p->max_bounces;
-    // chandelier.py:412-415: aspect = W/H; half_height = tan(radians(fov)/2); half_width = half_height*aspect
-    const double aspect = (double)p->W / (double)p->H;
-    const double half_h = std::tan((p->fov_deg * (M_PI / 180.0)) / 2), half_w = half_h * aspect;
-    pp.aspect = (T)aspect; pp.half_w = (T)half_w; pp.half_h = (T)half_h;
-    pp.inv_W = (T)(1.0 / (double)p->W); pp.inv_H = (T)(1.0 / (double)p->H);
+    path_camera(pp, p);
+    pp.y0 = p->y0; pp.y1 = p->y1; pp.s0 = p->s0; pp.s1 = p->s1; pp.max_bounces = p->max_bounces;
     pp.mirror_threshold = (T)p->mirror_threshold;
     pp.k0 = (uint32_t)p->seed; pp.k1 = (uint32_t)(p->seed >> 32);
     for (uint32_t r = 0; r < 10; ++r) { pp.rk[2 * r] = pp.k0 + r * 0x9E3779B9u; pp.rk[2 * r + 1] = pp.k1 + r * 0xBB67AE85u; }
     pp.accumulate = p->accumulate;
     pp.int_fold = sc->int_colours && (p->s1 - p->s0) <= 65536;
     pp.primary_cull = (p->schedule & 2) == 0;
-    pp.sink = RT_SINK_ACCUM; pp.tile_step = 1; pp.world = 1; pp.spp_total = p->s1 - p->s0;
-    pp.col_step = 1; pp.col_first = 0; pp.seg_w = p->W;
-    pp.ksplit_log2 = 0; pp.ksplit2_log2 = 0; pp.fine_pixels = 0; pp.gx2 = pp.gy2 = pp.stripe2 = 0;
+    pp.sink = RT_SINK_ACCUM; pp.world = 1; pp.spp_total = p->s1 - p->s0;
     if (sink && sink->mode != RT_SINK_ACCUM) {
         if (!pp.int_fold) return fail(RT_ERR_UNSUPPORTED, "fused sinks need integer colours and <= 65536 samples per launch");
         pp.sink = sink->mode;
         pp.timed_out = sink->timed_out;          // read under the frame protocol only (and by the RT_TRACE_WARPS development build)
         if (sink->mode == RT_SINK_IMAGE) {
             if (!sink->image || sink->tile_step < 1 || sink->tile_first < 0) return fail(RT_ERR_INVALID, "bad image sink");
-            pp.image = sink->image; pp.tile_step = sink->tile_step;
-            pp.y0 = sink->tile_first * 8; pp.y1 = p->H;
+            pp.image = sink->image;
             if (sink->col_split && sink->tile_step > 1) {
                 if (p->W % sink->tile_step != 0) return fail(RT_ERR_INVALID, "col_split: W must be a multiple of tile_step");
                 if (sink->tile_first >= sink->tile_step) return fail(RT_ERR_INVALID, "col_split: tile_first must be < tile_step");
-                pp.col_step = sink->tile_step; pp.col_first = sink->tile_first; pp.seg_w = p->W / sink->tile_step;
-                pp.tile_step = 1; pp.y0 = 0;              // every stripe, one column segment of each
             }
             if (p->s0 != 0) return fail(RT_ERR_INVALID, "an image sink resolves in the kernel: the launch must cover all samples");
         } else if (sink->mode == RT_SINK_SCATTER_ADD) {
@@ -719,69 +806,18 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
                 pp.spp_total = sink->spp_total;
             }
             pp.timed_out = sink->timed_out;
-            static int khz_cache[64] = {0};
-            int khz = sc->device >= 0 && sc->device < 64 ? khz_cache[sc->device] : 0;
-            if (khz == 0) {
-                if (cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, sc->device) != cudaSuccess || khz <= 0) khz = 2000000;
-                if (sc->device >= 0 && sc->device < 64) khz_cache[sc->device] = khz;
-            }
+            int khz = 0;
+            if (device_attr(sc->device, cudaDevAttrClockRate, &khz) != cudaSuccess || khz <= 0) khz = 2000000;
             pp.timeout_cycles = (long long)(sink->timeout_ms > 0 ? sink->timeout_ms : 20000) * (long long)khz;
         }
     }
-    // sample split (automatic): k lanes per pixel so that a lane keeps about 8 samples -- measured best at 8, 16, 32 and
-    // 64 samples per launch (k = 1, 2, 4, 8: tighter camera-ray cones against per-unit overhead) -- and, for small frames,
-    // more lanes per pixel until there are ~4 warp tiles per resident warp (every lane keeps >= 2 samples)
-    for (int attempt = 0; attempt < 2; ++attempt) {
-    pp.ksplit_log2 = 0; pp.ksplit2_log2 = 0; pp.fine_pixels = 0;
-    if (pp.int_fold && p->ksplit != 0 && !xr) {
-        static int sm_cache[64] = {0};
-        int sms = sc->device >= 0 && sc->device < 64 ? sm_cache[sc->device] : 0;
-        if (sms == 0) {
-            if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, sc->device) != cudaSuccess || sms <= 0) sms = 148;
-            if (sc->device >= 0 && sc->device < 64) sm_cache[sc->device] = sms;
-        }
-        const long long want = 4LL * 32 * sms;                 // warp tiles: 4 per resident warp (32 warps per SM)
-        const int rows = pp.y1 - pp.y0, step = pp.tile_step > 1 ? pp.tile_step : 1, ns = p->s1 - p->s0;
-        const long long pixels = (long long)pp.seg_w * ((rows + step - 1) / step);
-        int lk = 0;
-        if (p->ksplit > 0) { while ((1 << (lk + 1)) <= p->ksplit && lk < 5) ++lk; }
-        else {
-            // with a hierarchy the lanes of a pixel traverse together: coherence wins, 8 lanes per pixel whenever a
-            // lane keeps >= 2 samples (1e3-1e5-sphere scenes: 11.3 / 48.5 / 222 ms per 16 spp against 12.5 / 51.9 / 227)
-            const int per_lane = view.bvh.nodes > 0 ? 2 : 8;
-            while (lk < 3 && (ns >> (lk + 1)) >= per_lane) ++lk;
-            while (lk < 5 && (pixels << lk) / 32 < want && (ns >> (lk + 1)) >= 2) ++lk;
-            // the LAST work units of the launch are finer (more lanes per pixel, every lane still keeps >= 2 samples):
-            // 1.5 coarse units' worth of pixels per resident warp, so that the drain of the launch is a fine unit long
-            // instead of a coarse one (brute-force scenes; with a hierarchy the units are short already)
-            int lk2 = lk + 2 < 5 ? lk + 2 : 5;
-            while (lk2 > lk && (ns >> lk2) < 2) --lk2;
-            if (view.bvh.nodes == 0 && lk2 > lk) {
-                pp.ksplit2_log2 = lk2;
-                pp.fine_pixels = (int)(3LL * 32 * sms * (32 >> lk) / 2);
-            }
-        }
-        pp.ksplit_log2 = lk;
-    }
-    // 2-D interleave: a column segment must hold whole work units of both tile grids (32 / 16 / 8 / 4 pixels wide for
-    // 1-2 / 4 / 8-16 / 32 lanes per pixel); if it does not, the launch falls back to whole stripes and the split is
-    // chosen again for that geometry.  Every rank of a frame decides the same from the same numbers.
-    if (pp.col_step <= 1) break;
-    auto unit_w = [](int lk) { return 4 << (lk == 0 ? 3 : lk == 1 ? 3 : lk == 2 ? 2 : lk <= 4 ? 1 : 0); };
-    const int wa = unit_w(pp.ksplit_log2), wb = pp.ksplit2_log2 > pp.ksplit_log2 ? unit_w(pp.ksplit2_log2) : wa;
-    if (pp.seg_w % wa == 0 && pp.seg_w % wb == 0) break;
-    pp.col_step = 1; pp.col_first = 0; pp.seg_w = p->W;
-    pp.tile_step = sink->tile_step; pp.y0 = sink->tile_first * 8;
-    }
-    {   // table fold (parameter-block kernel only): worth its per-CTA build (n * 768 entries) from ~4 M pixel-samples up
-        const int step = pp.tile_step > 1 ? pp.tile_step : 1;
-        const long long work = (long long)pp.seg_w * ((pp.y1 - pp.y0 + step - 1) / step) * (p->s1 - p->s0);
-        pp.fold_tab = pp.int_fold && sc->byte_colours && !xr && work >= (4LL << 20);
-    }
+    int sms = 0;
+    if (device_attr(sc->device, cudaDevAttrMultiProcessorCount, &sms) != cudaSuccess || sms <= 0) sms = 148;
+    const PathLaunch pl = plan_path_launch<T>(pp, view, p, sink, xr != nullptr, sc->byte_colours,
+                                              sizeof(T) == 4 && sc->pkc_ok && !(p->schedule & 4) && !xr, sms);
     if (!sc->sched_dev) return fail(RT_ERR_INVALID, "scene has no scheduler counters (upload failed?)");
-    unsigned *sched = sc->sched_dev + 4 * (sc->sched_next.fetch_add(1u) % RT_SCHED_SLOTS);      // {next unit, warps done, CTAs resolved, -}
-    CU(launch_path<T>(view, pp, accum, reinterpret_cast<unsigned long long *>(stats), st,
-                      sizeof(T) == 4 && sc->pkc_ok && view.bvh.nodes == 0 && !(p->schedule & 4) && !xr ? &sc->pkc : nullptr, sched));
+    pp.sched = sc->sched_dev + 4 * (sc->sched_next.fetch_add(1u) % RT_SCHED_SLOTS);      // {next unit, warps done, CTAs resolved, -}
+    CU(launch_path<T>(view, pp, pl, accum, reinterpret_cast<unsigned long long *>(stats), st, &sc->pkc));
     return RT_OK;
 }
 
@@ -888,12 +924,8 @@ RT_EXPORT int rt_peer_wait(int device, const uint32_t *flags_dev, int32_t n, uin
                            int32_t *timed_out_dev, void *stream) {
     if (!flags_dev || n < 1 || n > 32) return fail(RT_ERR_INVALID, "bad arguments");
     CU(cudaSetDevice(device));
-    static int khz_cache[64] = {0};        // cudaDevAttrClockRate is a slow query: once per device
-    int khz = device >= 0 && device < 64 ? khz_cache[device] : 0;
-    if (khz == 0) {
-        CU(cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, device));
-        if (device >= 0 && device < 64) khz_cache[device] = khz;
-    }
+    int khz = 0;
+    CU(device_attr(device, cudaDevAttrClockRate, &khz));
     const long long cycles = (long long)(timeout_ms > 0 ? timeout_ms : 2000) * (long long)(khz > 0 ? khz : 2000000);
     CU(launch_peer_wait(flags_dev, n, epoch, cycles, timed_out_dev, S(stream)));
     return RT_OK;
@@ -1031,12 +1063,9 @@ static int wf_begin_t(rt_wavefront *wf, WaveDev<T> &w, PathDev<T> &pp, const rt_
     bind_wave<T>(w, wf->blob, (size_t)P, (size_t)wf->max_depth);
     w.P = (int)P; w.max_depth = wf->max_depth;
     w.W = p->W; w.H = p->H; w.y0 = p->y0; w.y1 = p->y1; w.s0 = p->s0; w.s1 = p->s1; w.max_bounces = p->max_bounces;
-    const double aspect = (double)p->W / (double)p->H;
-    const double half_h = std::tan((p->fov_deg * (M_PI / 180.0)) / 2), half_w = half_h * aspect;
-    for (int k = 0; k < 3; ++k) { w.cam[k] = (T)p->cam[k]; pp.cam[k] = (T)p->cam[k]; }
-    w.aspect = pp.aspect = (T)aspect; w.half_w = pp.half_w = (T)half_w; w.half_h = pp.half_h = (T)half_h;
-    pp.W = p->W; pp.H = p->H;
-    pp.inv_W = (T)(1.0 / (double)p->W); pp.inv_H = (T)(1.0 / (double)p->H);
+    path_camera(pp, p);
+    for (int k = 0; k < 3; ++k) w.cam[k] = pp.cam[k];
+    w.aspect = pp.aspect; w.half_w = pp.half_w; w.half_h = pp.half_h;
     w.mirror_threshold = (T)p->mirror_threshold; w.fb_prob = (T)fb_prob;
     w.k0 = (uint32_t)p->seed; w.k1 = (uint32_t)(p->seed >> 32);
     CU(launch_wf_begin<T>(w, pp, reinterpret_cast<unsigned long long *>(stats), st));

@@ -26,19 +26,6 @@ template <typename T> struct Staged {
     LightsB<T> lb;
 };
 
-template <typename T> __host__ __device__ inline size_t align32(size_t x) { return (x + 31) & ~size_t(31); }
-
-// bytes of dynamic shared memory the staged scene needs (host + device agree on the layout)
-template <typename T> __host__ __device__ inline size_t scene_smem_bytes(int n, int nG, int nP, int nL) {
-    const size_t v = sizeof(typename M<T>::v4);
-    size_t b = 0;
-    b += (2 * (size_t)((n + 7) & ~7) + 2 * (size_t)n) * v;  // sph (padded to 8), pk (sphere pairs), mat, col
-    b += 2 * (size_t)nG * v + 2 * (size_t)nP * v + 2 * (size_t)nL * v + RT_LPK_STRIDE * (size_t)((nL + 1) / 2) * v;
-    b = align32<T>(b);
-    b += sizeof(int) * ((size_t)n + nG + 2 * (size_t)nP + nL);
-    return align32<T>(b);
-}
-
 template <typename T> RT_DEV void coop_copy(T *dst, const T *src, int count) {
     for (int i = threadIdx.x; i < count; i += blockDim.x) dst[i] = src[i];
 }
@@ -473,8 +460,7 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     const unsigned u_ = fine ? unit - n_coarse : unit;
     const int lk = fine ? pp.ksplit2_log2 : pp.ksplit_log2, kk = 1 << lk;
     const int gx_ = fine ? pp.gx2 : pp.gx, stripe0 = fine ? pp.stripe2 : 0;
-    const int pw_sh = lk == 0 ? 3 : lk == 1 ? 3 : lk == 2 ? 2 : lk <= 4 ? 1 : 0;
-    const int ph_sh = (5 - lk) - pw_sh;
+    const int pw_sh = unit_pw_log2(lk), ph_sh = (5 - lk) - pw_sh;
     const int sub = lane_ & (kk - 1), pl = lane_ >> lk;
     // CTA rows: cth = 2 << ph_sh of them; tile_step > 1: this launch owns every tile_step-th 8-row stripe from y0
     const int cth_sh = ph_sh + 1, cps_sh = 3 - cth_sh;                 // CTA rows per stripe = 1 << cps_sh
@@ -1445,22 +1431,9 @@ __global__ void __maxnreg__(RT_ENV_REGS) env_step_kernel(SceneDev<T> sc, EnvDev<
 }
 
 // ------------------------------------------------------------------ launchers
-template <typename T> static inline size_t smem_for(const SceneDev<T> &sc) {
-    return scene_smem_bytes<T>(sc.n, sc.nG, sc.nP, sc.nL);
-}
-
-#define RT_SMEM_LIMIT (96 * 1024)
-
 template <typename K> static cudaError_t allow_smem(K kernel, size_t bytes) {
     if (bytes > 48 * 1024) return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     return cudaSuccess;
-}
-
-// kMode for a scene: shared-memory staging when it fits, hierarchy code only when a hierarchy exists
-template <typename T> static inline int mode_for(const SceneDev<T> &sc, size_t extra_smem = 0) {
-    const bool shared = smem_for(sc) + extra_smem <= RT_SMEM_LIMIT;
-    if (!shared) return 2;
-    return sc.bvh.nodes > 0 ? 1 : 0;
 }
 
 #define RT_DISPATCH_MODE(mode, KERNEL, grid, block, smem_bytes, st, ...)                                       \
@@ -1542,66 +1515,33 @@ cudaError_t launch_whitted(const SceneDev<T> &sc, const WhittedDev<T> &wp, void 
 }
 
 template <typename T>
-cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, void *accum, unsigned long long *stats,
-                        cudaStream_t st, const PkConst *pkc, unsigned *sched) {
-    const int rows = pp.y1 - pp.y0;
-    if (rows <= 0 || pp.W <= 0) return cudaSuccess;
-    const int tiles = (rows + 7) / 8, step = pp.tile_step > 1 ? pp.tile_step : 1;
-    const int lk = pp.ksplit_log2;
-    const int pw_sh = lk == 0 ? 3 : lk == 1 ? 3 : lk == 2 ? 2 : lk <= 4 ? 1 : 0, ph_sh = (5 - lk) - pw_sh;
-    const int ctw = 4 << pw_sh, cth = 2 << ph_sh;
-    // stripes of 8 rows (8 / cth CTA rows each); without interleaving the last stripe may be cut short
-    const unsigned gy = step > 1 ? (unsigned)((tiles + step - 1) / step) * (8 / cth) : (unsigned)((rows + cth - 1) / cth);
-    PathDev<T> ppl = pp;                                          // + the tile grid the persistent CTAs walk
-    ppl.gx = (pp.seg_w + ctw - 1) / ctw; ppl.gy = (int)gy;         // seg_w = W unless the launch holds one column segment per stripe
-    ppl.gx2 = ppl.gy2 = ppl.stripe2 = 0;
-    // fine grid over the last owned stripes (see path_kernel): at most half of them, whole 8-row stripes
-    const int lk2 = pp.ksplit2_log2;
-    if (lk2 > lk && lk2 <= 5 && pp.fine_pixels > 0) {
-        const int owned = (tiles + step - 1) / step;                              // 8-row stripes of this launch
-        int fs = (int)(((long long)pp.fine_pixels + 8LL * pp.seg_w - 1) / (8LL * pp.seg_w));
-        if (fs > owned / 2) fs = owned / 2;
-        if (fs >= 1) {
-            const int pw2 = lk2 == 0 ? 3 : lk2 == 1 ? 3 : lk2 == 2 ? 2 : lk2 <= 4 ? 1 : 0, ph2 = (5 - lk2) - pw2;
-            const int ctw2 = 4 << pw2, cth2 = 2 << ph2;
-            const int sb = owned - fs, rows_a = sb * 8;                            // (tile_step == 1: rows of the coarse part)
-            ppl.stripe2 = sb;
-            ppl.gy = step > 1 ? sb * (8 / cth) : (rows_a + cth - 1) / cth;
-            ppl.gx2 = (pp.seg_w + ctw2 - 1) / ctw2;
-            ppl.gy2 = step > 1 ? fs * (8 / cth2) : (rows - rows_a + cth2 - 1) / cth2;
-        }
-    }
-    ppl.sched = sched;
-    const long long tiles_total = (long long)ppl.gx * ppl.gy + (long long)ppl.gx2 * ppl.gy2;
+cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathLaunch &pl, void *accum,
+                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc) {
+    if (pp.y1 <= pp.y0 || pp.W <= 0) return cudaSuccess;
+    const long long tiles_total = (long long)pp.gx * pp.gy + (long long)pp.gx2 * pp.gy2;
     dim3 grid(1), block(256);
     using v4 = typename M<T>::v4;
-    const size_t extra = 256 * sizeof(double);                   // div255 table of the integer fold
-    int mode = mode_for(sc, extra);
-    // small brute-force FP32 scenes: sphere pairs through the parameter block (kMode 3)
-    if (mode == 0 && sizeof(T) == 4 && pkc && ((sc.n + 7) & ~7) <= RT_PKC_MAX && sc.nL <= RT_LPKC_MAX) mode = 3;
-    if (mode != 3 || !pp.int_fold) ppl.fold_tab = 0;
-    // kMode 3 uses static shared arrays; its dynamic part is the fold table [n][3][256] bytes
-    const size_t sm = mode == 3 ? (ppl.fold_tab ? (size_t)sc.n * 768 : 0) : (mode != 2 ? smem_for(sc) : 0) + extra;
+    const size_t sm = pl.smem;
     cudaError_t e = cudaSuccess;
 #define RT_PATH_CASE(M_, F_)                                                                                       \
     { e = allow_smem(path_kernel<T, M_, F_>, sm); if (e != cudaSuccess) return e;                                  \
       grid.x = persistent_ctas(path_kernel<T, M_, F_>, sm, tiles_total);                                           \
       if (pp.max_ctas > 0 && grid.x > (unsigned)pp.max_ctas) grid.x = (unsigned)pp.max_ctas;                        \
-      path_kernel<T, M_, F_><<<grid, block, sm, st>>>(sc, ppl, (v4 *)accum, stats, PkNone()); }
-    if (mode == 3) {
+      path_kernel<T, M_, F_><<<grid, block, sm, st>>>(sc, pp, (v4 *)accum, stats, PkNone()); }
+    if (pl.mode == 3) {
         if constexpr (sizeof(T) == 4) {
 #define RT_PATH_CASE3(F_)                                                                                          \
     { e = allow_smem(path_kernel<T, 3, F_>, sm ? sm + 8192 : 0); /* + the static arrays: opt in above 48 KB in all */ \
       if (e != cudaSuccess) return e;                                                                              \
       grid.x = persistent_ctas(path_kernel<T, 3, F_>, sm, tiles_total);                                            \
       if (pp.max_ctas > 0 && grid.x > (unsigned)pp.max_ctas) grid.x = (unsigned)pp.max_ctas;                        \
-      path_kernel<T, 3, F_><<<grid, block, sm, st>>>(sc, ppl, (v4 *)accum, stats, *pkc); }
+      path_kernel<T, 3, F_><<<grid, block, sm, st>>>(sc, pp, (v4 *)accum, stats, *pkc); }
             if (pp.int_fold) RT_PATH_CASE3(true) else RT_PATH_CASE3(false)
 #undef RT_PATH_CASE3
         }
         return cudaGetLastError();
     }
-    const int variant = mode * 2 + (pp.int_fold ? 1 : 0);
+    const int variant = pl.mode * 2 + (pp.int_fold ? 1 : 0);
     switch (variant) {
         case 0: RT_PATH_CASE(0, false) break;   case 1: RT_PATH_CASE(0, true) break;
         case 2: RT_PATH_CASE(1, false) break;   case 3: RT_PATH_CASE(1, true) break;
@@ -1724,8 +1664,8 @@ cudaError_t launch_env_step(const SceneDev<T> &sc, const EnvDev<T> &e, const flo
 #define RT_INSTANTIATE_LAUNCHERS(T)                                                                                     \
     template cudaError_t launch_whitted<T>(const SceneDev<T> &, const WhittedDev<T> &, void *, int *,                   \
                                            unsigned long long *, cudaStream_t, unsigned *, unsigned *, unsigned *);     \
-    template cudaError_t launch_path<T>(const SceneDev<T> &, const PathDev<T> &, void *, unsigned long long *,          \
-                                        cudaStream_t, const PkConst *, unsigned *);                                     \
+    template cudaError_t launch_path<T>(const SceneDev<T> &, const PathDev<T> &, const PathLaunch &, void *,           \
+                                        unsigned long long *, cudaStream_t, const PkConst *);                           \
     template cudaError_t launch_resolve<T>(const void *, int, int, int, int, float *, cudaStream_t);                    \
     template cudaError_t launch_trajectories<T>(const SceneDev<T> &, int, int, int, uint64_t, float *, float *, float *,  \
                                                 float *, uint8_t *, int *, uint8_t *, unsigned long long *, cudaStream_t); \

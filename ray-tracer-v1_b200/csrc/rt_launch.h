@@ -23,19 +23,25 @@ template <typename T> struct WhittedDev {
     unsigned *sched2;            // pass 2: {next unit, warps done}
 };
 
-// Algorithm B frame (rt_path_params)
+// Path-kernel work unit with 2^lk lanes per pixel: one warp traces a 2^pw x 2^ph pixel block, pw = unit_pw_log2(lk) and
+// ph = (5 - lk) - pw (8x4, 8x2, 4x2, 2x2, 2x1, 1x1 for lk = 0..5), and a CTA of 4 x 2 warps a (4 << pw) x (2 << ph) one
+__host__ __device__ constexpr int unit_pw_log2(int lk) { return lk == 0 ? 3 : lk == 1 ? 3 : lk == 2 ? 2 : lk <= 4 ? 1 : 0; }
+
+// Algorithm B frame (rt_path_params).  The launch geometry -- ksplit_log2, ksplit2_log2, the tile grids, the band
+// (y0, tile_step, col_*, seg_w) and fold_tab -- is set by plan_path_launch (rt_api.cu).
 template <typename T> struct PathDev {
     T cam[3];
     int W, H, y0, y1, s0, s1, max_bounces;
     T aspect, half_w, half_h;    // W/H, tan(fov/2)*aspect, tan(fov/2)   (chandelier.py:412-415)
     T inv_W, inv_H;              // product build: 1/W, 1/H (the parity build divides like the reference)
     T mirror_threshold;
-    int gx, gy;                          // tile grid of the launch (set by launch_path)
+    int gx, gy;                          // tile grid of the launch
     // second ("fine") tile grid over the last owned stripes of the launch: same pixels-per-CTA logic with MORE lanes per
     // pixel (ksplit2_log2 > ksplit_log2), i.e. work units a quarter as long, handed out after the coarse ones so that
-    // the drain at the end of the launch is a quarter as long (gx2 * gy2 = 0: none).  Set by launch_path from
-    // ksplit2_log2 / fine_pixels, which the API fills in.
-    int gx2, gy2, stripe2, ksplit2_log2, fine_pixels;
+    // the drain at the end of the launch is a quarter as long (gx2 * gy2 = 0: none)
+    int gx2, gy2, stripe2, ksplit2_log2;
+    int depth0;                          // explicit rays (below); placed here because moving the fields after it by 8
+                                         // bytes changes the instruction schedule ptxas picks for path_kernel
     unsigned *sched;                     // {next work unit, warps done}: zero between launches (self-resetting)
     uint32_t k0, k1;
     uint32_t rk[20];                     // Philox round keys k0 + r*W0, k1 + r*W1 (constant-bank operands of the rounds)
@@ -64,7 +70,6 @@ template <typename T> struct PathDev {
     // the Philox stream of pixel ray_ids[i] (or i).  W = n, H = 1.  Not available in the parameter-block kernel (kMode 3).
     const double *rays;
     const int *ray_ids;
-    int depth0;
 };
 
 // "Algorithm C" frame (rt_simple_params)
@@ -101,16 +106,43 @@ template <typename T> struct EnvDev {
     double *total;
 };
 
+template <typename T> __host__ __device__ inline size_t align32(size_t x) { return (x + 31) & ~size_t(31); }
+
+// bytes of dynamic shared memory the staged scene needs (host + device agree on the layout)
+template <typename T> __host__ __device__ inline size_t scene_smem_bytes(int n, int nG, int nP, int nL) {
+    const size_t v = sizeof(typename M<T>::v4);
+    size_t b = 0;
+    b += (2 * (size_t)((n + 7) & ~7) + 2 * (size_t)n) * v;  // sph (padded to 8), pk (sphere pairs), mat, col
+    b += 2 * (size_t)nG * v + 2 * (size_t)nP * v + 2 * (size_t)nL * v + RT_LPK_STRIDE * (size_t)((nL + 1) / 2) * v;
+    b = align32<T>(b);
+    b += sizeof(int) * ((size_t)n + nG + 2 * (size_t)nP + nL);
+    return align32<T>(b);
+}
+template <typename T> static inline size_t smem_for(const SceneDev<T> &sc) {
+    return scene_smem_bytes<T>(sc.n, sc.nG, sc.nP, sc.nL);
+}
+
+#define RT_SMEM_LIMIT (96 * 1024)
+
+// kMode for a scene: shared-memory staging when it fits, hierarchy code only when a hierarchy exists
+template <typename T> static inline int mode_for(const SceneDev<T> &sc, size_t extra_smem = 0) {
+    const bool shared = smem_for(sc) + extra_smem <= RT_SMEM_LIMIT;
+    if (!shared) return 2;
+    return sc.bvh.nodes > 0 ? 1 : 0;
+}
+
 template <typename T>
 cudaError_t launch_whitted(const SceneDev<T> &sc, const WhittedDev<T> &wp, void *accum, int *hit,
                            unsigned long long *stats, cudaStream_t st, unsigned *sched, unsigned *sched2 = nullptr,
                            unsigned *heavy = nullptr);
 // sched2 / heavy non-NULL: the caller allows the two-pass schedule (exact only for integer-valued colours: it adds the
 // samples of a pixel with FP32 reductions in no fixed order)
+// kernel variant (kMode) and dynamic shared memory of a path-kernel launch (plan_path_launch, rt_api.cu)
+struct PathLaunch { int mode; size_t smem; };
 template <typename T>
-cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, void *accum, unsigned long long *stats,
-                        cudaStream_t st, const PkConst *pkc, unsigned *sched);
-// pkc: host copy of the FP32 pair arrays (small scenes) or NULL; sched: two zeroed device counters owned by this launch
+cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathLaunch &pl, void *accum,
+                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc);
+// pkc: host copy of the FP32 pair arrays, read by kMode 3; pp.sched: two zeroed device counters owned by this launch
 template <typename T>
 cudaError_t launch_trajectories(const SceneDev<T> &sc, int n_traj, int max_steps, int max_bounces, uint64_t seed, float *obs,
                                 float *action, float *next_obs, float *reward, uint8_t *hit, int *length,
