@@ -181,6 +181,13 @@ typedef struct rt_path_params {
  * [5] sphere tests, [6] AABB tests (LBVH only). */
 int rt_render_path(rt_scene *scene, int precision, const rt_path_params *p, void *accum_dev, uint64_t *stats_dev,
                    void *stream);
+/* rt_render_path that also stores the second moments of every pixel's samples: moments_dev [H,W,4] double =
+ * (sum r^2, sum g^2, sum b^2, n) over the sample range of the launch, with the squares of the same folded integer
+ * colours accum_dev sums (exact: integer colours <= 65535 are squared and summed in 64-bit integers, non-integer
+ * colours in double).  p->accumulate adds into moments_dev as into accum_dev.  accum_dev and stats_dev are
+ * bit-identical to rt_render_path's. */
+int rt_render_path_moments(rt_scene *scene, int precision, const rt_path_params *p, void *accum_dev,
+                           double *moments_dev, uint64_t *stats_dev, void *stream);
 /* TraditionalRenderer.trace_ray_traditional(ray, bounce_count) (FB/fb_vs_traditional_chandelier.py:431-521) for n
  * explicit rays at once: rays_dev [n,6] doubles = origin, direction AS GIVEN (Ray() has normalised it); the path starts
  * at recursion depth bounce_count (a call with bounce_count >= max_bounces returns (2,2,5)); ray i draws its bounce
@@ -194,6 +201,11 @@ int rt_trace_paths(rt_scene *scene, int precision, const rt_path_params *p, int3
  * rows [y0,y1) only. */
 int rt_resolve(int device, int precision, const void *accum_dev, int32_t W, int32_t H, int32_t y0, int32_t y1,
                int32_t spp, float *image_dev, void *stream);
+/* accum [H,W,4] (float / double per precision) and moments [H,W,4] double -> var [H,W,3] float32 = the variance of
+ * each pixel's mean in colour levels^2 (0-255 scale), (Q - S^2/n) / (n(n-1)) with S = sum, Q = sum of squares, n = the
+ * sample count; 0 where n < 2.  Rows [y0,y1) only. */
+int rt_resolve_variance(int device, int precision, const void *accum_dev, const double *moments_dev, int32_t W,
+                        int32_t H, int32_t y0, int32_t y1, float *var_dev, void *stream);
 
 /* ---- "Algorithm C" frame: SimplifiedFBRenderer.render_original_style / trace_ray_simple /
  *      calculate_lighting_exact_original in traditional mode (fb_usage_prob = 0): FB/output6.py:197-306, :434-654.
@@ -256,6 +268,9 @@ int rt_wf_trace(rt_wavefront *wf, float *obs_dev, uint8_t *need_dev, uint64_t *s
 int rt_wf_bounce(rt_wavefront *wf, const uint8_t *need_dev, const float *actions_dev, uint64_t *stats_dev, int32_t *live_dev,
                  void *stream);
 int rt_wf_finish(rt_wavefront *wf, void *accum_dev, void *stream);
+/* rt_wf_finish that also adds c^2 per channel and 1 to the count of moments_dev [H,W,4] double, as
+ * rt_render_path_moments stores them. */
+int rt_wf_finish_moments(rt_wavefront *wf, void *accum_dev, double *moments_dev, void *stream);
 
 /* ---- fused multi-GPU sinks for Algorithm B frames (SURVEY.md 8e) ---------------------------------------------
  * One process per GPU; a rank's path kernel stores its result where it is needed -- its own accumulators, the

@@ -122,14 +122,17 @@ SIGNATURES = {
     "rt_terminal_rgb": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int, vp, vp]),
     "rt_render_whitted": (C.c_int, [vp, C.c_int, C.POINTER(WhittedParams), vp, vp, vp, vp]),
     "rt_render_path": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), vp, vp, vp]),
+    "rt_render_path_moments": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), vp, vp, vp, vp]),
     "rt_trace_paths": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), C.c_int32, vp, vp, C.c_int32, vp, vp, vp]),
     "rt_resolve": (C.c_int, [C.c_int, C.c_int, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
+    "rt_resolve_variance": (C.c_int, [C.c_int, C.c_int, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
     "rt_wf_create": (C.c_int, [vp, C.c_int, C.c_int32, C.c_int32, C.POINTER(vp)]),
     "rt_wf_destroy": (C.c_int, [vp]),
     "rt_wf_begin": (C.c_int, [vp, C.POINTER(PathParams), C.c_double, vp, vp]),
     "rt_wf_trace": (C.c_int, [vp, vp, vp, vp, vp]),
     "rt_wf_bounce": (C.c_int, [vp, vp, vp, vp, vp, vp]),
     "rt_wf_finish": (C.c_int, [vp, vp, vp]),
+    "rt_wf_finish_moments": (C.c_int, [vp, vp, vp, vp]),
     "rt_generate_trajectories": (C.c_int, [vp, C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_uint64, vp, vp, vp, vp, vp, vp, vp,
                                             vp, vp]),
     "rt_render_simple": (C.c_int, [vp, C.c_int, C.POINTER(SimpleParams), vp, vp, vp, vp]),
@@ -454,8 +457,14 @@ class DeviceScene:
         """Asynchronous launch into device buffers (accum [H,W,4] of the precision's float type)."""
         check(lib().rt_render_whitted(self.handle, precision, C.byref(params), _ptr(accum), _ptr(hit), _ptr(stats), stream))
 
-    def render_path(self, params, accum, precision=F32, stats=None, stream=None):
-        check(lib().rt_render_path(self.handle, precision, C.byref(params), _ptr(accum), _ptr(stats), stream))
+    def render_path(self, params, accum, precision=F32, stats=None, stream=None, moments=None):
+        """Asynchronous launch into device buffers.  ``moments`` (float64 [H,W,4], optional) also receives the sums of
+        the squared sample colours and the sample count (``rt_render_path_moments``); accum and stats are the same."""
+        if moments is None:
+            check(lib().rt_render_path(self.handle, precision, C.byref(params), _ptr(accum), _ptr(stats), stream))
+        else:
+            check(lib().rt_render_path_moments(self.handle, precision, C.byref(params), _ptr(accum), _ptr(moments),
+                                               _ptr(stats), stream))
 
     def trace_paths(self, rays, max_bounces, mirror_threshold, bounce_count=0, seed=0, ray_ids=None, samples=(0, 1),
                     precision=F64):
@@ -480,6 +489,13 @@ class DeviceScene:
         y0, y1 = (0, H) if rows is None else rows
         check(lib().rt_resolve(self.device, precision, _ptr(accum), int(W), int(H), int(y0), int(y1), int(spp),
                                _ptr(image), stream))
+
+    def resolve_variance(self, accum, moments, W, H, var, precision=F32, rows=None, stream=None):
+        """accum [H,W,4] + moments [H,W,4] float64 -> var [H,W,3] float32: the variance of each pixel's mean in colour
+        levels^2 (0 where a pixel has fewer than two samples), rows [y0, y1) only."""
+        y0, y1 = (0, H) if rows is None else rows
+        check(lib().rt_resolve_variance(self.device, precision, _ptr(accum), _ptr(moments), int(W), int(H), int(y0), int(y1),
+                                        _ptr(var), stream))
 
     def render_whitted_host(self, params, precision=F32, want_accum=True, want_hit=True):
         """Host-buffer entry: -> (image [H,W,3] f32, sums [H,W,4], hit [H,W] i32, stats u64[8])."""

@@ -345,7 +345,7 @@ static inline cudaStream_t S(void *stream) { return reinterpret_cast<cudaStream_
 
 // ------------------------------------------------------------------ library / device
 RT_EXPORT const char *rt_last_error(void) { return g_err.c_str(); }
-RT_EXPORT int rt_version(void) { return 100; }
+RT_EXPORT int rt_version(void) { return 101; }
 
 RT_EXPORT int rt_device_count(int *count) {
     if (!count) return fail(RT_ERR_INVALID, "count is NULL");
@@ -749,7 +749,8 @@ static PathLaunch plan_path_launch(PathDev<T> &pp, const SceneDev<T> &sc, const 
 
 template <typename T>
 static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_path_params *p, void *accum, uint64_t *stats,
-                         cudaStream_t st, const rt_path_sink *sink = nullptr, const ExplicitRays *xr = nullptr) {
+                         cudaStream_t st, const rt_path_sink *sink = nullptr, const ExplicitRays *xr = nullptr,
+                         double *moments = nullptr) {
     // bit 1: no camera-ray candidate lists, bit 2: no parameter-block kernel (include/rt_b200.h)
     if (p->schedule & ~6) return fail(RT_ERR_INVALID, "unknown schedule bits");
     PathDev<T> pp;
@@ -817,7 +818,7 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
                                               sizeof(T) == 4 && sc->pkc_ok && !(p->schedule & 4) && !xr, sms);
     if (!sc->sched_dev) return fail(RT_ERR_INVALID, "scene has no scheduler counters (upload failed?)");
     pp.sched = sc->sched_dev + 4 * (sc->sched_next.fetch_add(1u) % RT_SCHED_SLOTS);      // {next unit, warps done, CTAs resolved, -}
-    CU(launch_path<T>(view, pp, pl, accum, reinterpret_cast<unsigned long long *>(stats), st, &sc->pkc));
+    CU(launch_path<T>(view, pp, pl, accum, reinterpret_cast<unsigned long long *>(stats), st, &sc->pkc, moments));
     return RT_OK;
 }
 
@@ -830,6 +831,18 @@ RT_EXPORT int rt_render_path(rt_scene *scene, int precision, const rt_path_param
     CU(cudaSetDevice(scene->device));
     if (precision == RT_F64) return render_path_t<double>(scene, scene->d.view, p, accum_dev, stats_dev, S(stream));
     if (precision == RT_F32) return render_path_t<float>(scene, scene->f.view, p, accum_dev, stats_dev, S(stream));
+    return fail(RT_ERR_INVALID, "unknown precision");
+}
+
+RT_EXPORT int rt_render_path_moments(rt_scene *scene, int precision, const rt_path_params *p, void *accum_dev,
+                                     double *moments_dev, uint64_t *stats_dev, void *stream) {
+    if (!scene || !p || !accum_dev || !moments_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    int rc = check_band(p->W, p->H, p->y0, p->y1, p->s0, p->s1);
+    if (rc) return rc;
+    if (p->max_bounces > RT_PATH_MAX_DEPTH) return fail(RT_ERR_UNSUPPORTED, "max_bounces above 32 is not supported by the path kernel");
+    CU(cudaSetDevice(scene->device));
+    if (precision == RT_F64) return render_path_t<double>(scene, scene->d.view, p, accum_dev, stats_dev, S(stream), nullptr, nullptr, moments_dev);
+    if (precision == RT_F32) return render_path_t<float>(scene, scene->f.view, p, accum_dev, stats_dev, S(stream), nullptr, nullptr, moments_dev);
     return fail(RT_ERR_INVALID, "unknown precision");
 }
 
@@ -940,6 +953,18 @@ RT_EXPORT int rt_resolve(int device, int precision, const void *accum_dev, int32
     CU(cudaSetDevice(device));
     if (precision == RT_F64) CU(launch_resolve<double>(accum_dev, W, y0, y1, spp, image_dev, S(stream)));
     else if (precision == RT_F32) CU(launch_resolve<float>(accum_dev, W, y0, y1, spp, image_dev, S(stream)));
+    else return fail(RT_ERR_INVALID, "unknown precision");
+    return RT_OK;
+}
+
+RT_EXPORT int rt_resolve_variance(int device, int precision, const void *accum_dev, const double *moments_dev, int32_t W,
+                                  int32_t H, int32_t y0, int32_t y1, float *var_dev, void *stream) {
+    if (!accum_dev || !moments_dev || !var_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    int rc = check_band(W, H, y0, y1, 0, 0);
+    if (rc) return rc;
+    CU(cudaSetDevice(device));
+    if (precision == RT_F64) CU(launch_resolve_variance<double>(accum_dev, moments_dev, W, y0, y1, var_dev, S(stream)));
+    else if (precision == RT_F32) CU(launch_resolve_variance<float>(accum_dev, moments_dev, W, y0, y1, var_dev, S(stream)));
     else return fail(RT_ERR_INVALID, "unknown precision");
     return RT_OK;
 }
@@ -1105,14 +1130,23 @@ RT_EXPORT int rt_wf_bounce(rt_wavefront *wf, const uint8_t *need_dev, const floa
     return RT_OK;
 }
 
-RT_EXPORT int rt_wf_finish(rt_wavefront *wf, void *accum_dev, void *stream) {
-    if (!wf || !accum_dev) return fail(RT_ERR_INVALID, "NULL argument");
+static int wf_finish(rt_wavefront *wf, void *accum_dev, double *moments_dev, void *stream) {
     if (!wf->begun) return fail(RT_ERR_INVALID, "rt_wf_begin has not been called");
     CU(cudaSetDevice(wf->scene->device));
-    if (wf->precision == RT_F64) CU(launch_wf_finish<double>(wf->scene->d.view, wf->d, accum_dev, S(stream)));
-    else CU(launch_wf_finish<float>(wf->scene->f.view, wf->f, accum_dev, S(stream)));
+    if (wf->precision == RT_F64) CU(launch_wf_finish<double>(wf->scene->d.view, wf->d, accum_dev, moments_dev, S(stream)));
+    else CU(launch_wf_finish<float>(wf->scene->f.view, wf->f, accum_dev, moments_dev, S(stream)));
     wf->begun = false;
     return RT_OK;
+}
+
+RT_EXPORT int rt_wf_finish(rt_wavefront *wf, void *accum_dev, void *stream) {
+    if (!wf || !accum_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    return wf_finish(wf, accum_dev, nullptr, stream);
+}
+
+RT_EXPORT int rt_wf_finish_moments(rt_wavefront *wf, void *accum_dev, double *moments_dev, void *stream) {
+    if (!wf || !accum_dev || !moments_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    return wf_finish(wf, accum_dev, moments_dev, stream);
 }
 
 // ------------------------------------------------------------------ FB training trajectories

@@ -340,10 +340,15 @@ template <typename T> RT_DEV V3<T> path_camera_ray(const PathDev<T> &pp, int x, 
 // s+1 together.  Everything outside the sphere loop (camera ray, Philox, fold) runs once per sample at full lane
 // occupancy.
 // kIntFold: integer fold through the div255 table (all leaf colours integer-valued), else the double-division fold.
-template <typename T, int kMode, bool kIntFold>
+// kMoments: also store the second moments of the pixel's samples, moments[o] = (sum r^2, sum g^2, sum b^2, n) (the
+// trailing parameter is empty otherwise, so the plain kernels keep their parameter offsets).  Exact: an integer-fold
+// colour is <= 65535, so its square fits a uint32 and a uint64 sum of 65536 of them stays below 2^53; the double fold
+// sums its squares in double.
+template <typename T, int kMode, bool kIntFold, bool kMoments>
 __global__ void __launch_bounds__(256, (sizeof(T) == 4 ? (kMode == 3 ? RT_PATH_MIN_BLOCKS_PKC : RT_PATH_MIN_BLOCKS) : 1))
 path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned long long *stats,
-            const __grid_constant__ typename std::conditional<kMode == 3, PkConst, PkNone>::type pkc) {
+            const __grid_constant__ typename std::conditional<kMode == 3, PkConst, PkNone>::type pkc,
+            typename std::conditional<kMoments, double4 *, PkNone>::type moments) {
     RT_MODE_DECL;
     using PK = typename std::conditional<kMode == 3, PkConst, PkNone>::type;
     extern __shared__ __align__(32) unsigned char smem[];
@@ -477,6 +482,7 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     const uint32_t pixel = (uint32_t)(y * pp.W + x);
     // integer-valued sums: exact in uint32 (int fold: colours <= 65535, samples per launch <= 65536) / in double
     typename std::conditional<kIntFold, unsigned, double>::type a0 = 0, a1 = 0, a2 = 0;
+    typename std::conditional<kIntFold, unsigned long long, double>::type q0 = 0, q1 = 0, q2 = 0;     // kMoments: squares
     // primary rays of this warp tile: spheres its cone of camera rays can touch (cone_candidates, rt_trace.cuh)
     unsigned long long cand = ~0ull;
     bool first_trip = false;                          // warp-uniform: every live lane is about to trace its camera ray
@@ -497,6 +503,7 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
         const int mine = has_pixel ? (ns - sub + kk - 1) >> lk : 0;      // samples of this lane
         n_rays += (unsigned)mine;
         a0 = 2 * mine; a1 = 2 * mine; a2 = 5 * mine;
+        if constexpr (kMoments) { q0 = 4 * mine; q1 = 4 * mine; q2 = 25 * mine; }
     } else {
         int s = pp.s0 + sub, depth = 0;
         bool alive = has_pixel && s < pp.s1;          // lane has a path in flight
@@ -619,10 +626,16 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                     fold_path_int<T, kMode == 3>(S.g, st, depth, div255, c, fold_from, s_base + 32u * RT_PKC_MAX,
                                                  (kMode == 3 && pp.fold_tab) ? (unsigned)__cvta_generic_to_shared(smem) : 0u);
                     a0 += (unsigned)c[0]; a1 += (unsigned)c[1]; a2 += (unsigned)c[2];
+                    if constexpr (kMoments) {
+                        q0 += (unsigned long long)((unsigned)c[0] * (unsigned)c[0]);
+                        q1 += (unsigned long long)((unsigned)c[1] * (unsigned)c[1]);
+                        q2 += (unsigned long long)((unsigned)c[2] * (unsigned)c[2]);
+                    }
                 } else {
                     double c[3] = {lf0, lf1, lf2};
                     fold_path<T, kMode == 3>(S.g, st, depth, c, fold_from);
                     a0 += c[0]; a1 += c[1]; a2 += c[2];
+                    if constexpr (kMoments) { q0 += __dmul_rn(c[0], c[0]); q1 += __dmul_rn(c[1], c[1]); q2 += __dmul_rn(c[2], c[2]); }
                 }
             }
             s += kk;
@@ -635,6 +648,10 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
         for (int o = 1; o < kk; o <<= 1) {
             a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o);
             a2 += __shfl_xor_sync(0xffffffffu, a2, o);
+            if constexpr (kMoments) {
+                q0 += __shfl_xor_sync(0xffffffffu, q0, o); q1 += __shfl_xor_sync(0xffffffffu, q1, o);
+                q2 += __shfl_xor_sync(0xffffffffu, q2, o);
+            }
         }
     }
     if (has_pixel && ns > 0 && sub == 0) {
@@ -668,6 +685,14 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                 out.x += old.x; out.y += old.y; out.z += old.z; out.w += old.w;
             }
             accum[o] = out;
+            if constexpr (kMoments) {
+                double4 m = make_double4((double)q0, (double)q1, (double)q2, (double)ns);
+                if (pp.accumulate) {
+                    const double4 old = moments[o];
+                    m.x += old.x; m.y += old.y; m.z += old.z; m.w += old.w;
+                }
+                moments[o] = m;
+            }
         }
     }
     unsigned nxt = 0;
@@ -1019,6 +1044,30 @@ __global__ void resolve_kernel(const typename M<T>::v4 *accum, int W, int y0, in
     image[3 * o + 0] = (float)(r < 1.0 ? r : 1.0);
     image[3 * o + 1] = (float)(g < 1.0 ? g : 1.0);
     image[3 * o + 2] = (float)(b < 1.0 ? b : 1.0);
+}
+
+// variance of the pixel's mean in colour levels^2, from the sums S (accum) and the sums of squares Q (moments) of its n
+// samples: (Q - S^2/n) / (n (n-1)), evaluated as (n Q - S^2) / (n^2 (n-1)) -- the numerator is exact while n Q and S^2
+// stay below 2^53 (integer colours), so a pixel whose samples all agree gets exactly 0; 0 where n < 2
+template <typename T>
+__global__ void resolve_variance_kernel(const typename M<T>::v4 *accum, const double4 *moments, int W, int y0, int y1,
+                                        float *var) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t n = (size_t)(y1 - y0) * W;
+    if (i >= n) return;
+    const size_t o = (size_t)y0 * W + i;
+    const typename M<T>::v4 a = accum[o];
+    const double4 q = moments[o];
+    const double k = q.w, S[3] = {(double)a.x, (double)a.y, (double)a.z}, Q[3] = {q.x, q.y, q.z};
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        double v = 0.0;
+        if (k >= 2.0) {
+            v = __ddiv_rn(__dsub_rn(__dmul_rn(k, Q[c]), __dmul_rn(S[c], S[c])), __dmul_rn(__dmul_rn(k, k), k - 1.0));
+            v = v > 0.0 ? v : 0.0;
+        }
+        var[3 * o + c] = (float)v;
+    }
 }
 
 // ------------------------------------------------------------------ batched primitives
@@ -1516,26 +1565,29 @@ cudaError_t launch_whitted(const SceneDev<T> &sc, const WhittedDev<T> &wp, void 
 
 template <typename T>
 cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathLaunch &pl, void *accum,
-                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc) {
+                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, double *moments) {
     if (pp.y1 <= pp.y0 || pp.W <= 0) return cudaSuccess;
     const long long tiles_total = (long long)pp.gx * pp.gy + (long long)pp.gx2 * pp.gy2;
     dim3 grid(1), block(256);
     using v4 = typename M<T>::v4;
     const size_t sm = pl.smem;
     cudaError_t e = cudaSuccess;
-#define RT_PATH_CASE(M_, F_)                                                                                       \
-    { e = allow_smem(path_kernel<T, M_, F_>, sm); if (e != cudaSuccess) return e;                                  \
-      grid.x = persistent_ctas(path_kernel<T, M_, F_>, sm, tiles_total);                                           \
+    double4 *const mom = reinterpret_cast<double4 *>(moments);
+    // one launch of path_kernel<T, M_, F_, Q_>; SMOPT_: the shared memory to opt in to, PKC_: the parameter-block
+    // scene (kMode 3), MOM_: the moments buffer (Q_ = true)
+#define RT_PATH_LAUNCH(M_, F_, Q_, SMOPT_, PKC_, MOM_)                                                               \
+    { e = allow_smem(path_kernel<T, M_, F_, Q_>, SMOPT_); if (e != cudaSuccess) return e;                          \
+      grid.x = persistent_ctas(path_kernel<T, M_, F_, Q_>, sm, tiles_total);                                       \
       if (pp.max_ctas > 0 && grid.x > (unsigned)pp.max_ctas) grid.x = (unsigned)pp.max_ctas;                        \
-      path_kernel<T, M_, F_><<<grid, block, sm, st>>>(sc, pp, (v4 *)accum, stats, PkNone()); }
+      path_kernel<T, M_, F_, Q_><<<grid, block, sm, st>>>(sc, pp, (v4 *)accum, stats, PKC_, MOM_); }
+#define RT_PATH_CASE(M_, F_)                                                                                       \
+    { if (mom) RT_PATH_LAUNCH(M_, F_, true, sm, PkNone(), mom) else RT_PATH_LAUNCH(M_, F_, false, sm, PkNone(), PkNone()) }
     if (pl.mode == 3) {
         if constexpr (sizeof(T) == 4) {
+            // + the static arrays: opt in above 48 KB in all
 #define RT_PATH_CASE3(F_)                                                                                          \
-    { e = allow_smem(path_kernel<T, 3, F_>, sm ? sm + 8192 : 0); /* + the static arrays: opt in above 48 KB in all */ \
-      if (e != cudaSuccess) return e;                                                                              \
-      grid.x = persistent_ctas(path_kernel<T, 3, F_>, sm, tiles_total);                                            \
-      if (pp.max_ctas > 0 && grid.x > (unsigned)pp.max_ctas) grid.x = (unsigned)pp.max_ctas;                        \
-      path_kernel<T, 3, F_><<<grid, block, sm, st>>>(sc, pp, (v4 *)accum, stats, *pkc); }
+    { if (mom) RT_PATH_LAUNCH(3, F_, true, sm ? sm + 8192 : 0, *pkc, mom)                                          \
+      else RT_PATH_LAUNCH(3, F_, false, sm ? sm + 8192 : 0, *pkc, PkNone()) }
             if (pp.int_fold) RT_PATH_CASE3(true) else RT_PATH_CASE3(false)
 #undef RT_PATH_CASE3
         }
@@ -1548,6 +1600,7 @@ cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathL
         case 4: RT_PATH_CASE(2, false) break;   default: RT_PATH_CASE(2, true) break;
     }
 #undef RT_PATH_CASE
+#undef RT_PATH_LAUNCH
     return cudaGetLastError();
 }
 
@@ -1579,6 +1632,15 @@ cudaError_t launch_resolve(const void *accum, int W, int y0, int y1, int spp, fl
     const size_t n = (size_t)(y1 - y0) * W;
     if (n == 0) return cudaSuccess;
     resolve_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const typename M<T>::v4 *)accum, W, y0, y1, spp, image);
+    return cudaGetLastError();
+}
+
+template <typename T>
+cudaError_t launch_resolve_variance(const void *accum, const double *moments, int W, int y0, int y1, float *var, cudaStream_t st) {
+    const size_t n = (size_t)(y1 - y0) * W;
+    if (n == 0) return cudaSuccess;
+    resolve_variance_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const typename M<T>::v4 *)accum,
+                                                                          (const double4 *)moments, W, y0, y1, var);
     return cudaGetLastError();
 }
 
@@ -1665,8 +1727,9 @@ cudaError_t launch_env_step(const SceneDev<T> &sc, const EnvDev<T> &e, const flo
     template cudaError_t launch_whitted<T>(const SceneDev<T> &, const WhittedDev<T> &, void *, int *,                   \
                                            unsigned long long *, cudaStream_t, unsigned *, unsigned *, unsigned *);     \
     template cudaError_t launch_path<T>(const SceneDev<T> &, const PathDev<T> &, const PathLaunch &, void *,           \
-                                        unsigned long long *, cudaStream_t, const PkConst *);                           \
+                                        unsigned long long *, cudaStream_t, const PkConst *, double *);                 \
     template cudaError_t launch_resolve<T>(const void *, int, int, int, int, float *, cudaStream_t);                    \
+    template cudaError_t launch_resolve_variance<T>(const void *, const double *, int, int, int, float *, cudaStream_t); \
     template cudaError_t launch_trajectories<T>(const SceneDev<T> &, int, int, int, uint64_t, float *, float *, float *,  \
                                                 float *, uint8_t *, int *, uint8_t *, unsigned long long *, cudaStream_t); \
     template cudaError_t launch_simple<T>(const SceneDev<T> &, const SimpleDev<T> &, int4 *, float *,                   \

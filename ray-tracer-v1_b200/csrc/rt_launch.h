@@ -141,8 +141,9 @@ cudaError_t launch_whitted(const SceneDev<T> &sc, const WhittedDev<T> &wp, void 
 struct PathLaunch { int mode; size_t smem; };
 template <typename T>
 cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathLaunch &pl, void *accum,
-                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc);
-// pkc: host copy of the FP32 pair arrays, read by kMode 3; pp.sched: two zeroed device counters owned by this launch
+                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, double *moments);
+// pkc: host copy of the FP32 pair arrays, read by kMode 3; pp.sched: two zeroed device counters owned by this launch;
+// moments: NULL, or [H,W,4] doubles that receive (sum r^2, sum g^2, sum b^2, n) like accum (the kMoments kernels)
 template <typename T>
 cudaError_t launch_trajectories(const SceneDev<T> &sc, int n_traj, int max_steps, int max_bounces, uint64_t seed, float *obs,
                                 float *action, float *next_obs, float *reward, uint8_t *hit, int *length,
@@ -186,7 +187,10 @@ template <typename T>
 cudaError_t launch_wf_bounce(const WaveDev<T> &w, const uint8_t *need, const float *actions, unsigned long long *stats,
                              int *live_count, cudaStream_t st);
 template <typename T>
-cudaError_t launch_wf_finish(const SceneDev<T> &sc, const WaveDev<T> &w, void *accum, cudaStream_t st);
+cudaError_t launch_wf_finish(const SceneDev<T> &sc, const WaveDev<T> &w, void *accum, double *moments, cudaStream_t st);
+// variance of each pixel's mean from accum and moments (rt_resolve_variance): rows [y0, y1) of var [H,W,3]
+template <typename T>
+cudaError_t launch_resolve_variance(const void *accum, const double *moments, int W, int y0, int y1, float *var, cudaStream_t st);
 
 // FFMA issue-rate micro-benchmark (rt_f32.cu): `iters` trips of 16 independent FFMA per thread
 cudaError_t launch_fp32_peak(int blocks, int threads, int iters, float *sink, cudaStream_t st);

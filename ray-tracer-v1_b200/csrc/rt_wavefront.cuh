@@ -173,9 +173,11 @@ __global__ void __launch_bounds__(256) wf_bounce_kernel(WaveDev<T> w, const uint
     if ((threadIdx.x & 31) == 0 && live) atomicAdd(live_count, (int)live);
 }
 
-// fold (chandelier.py:509-521) in double with the true division (both builds), sums added to the pixel
-template <typename T>
-__global__ void __launch_bounds__(256) wf_finish_kernel(SceneDev<T> sc, WaveDev<T> w, typename M<T>::v4 *accum) {
+// fold (chandelier.py:509-521) in double with the true division (both builds), sums added to the pixel; kMoments: the
+// squares and the count go into moments [H,W,4] as well (double atomics: exact for integer-valued squares)
+template <typename T, bool kMoments>
+__global__ void __launch_bounds__(256) wf_finish_kernel(SceneDev<T> sc, WaveDev<T> w, typename M<T>::v4 *accum,
+                                                        typename std::conditional<kMoments, double *, PkNone>::type moments) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= w.P) return;
     const size_t P = (size_t)w.P;
@@ -194,6 +196,11 @@ __global__ void __launch_bounds__(256) wf_finish_kernel(SceneDev<T> sc, WaveDev<
     wf_path_id<T>(w, i, x, y, s);
     T *px = reinterpret_cast<T *>(accum + ((size_t)y * w.W + x));
     atomicAdd(px + 0, (T)c[0]); atomicAdd(px + 1, (T)c[1]); atomicAdd(px + 2, (T)c[2]); atomicAdd(px + 3, T(1));
+    if constexpr (kMoments) {
+        double *q = moments + 4 * ((size_t)y * w.W + x);
+        atomicAdd(q + 0, __dmul_rn(c[0], c[0])); atomicAdd(q + 1, __dmul_rn(c[1], c[1])); atomicAdd(q + 2, __dmul_rn(c[2], c[2]));
+        atomicAdd(q + 3, 1.0);
+    }
 }
 
 // ------------------------------------------------------------------ launchers
@@ -220,9 +227,10 @@ cudaError_t launch_wf_bounce(const WaveDev<T> &w, const uint8_t *need, const flo
     return cudaGetLastError();
 }
 template <typename T>
-cudaError_t launch_wf_finish(const SceneDev<T> &sc, const WaveDev<T> &w, void *accum, cudaStream_t st) {
+cudaError_t launch_wf_finish(const SceneDev<T> &sc, const WaveDev<T> &w, void *accum, double *moments, cudaStream_t st) {
     if (w.P <= 0) return cudaSuccess;
-    wf_finish_kernel<T><<<(w.P + 255) / 256, 256, 0, st>>>(sc, w, (typename M<T>::v4 *)accum);
+    if (moments) wf_finish_kernel<T, true><<<(w.P + 255) / 256, 256, 0, st>>>(sc, w, (typename M<T>::v4 *)accum, moments);
+    else wf_finish_kernel<T, false><<<(w.P + 255) / 256, 256, 0, st>>>(sc, w, (typename M<T>::v4 *)accum, PkNone());
     return cudaGetLastError();
 }
 
@@ -232,6 +240,6 @@ cudaError_t launch_wf_finish(const SceneDev<T> &sc, const WaveDev<T> &w, void *a
                                             unsigned long long *, cudaStream_t);                                         \
     template cudaError_t launch_wf_bounce<T>(const WaveDev<T> &, const uint8_t *, const float *, unsigned long long *,    \
                                              int *, cudaStream_t);                                                       \
-    template cudaError_t launch_wf_finish<T>(const SceneDev<T> &, const WaveDev<T> &, void *, cudaStream_t);
+    template cudaError_t launch_wf_finish<T>(const SceneDev<T> &, const WaveDev<T> &, void *, double *, cudaStream_t);
 
 }  // namespace rt

@@ -22,6 +22,8 @@ class FrameContext:
         self._key = None
         self.accum = self.image = self.stats = self.hit = None
         self.host_image = self.host_stats = None
+        self.moments = self.var = None      # variance frames only: [H,W,4] float64 moments, [H,W,3] float32 variance
+        self.host_var_ring, self.host_var = [], None
         self.h2d_bytes = 0          # bytes of the last scene upload
         self.d2h_bytes = 0          # bytes of the last read-back
 
@@ -43,10 +45,14 @@ class FrameContext:
         return self.scene
 
     # ---- buffers ---------------------------------------------------------------------------------------------
-    def ensure(self, W, H, precision=nat.F32, want_hit=False):
+    def _buffers(self):
+        return [self.accum, self.image, self.stats, self.hit, self.host_stats, self.moments, self.var] + \
+            list(getattr(self, "host_ring", [])) + list(self.host_var_ring)
+
+    def ensure(self, W, H, precision=nat.F32, want_hit=False, want_variance=False):
         key = (int(W), int(H), precision)
         if self._key != key:
-            for b in [self.accum, self.image, self.stats, self.hit, self.host_stats] + list(getattr(self, "host_ring", [])):
+            for b in self._buffers():
                 if b is not None:
                     b.free()
             ft = np.float64 if precision == nat.F64 else np.float32
@@ -60,30 +66,49 @@ class FrameContext:
             self.host_image = self.host_ring[0]
             self.host_stats = nat.PinnedArray(8, np.uint64)
             self.hit = None
+            self.moments = self.var = None
+            self.host_var_ring = []
             self._key = key
         if want_hit and self.hit is None:
             self.hit = nat.DeviceBuffer((H, W), np.int32, self.device)
+        if want_variance and self.moments is None:
+            # allocated on the first variance frame: frames without it neither allocate nor write these buffers
+            self.moments = nat.DeviceBuffer((H, W, 4), np.float64, self.device)
+            self.var = nat.DeviceBuffer((H, W, 3), np.float32, self.device)
+            self.host_var_ring = [nat.PinnedArray((H, W, 3), np.float32) for _ in range(self.HOST_RING)]
 
     # ---- frames ----------------------------------------------------------------------------------------------
     def render_path(self, cam, W, H, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, precision=nat.F32, rows=None,
-                    samples=None, resolve=True, read_back=True, stream=None):
-        """Algorithm B over rows x samples of this rank.  Returns (host image view or None, stats u64[8] or None)."""
-        self.ensure(W, H, precision)
+                    samples=None, resolve=True, read_back=True, stream=None, variance=False):
+        """Algorithm B over rows x samples of this rank.  Returns (host image view or None, stats u64[8] or None).
+
+        variance=True: the launch also stores the second moments of every pixel's samples (``self.moments``), and the
+        result gains a third item, the float32 [H,W,3] variance of each pixel's mean in colour levels^2 -- a view of a
+        pinned host ring like the image (None when not read back; ``self.var`` holds it in HBM when resolved)."""
+        self.ensure(W, H, precision, want_variance=variance)
         L = nat.lib()
         p = self.scene.path_params(cam, W, H, spp, max_bounces, mirror_threshold, seed=seed, fov=fov, rows=rows,
                                    samples=samples)
         self.stats.fill(0, stream)
+        moments = self.moments if variance else None
         bands = self._bands(W, p.y0, p.y1, p.s1 - p.s0) if (resolve and read_back) else None
         if bands:
-            return self._render_path_banded(p, bands, W, H, precision, stream)
-        self.scene.render_path(p, self.accum, precision, stats=self.stats, stream=stream)
+            return self._render_path_banded(p, bands, W, H, precision, stream, variance)
+        self.scene.render_path(p, self.accum, precision, stats=self.stats, stream=stream, moments=moments)
         self.launches = 1
         if resolve:
             self.scene.resolve(self.accum, W, H, p.s1 - p.s0, self.image, precision, rows=(p.y0, p.y1), stream=stream)
             self.launches += 1
+            if variance:
+                self.scene.resolve_variance(self.accum, self.moments, W, H, self.var, precision, rows=(p.y0, p.y1),
+                                            stream=stream)
+                self.launches += 1
         if not read_back:
-            return None, None
-        return self.read_back(W, H, (p.y0, p.y1), stream)
+            return (None, None, None) if variance else (None, None)
+        image, stats = self.read_back(W, H, (p.y0, p.y1), stream, variance=variance and resolve)
+        if variance:
+            return image, stats, (self.host_var.array if resolve else None)
+        return image, stats
 
     # a frame whose image takes longer to copy out than a launch costs is rendered in row bands: band b is copied to the
     # pinned host image (copy stream) while band b + 1 renders.  Pixels are keyed by (pixel, sample), so the frame is the
@@ -107,7 +132,7 @@ class FrameContext:
         cuts = [y0 + 8 * ((stripes * sum(w[:k])) // sum(w)) for k in range(self.BANDS)] + [y1]
         return [(a, b) for a, b in zip(cuts[:-1], cuts[1:]) if b > a]
 
-    def _render_path_banded(self, p, bands, W, H, precision, stream):
+    def _render_path_banded(self, p, bands, W, H, precision, stream, variance=False):
         L = nat.lib()
         if getattr(self, "_copy_stream", None) is None:
             cs = nat.vp()
@@ -116,21 +141,31 @@ class FrameContext:
         cs = self._copy_stream
         self._ring_at = (self._ring_at + 1) % self.HOST_RING
         self.host_image = self.host_ring[self._ring_at]
+        if variance:
+            self.host_var = self.host_var_ring[self._ring_at]
         ns, y0, y1 = p.s1 - p.s0, p.y0, p.y1
         self.launches = 0
         for (a, b) in bands:
             p.y0, p.y1 = a, b
-            self.scene.render_path(p, self.accum, precision, stats=self.stats, stream=stream)
+            self.scene.render_path(p, self.accum, precision, stats=self.stats, stream=stream,
+                                   moments=self.moments if variance else None)
             self.scene.resolve(self.accum, W, H, ns, self.image, precision, rows=(a, b), stream=stream)
             self.launches += 2
+            if variance:
+                self.scene.resolve_variance(self.accum, self.moments, W, H, self.var, precision, rows=(a, b), stream=stream)
+                self.launches += 1
             nat.check(L.rt_stream_wait_stream(self.device, cs, stream))
             off, nbytes = a * W * 12, (b - a) * W * 12
             nat.check(L.rt_memcpy_d2h(self.device, self.host_image.ptr + off, self.image.ptr + off, nbytes, cs))
+            if variance:
+                nat.check(L.rt_memcpy_d2h(self.device, self.host_var.ptr + off, self.var.ptr + off, nbytes, cs))
         p.y0, p.y1 = y0, y1
         nat.check(L.rt_memcpy_d2h(self.device, self.host_stats.ptr, self.stats.ptr, 64, stream))
         nat.check(L.rt_stream_sync(self.device, stream))
         nat.check(L.rt_stream_sync(self.device, cs))
-        self.d2h_bytes = (y1 - y0) * W * 12 + 64
+        self.d2h_bytes = (y1 - y0) * W * (24 if variance else 12) + 64
+        if variance:
+            return self.host_image.array, self.host_stats.array, self.host_var.array
         return self.host_image.array, self.host_stats.array
 
     def render_whitted(self, cam, X, Y, spp=1, max_bounces=1, shadow_max_bounces=0, miss=None, seed=0, prenorm=False,
@@ -147,8 +182,9 @@ class FrameContext:
             return None, None
         return self.read_back(W, H, (p.y0, p.y1), stream)
 
-    def read_back(self, W, H, rows, stream=None):
-        """D2H of the resolved rows (float32) + the stats block into pinned memory; synchronises the stream."""
+    def read_back(self, W, H, rows, stream=None, variance=False):
+        """D2H of the resolved rows (float32) + the stats block into pinned memory; synchronises the stream.  variance:
+        the rows of the variance image too, into ``self.host_var`` (the pinned ring slot of this frame)."""
         L = nat.lib()
         y0, y1 = rows
         self._ring_at = (self._ring_at + 1) % self.HOST_RING
@@ -156,16 +192,22 @@ class FrameContext:
         off, nbytes = y0 * W * 3 * 4, (y1 - y0) * W * 3 * 4
         if nbytes:
             nat.check(L.rt_memcpy_d2h(self.device, self.host_image.ptr + off, self.image.ptr + off, nbytes, stream))
+        if variance:
+            self.host_var = self.host_var_ring[self._ring_at]
+            if nbytes:
+                nat.check(L.rt_memcpy_d2h(self.device, self.host_var.ptr + off, self.var.ptr + off, nbytes, stream))
         nat.check(L.rt_memcpy_d2h(self.device, self.host_stats.ptr, self.stats.ptr, 64, stream))
         nat.check(L.rt_stream_sync(self.device, stream))
-        self.d2h_bytes = nbytes + 64
+        self.d2h_bytes = nbytes * (2 if variance else 1) + 64
         return self.host_image.array, self.host_stats.array
 
     def close(self):
-        for b in [self.accum, self.image, self.stats, self.hit, self.host_stats] + list(getattr(self, "host_ring", [])):
+        for b in self._buffers():
             if b is not None:
                 b.free()
         self.host_ring = []
+        self.host_var_ring = []
+        self.moments = self.var = None
         if getattr(self, "_copy_stream", None) is not None:
             nat.lib().rt_stream_destroy(self.device, self._copy_stream)
             self._copy_stream = None

@@ -79,23 +79,38 @@ def render_whitted(fs, camera, X, Y, spp=1, max_bounces=1, shadow_max_bounces=0,
     return image
 
 
+def _variance_frame(sc, p, prec, W, H):
+    """One path-kernel launch with the second moments -> (image [H,W,3], sums [H,W,4], stats u64[8], variance [H,W,3])."""
+    ft = np.float64 if prec == nat.F64 else np.float32
+    accum, moments = nat.DeviceBuffer((H, W, 4), ft, sc.device), nat.DeviceBuffer((H, W, 4), np.float64, sc.device)
+    stats = nat.DeviceBuffer(8, np.uint64, sc.device)
+    image, var = nat.DeviceBuffer((H, W, 3), np.float32, sc.device), nat.DeviceBuffer((H, W, 3), np.float32, sc.device)
+    sc.render_path(p, accum, prec, stats=stats, moments=moments)
+    sc.resolve(accum, W, H, p.s1 - p.s0, image, prec)
+    sc.resolve_variance(accum, moments, W, H, var, prec)
+    return image.download(), accum.download(), stats.download(), var.download()
+
+
 def render_path(fs, camera, width, height, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, precision="f32",
-                device=0, lbvh=None, return_raw=False):
+                device=0, lbvh=None, return_raw=False, variance=False):
     """Algorithm B frame -> float32 image [H,W,3] (``sum // spp / 255``).  lbvh: None = build the on-device LBVH when
-    the scene has more than 256 spheres, True/False to force."""
+    the scene has more than 256 spheres, True/False to force.  variance=True appends the float32 [H,W,3] variance of
+    each pixel's mean in colour levels^2 (0-255 scale), estimated from the same samples in the same launch."""
     sc = nat.DeviceScene(fs, device)
     try:
         if lbvh or (lbvh is None and sc.n > 256):
             sc.build_lbvh()
         p = sc.path_params(_xyz(camera), width, height, spp, max_bounces, mirror_threshold, seed=seed, fov=fov)
-        image, sums, st = sc.render_path_host(p, _precision(precision), want_accum=return_raw)
+        if variance:
+            image, sums, st, var = _variance_frame(sc, p, _precision(precision), int(width), int(height))
+        else:
+            image, sums, st = sc.render_path_host(p, _precision(precision), want_accum=return_raw)
     finally:
         sc.close()
     stats = {"total_rays": int(st[0]), "total_intersections": int(st[1]), "light_hits": int(st[2]),
              "small_light_hits": int(st[3]), "queries": int(st[4]), "sphere_tests": int(st[5]), "aabb_tests": int(st[6])}
-    if return_raw:
-        return image, sums, stats
-    return image, stats
+    out = (image, sums, stats) if return_raw else (image, stats)
+    return out + (var,) if variance else out
 
 
 class TraditionalRenderer:
@@ -108,6 +123,9 @@ class TraditionalRenderer:
 
     mirror_threshold = 0.0
     reuse_output = True
+    # True: render() also sets self.variance, the float32 [H,W,3] variance of each pixel's mean in colour levels^2,
+    # estimated from the frame's own samples in the same launch (a view of a pinned ring, like the image)
+    track_variance = False
 
     def __init__(self, device=0, precision="f32", seed=None):
         self.scene = []
@@ -176,9 +194,12 @@ class TraditionalRenderer:
         if self._ctx is None:
             self._ctx = FrameContext(self.device)
         self._ctx.set_scene(self.flat_scene())          # re-flattened every render: the scene list is mutable
-        view, st = self._ctx.render_path(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
-                                         self.mirror_threshold, seed=seed, fov=self.fov,
-                                         precision=_precision(self.precision))
+        out = self._ctx.render_path(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
+                                    self.mirror_threshold, seed=seed, fov=self.fov, precision=_precision(self.precision),
+                                    variance=self.track_variance)
+        view, st = out[:2]
+        if self.track_variance:
+            self.variance = out[2] if self.reuse_output else out[2].copy()
         # reuse_output (default True): the image is a view of one of the renderer's FrameContext.HOST_RING pinned host
         # buffers -- it stays valid until two more frames have been rendered by THIS renderer, which covers every use
         # in the reference's drivers (plot / save / compare right after render()).  reuse_output = False returns a
@@ -414,12 +435,13 @@ def _batched_policy(agent):
 
 
 def render_path_wavefront(fs, camera, width, height, spp, max_bounces, mirror_threshold, policy=None, fb_usage_prob=1.0,
-                          seed=0, fov=60.0, precision="f32", device=0, max_paths=1 << 22, scene=None):
+                          seed=0, fov=60.0, precision="f32", device=0, max_paths=1 << 22, scene=None, variance=False):
     """Algorithm B frame with ``policy(obs [m,22] float32 CUDA tensor) -> actions [m,2]`` choosing the diffuse bounce
     direction with probability ``fb_usage_prob`` (``WorkingFBRenderer.trace_ray_fb``,
     FB/fb_vs_traditional_complex.py:487-601).  Wavefront on the GPU: per bounce one trace kernel, the policy on the
     asking paths, one bounce kernel; sample ranges are processed ``max_paths`` paths at a time.
-    -> (image [H,W,3] float32 numpy, sums [H,W,4] numpy, stats dict)."""
+    -> (image [H,W,3] float32 numpy, sums [H,W,4] numpy, stats dict), plus the float32 [H,W,3] variance of each pixel's
+    mean (colour levels^2) when ``variance`` is set."""
     import ctypes as C
     import torch
     prec = _precision(precision)
@@ -436,6 +458,7 @@ def render_path_wavefront(fs, camera, width, height, spp, max_bounces, mirror_th
         nat.check(nat.lib().rt_wf_create(sc.handle, prec, P, max(1, int(max_bounces)), C.byref(wf)))
         ft = torch.float64 if prec == nat.F64 else torch.float32
         accum = torch.zeros((height, width, 4), dtype=ft, device=dev)
+        moments = torch.zeros((height, width, 4), dtype=torch.float64, device=dev) if variance else None
         obs = torch.zeros((P, 22), dtype=torch.float32, device=dev)
         need = torch.zeros(P, dtype=torch.uint8, device=dev)
         actions = torch.zeros((P, 2), dtype=torch.float32, device=dev)
@@ -457,13 +480,21 @@ def render_path_wavefront(fs, camera, width, height, spp, max_bounces, mirror_th
                 nat.check(nat.lib().rt_wf_bounce(wf, need.data_ptr(), actions.data_ptr(), stats.data_ptr(), live.data_ptr(), None))
                 if int(live.item()) == 0:
                     break
-            nat.check(nat.lib().rt_wf_finish(wf, accum.data_ptr(), None))
+            if variance:
+                nat.check(nat.lib().rt_wf_finish_moments(wf, accum.data_ptr(), moments.data_ptr(), None))
+            else:
+                nat.check(nat.lib().rt_wf_finish(wf, accum.data_ptr(), None))
         image = torch.zeros((height, width, 3), dtype=torch.float32, device=dev)
         sc.resolve(accum, width, height, spp, image, prec)
+        if variance:
+            var = torch.zeros((height, width, 3), dtype=torch.float32, device=dev)
+            sc.resolve_variance(accum, moments, width, height, var, prec)
         torch.cuda.synchronize(dev)
         st = stats.cpu().numpy()
         out = {"total_rays": int(st[0]), "total_intersections": int(st[1]), "light_hits": int(st[2]), "small_light_hits": int(st[3]),
                "queries": int(st[4]), "sphere_tests": int(st[5]), "fb_used": int(st[7])}
+        if variance:
+            return image.cpu().numpy(), accum.cpu().numpy(), out, var.cpu().numpy()
         return image.cpu().numpy(), accum.cpu().numpy(), out
     finally:
         if wf.value:
@@ -483,6 +514,7 @@ class WorkingFBRenderer:
 
     mirror_threshold = 0.9
     reuse_output = True         # agent-less frames: see TraditionalRenderer.render
+    track_variance = False      # True: render() also sets self.variance (see TraditionalRenderer), on both branches
 
     def __init__(self, model_path=None, scene_small_lights=None, camera_position=None, device=0, precision="f32", seed=None):
         if model_path is not None:
@@ -521,19 +553,25 @@ class WorkingFBRenderer:
             if self._ctx is None:
                 self._ctx = FrameContext(self.device)
             self._ctx.set_scene(fs)
-            view, st = self._ctx.render_path(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
-                                             self.mirror_threshold, seed=seed, fov=self.fov,
-                                             precision=_precision(self.precision))
+            out = self._ctx.render_path(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
+                                        self.mirror_threshold, seed=seed, fov=self.fov, precision=_precision(self.precision),
+                                        variance=self.track_variance)
+            view, st = out[:2]
+            if self.track_variance:
+                self.variance = out[2] if self.reuse_output else out[2].copy()
             for i, k in enumerate(('total_rays', 'total_intersections', 'light_hits', 'small_light_hits')):
                 self.stats[k] = int(st[i])
             self.stats['render_time'] = time.time() - start
             if self.stats['render_time'] > 0:
                 self.stats['rays_per_second'] = self.stats['total_rays'] / self.stats['render_time']
             return view if self.reuse_output else view.copy()      # as TraditionalRenderer.render: a view of the pinned ring
-        image, _, st = render_path_wavefront(fs, _xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
-                                             self.mirror_threshold, policy=_batched_policy(self.fb_agent) if use else None,
-                                             fb_usage_prob=self.fb_usage_prob if use else 0.0, seed=seed, fov=self.fov,
-                                             precision=self.precision, device=self.device)
+        res = render_path_wavefront(fs, _xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
+                                    self.mirror_threshold, policy=_batched_policy(self.fb_agent) if use else None,
+                                    fb_usage_prob=self.fb_usage_prob if use else 0.0, seed=seed, fov=self.fov,
+                                    precision=self.precision, device=self.device, variance=self.track_variance)
+        image, _, st = res[:3]
+        if self.track_variance:
+            self.variance = res[3]
         for k in ('total_rays', 'total_intersections', 'light_hits', 'small_light_hits', 'fb_used'):
             self.stats[k] = st[k]
         self.stats['fb_success'] = st['fb_used']                     # the reference counts both at the same place (:539-544)

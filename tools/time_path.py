@@ -1,6 +1,9 @@
 #!/usr/bin/env python
 """Device-time the path kernel alone (CUDA events) for scene / spp / ksplit variants and the diagnostic schedule bits
-(rt_path_params.schedule: 2 = no camera-ray candidate lists, 4 = no parameter-block kernel).  Development aid."""
+(rt_path_params.schedule: 2 = no camera-ray candidate lists, 4 = no parameter-block kernel).  Development aid.
+
+--moments: the plain launch and the launch that also stores the per-pixel second moments (rt_render_path_moments),
+alternately in one process; prints both times, the overhead, and whether the two accumulation buffers are the same."""
 import argparse
 import os
 import sys
@@ -26,6 +29,7 @@ def main():
     ap.add_argument("--schedules", default="0", help="comma-separated schedule values, e.g. 0,2,4")
     ap.add_argument("--no-stats", action="store_true", help="launch without the statistics counters")
     ap.add_argument("--save", default=None, help="write the last accumulation buffer to this .npy")
+    ap.add_argument("--moments", action="store_true", help="time the plain and the moments launch alternately")
     args = ap.parse_args()
     if args.scene.startswith("scaled"):           # scaled1000 / scaled10000 / scaled100000: SURVEY 8d's LBVH variant of C4
         spec = scenes.build_chandelier()
@@ -41,6 +45,9 @@ def main():
     accum = torch.zeros((H, W, 4), dtype=torch.float32, device="cuda")
     stats = torch.zeros(8, dtype=torch.int64, device="cuda")
     ref = None
+    if args.moments:
+        time_moments(sc, spec, args, accum, stats)
+        return
     for schedule in [int(v) for v in args.schedules.split(',')]:
         p = sc.path_params(spec.camera, W, H, args.spp, spec.max_bounces, spec.mirror_threshold, seed=1, schedule=schedule, ksplit=args.ksplit)
         sc.render_path(p, accum, nat.F32, stats=stats)
@@ -61,6 +68,31 @@ def main():
         print(f"{args.scene} {W}x{H} spp {args.spp} schedule {schedule} ksplit {args.ksplit}: {best:.3f} ms  {st[4] / best / 1e6:.2f} Gqueries/s "
               f"rays/sample {st[0] / (W * H * args.spp):.3f}  tests/query {st[5] / st[4]:.1f} boxes/query {st[6] / st[4]:.1f} same_image={same} "
               f"sha1 {hashlib.sha1(np.ascontiguousarray(img).tobytes()).hexdigest()[:12]}", flush=True)
+
+
+def time_moments(sc, spec, args, accum, stats):
+    W, H = args.w, args.h
+    moments = torch.zeros((H, W, 4), dtype=torch.float64, device="cuda")
+    sha = lambda t: hashlib.sha1(np.ascontiguousarray(t.cpu().numpy()).tobytes()).hexdigest()[:12]      # noqa: E731
+    for schedule in [int(v) for v in args.schedules.split(',')]:
+        p = sc.path_params(spec.camera, W, H, args.spp, spec.max_bounces, spec.mirror_threshold, seed=1, schedule=schedule, ksplit=args.ksplit)
+        variants = (("plain", None), ("moments", moments))
+        for _, m in variants:                                              # warm-up: module load, smem opt-in
+            sc.render_path(p, accum, nat.F32, stats=stats, moments=m)
+        torch.cuda.synchronize()
+        times, digest = {k: [] for k, _ in variants}, {}
+        for _ in range(args.reps):
+            for name, m in variants:
+                a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                a.record(); sc.render_path(p, accum, nat.F32, stats=None if args.no_stats else stats, moments=m); b.record()
+                torch.cuda.synchronize()
+                times[name].append(a.elapsed_time(b))
+                digest[name] = sha(accum)
+        t0, t1 = np.median(times["plain"]), np.median(times["moments"])
+        print(f"{args.scene} {W}x{H} spp {args.spp} schedule {schedule} ksplit {args.ksplit} ({args.reps} alternating reps, "
+              f"median / min): plain {t0:.3f} / {min(times['plain']):.3f} ms  moments {t1:.3f} / {min(times['moments']):.3f} ms  "
+              f"overhead {100.0 * (t1 / t0 - 1):+.2f} %  accum sha1 plain {digest['plain']} moments {digest['moments']} "
+              f"same={digest['plain'] == digest['moments']}", flush=True)
 
 
 if __name__ == "__main__":
