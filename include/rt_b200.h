@@ -346,6 +346,27 @@ int rt_render_path_sink(rt_scene *scene, const rt_path_params *p, const rt_path_
  * the next frame. */
 int rt_resolve_clear(int device, void *accum_dev, int32_t W, int32_t H, int32_t y0, int32_t y1, int32_t spp,
                      float *image_dev, int32_t clear, void *stream);
+/* per-pixel variance through the fused sinks (rt_render_path_sink_moments): where the second moments of the samples go.
+ *   RT_SINK_IMAGE        reads var only: rank 0's [H,W,3] float32 variance image (device or peer pointer), which
+ *                        receives what rt_resolve_variance gives for the resolved pixels.
+ *   RT_SINK_SCATTER_ADD  reads moments[0..world): per-owner [H,W,4] float64 (sum r^2, sum g^2, sum b^2, n), zeroed by the
+ *                        owner, into which each pixel's moments are added with system-scope f64 reductions (integer-valued
+ *                        doubles below 2^53: exact in any order); with sync also var, into which the own band's
+ *                        variance is resolved (the moments band is then cleared like the sums). */
+typedef struct rt_path_moments_sink {
+    void *moments[RT_MAX_PEERS];
+    float *var;
+} rt_path_moments_sink;
+/* rt_render_path_sink that also carries the second moments of every pixel's samples into msink.  The image, the sums and
+ * stats_dev are bit-identical to rt_render_path_sink's, and the variance equals rt_render_path_moments +
+ * rt_resolve_variance of the unsharded frame bit for bit.  RT_ERR_INVALID for a NULL var (IMAGE, or SCATTER_ADD with
+ * sync) or a NULL moments[k], k < world (SCATTER_ADD).  Every rank of a frame must ask for the moments, or none. */
+int rt_render_path_sink_moments(rt_scene *scene, const rt_path_params *p, const rt_path_sink *sink,
+                                const rt_path_moments_sink *msink, uint64_t *stats_dev, void *stream);
+/* rt_resolve_clear that also resolves rows [y0,y1) of moments_dev [H,W,4] double (with accum_dev) into var_dev [H,W,3]
+ * float32 (device or peer pointer) as rt_resolve_variance does and, when clear != 0, zeroes those rows of both buffers. */
+int rt_resolve_clear_moments(int device, void *accum_dev, double *moments_dev, int32_t W, int32_t H, int32_t y0, int32_t y1,
+                             int32_t spp, float *image_dev, float *var_dev, int32_t clear, void *stream);
 
 /* peer memory (CUDA IPC): rt_peer_alloc = cudaMalloc + zero + export; the handle travels to the other ranks by any
  * means (torch.distributed.all_gather_object), which open it with rt_peer_open. */

@@ -83,6 +83,12 @@ class PathSink(C.Structure):
                 ("max_ctas", C.c_int32), ("spp_total", C.c_int32), ("col_split", C.c_int32)]
 
 
+class PathMomentsSink(C.Structure):
+    """rt_path_moments_sink: where the fused sinks put the second moments (image sink: ``var``; scatter-add sink:
+    ``moments[k]`` of every owner, and ``var`` under ``sync``)."""
+    _fields_ = [("moments", C.c_void_p * RT_MAX_PEERS), ("var", C.c_void_p)]
+
+
 FLAG_WORDS = 64
 
 
@@ -139,6 +145,10 @@ SIGNATURES = {
     "rt_render_simple_host": (C.c_int, [vp, C.c_int, C.POINTER(SimpleParams), vp, vp, vp, vp]),
     "rt_render_path_sink": (C.c_int, [vp, C.POINTER(PathParams), C.POINTER(PathSink), vp, vp]),
     "rt_resolve_clear": (C.c_int, [C.c_int, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, C.c_int32, vp]),
+    "rt_render_path_sink_moments": (C.c_int, [vp, C.POINTER(PathParams), C.POINTER(PathSink), C.POINTER(PathMomentsSink), vp,
+                                              vp]),
+    "rt_resolve_clear_moments": (C.c_int, [C.c_int, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp,
+                                           C.c_int32, vp]),
     "rt_peer_alloc": (C.c_int, [C.c_int, C.c_size_t, C.POINTER(vp), C.c_char_p]),
     "rt_peer_open": (C.c_int, [C.c_int, C.c_char_p, C.POINTER(vp)]),
     "rt_peer_close": (C.c_int, [C.c_int, vp]),
@@ -481,9 +491,15 @@ class DeviceScene:
         check(lib().rt_trace_paths(self.handle, precision, C.byref(p), m, r.ptr, _ptr(ids), int(bounce_count), acc.ptr, st.ptr, None))
         return acc.download(), st.download()
 
-    def render_path_sink(self, params, sink, stats=None, stream=None):
-        """FP32 path kernel with a fused multi-GPU sink (``PathSink``: image store / scatter-add over peer memory)."""
-        check(lib().rt_render_path_sink(self.handle, C.byref(params), C.byref(sink), _ptr(stats), stream))
+    def render_path_sink(self, params, sink, stats=None, stream=None, moments_sink=None):
+        """FP32 path kernel with a fused multi-GPU sink (``PathSink``: image store / scatter-add over peer memory).
+        ``moments_sink`` (``PathMomentsSink``, optional) also carries the per-pixel variance through the sink
+        (``rt_render_path_sink_moments``); the image and stats are the same."""
+        if moments_sink is None:
+            check(lib().rt_render_path_sink(self.handle, C.byref(params), C.byref(sink), _ptr(stats), stream))
+        else:
+            check(lib().rt_render_path_sink_moments(self.handle, C.byref(params), C.byref(sink), C.byref(moments_sink),
+                                                    _ptr(stats), stream))
 
     def resolve(self, accum, W, H, spp, image, precision=F32, rows=None, stream=None):
         y0, y1 = (0, H) if rows is None else rows

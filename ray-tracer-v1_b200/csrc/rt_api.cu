@@ -345,7 +345,7 @@ static inline cudaStream_t S(void *stream) { return reinterpret_cast<cudaStream_
 
 // ------------------------------------------------------------------ library / device
 RT_EXPORT const char *rt_last_error(void) { return g_err.c_str(); }
-RT_EXPORT int rt_version(void) { return 101; }
+RT_EXPORT int rt_version(void) { return 102; }
 
 RT_EXPORT int rt_device_count(int *count) {
     if (!count) return fail(RT_ERR_INVALID, "count is NULL");
@@ -750,7 +750,7 @@ static PathLaunch plan_path_launch(PathDev<T> &pp, const SceneDev<T> &sc, const 
 template <typename T>
 static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_path_params *p, void *accum, uint64_t *stats,
                          cudaStream_t st, const rt_path_sink *sink = nullptr, const ExplicitRays *xr = nullptr,
-                         double *moments = nullptr) {
+                         double *moments = nullptr, const rt_path_moments_sink *msink = nullptr) {
     // bit 1: no camera-ray candidate lists, bit 2: no parameter-block kernel (include/rt_b200.h)
     if (p->schedule & ~6) return fail(RT_ERR_INVALID, "unknown schedule bits");
     PathDev<T> pp;
@@ -812,13 +812,29 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
             pp.timeout_cycles = (long long)(sink->timeout_ms > 0 ? sink->timeout_ms : 20000) * (long long)khz;
         }
     }
+    // the moments sinks of the kMoments kernels: accum mode keeps them beside accum, the fused sinks where their sums go
+    MomentsDev md;
+    std::memset(&md, 0, sizeof md);
+    md.local = reinterpret_cast<double4 *>(moments);
+    if (msink) {
+        if (pp.sink == RT_SINK_IMAGE || pp.sync) {
+            if (!msink->var) return fail(RT_ERR_INVALID, "moments sink: missing variance image");
+            md.var = msink->var;
+        }
+        if (pp.sink == RT_SINK_SCATTER_ADD)
+            for (int k = 0; k < pp.world; ++k) {
+                if (!msink->moments[k]) return fail(RT_ERR_INVALID, "moments sink: missing peer moments");
+                md.peer[k] = reinterpret_cast<double4 *>(msink->moments[k]);
+            }
+    }
     int sms = 0;
     if (device_attr(sc->device, cudaDevAttrMultiProcessorCount, &sms) != cudaSuccess || sms <= 0) sms = 148;
     const PathLaunch pl = plan_path_launch<T>(pp, view, p, sink, xr != nullptr, sc->byte_colours,
                                               sizeof(T) == 4 && sc->pkc_ok && !(p->schedule & 4) && !xr, sms);
     if (!sc->sched_dev) return fail(RT_ERR_INVALID, "scene has no scheduler counters (upload failed?)");
     pp.sched = sc->sched_dev + 4 * (sc->sched_next.fetch_add(1u) % RT_SCHED_SLOTS);      // {next unit, warps done, CTAs resolved, -}
-    CU(launch_path<T>(view, pp, pl, accum, reinterpret_cast<unsigned long long *>(stats), st, &sc->pkc, moments));
+    CU(launch_path<T>(view, pp, pl, accum, reinterpret_cast<unsigned long long *>(stats), st, &sc->pkc,
+                      (moments || msink) ? &md : nullptr));
     return RT_OK;
 }
 
@@ -875,12 +891,37 @@ RT_EXPORT int rt_render_path_sink(rt_scene *scene, const rt_path_params *p, cons
     return render_path_t<float>(scene, scene->f.view, &q, nullptr, stats_dev, S(stream), sink);
 }
 
+RT_EXPORT int rt_render_path_sink_moments(rt_scene *scene, const rt_path_params *p, const rt_path_sink *sink,
+                                          const rt_path_moments_sink *msink, uint64_t *stats_dev, void *stream) {
+    if (!scene || !p || !sink || !msink) return fail(RT_ERR_INVALID, "NULL argument");
+    int rc = check_band(p->W, p->H, 0, p->H, p->s0, p->s1);
+    if (rc) return rc;
+    if (p->max_bounces > RT_PATH_MAX_DEPTH) return fail(RT_ERR_UNSUPPORTED, "max_bounces above 32 is not supported by the path kernel");
+    if (sink->mode == RT_SINK_ACCUM) return fail(RT_ERR_INVALID, "use rt_render_path_moments for the accumulator sink");
+    CU(cudaSetDevice(scene->device));
+    rt_path_params q = *p;
+    q.y0 = 0; q.y1 = p->H;
+    return render_path_t<float>(scene, scene->f.view, &q, nullptr, stats_dev, S(stream), sink, nullptr, nullptr, msink);
+}
+
 RT_EXPORT int rt_resolve_clear(int device, void *accum_dev, int32_t W, int32_t H, int32_t y0, int32_t y1, int32_t spp,
                                float *image_dev, int32_t clear, void *stream) {
     if (!accum_dev || !image_dev) return fail(RT_ERR_INVALID, "NULL argument");
     if (W <= 0 || H <= 0 || y0 < 0 || y1 > H || y0 > y1 || spp <= 0) return fail(RT_ERR_INVALID, "bad arguments");
     CU(cudaSetDevice(device));
     CU(launch_resolve_clear(reinterpret_cast<float4 *>(accum_dev), W, y0, y1, spp, image_dev, clear, S(stream)));
+    return RT_OK;
+}
+
+RT_EXPORT int rt_resolve_clear_moments(int device, void *accum_dev, double *moments_dev, int32_t W, int32_t H, int32_t y0,
+                                       int32_t y1, int32_t spp, float *image_dev, float *var_dev, int32_t clear, void *stream) {
+    if (!accum_dev || !moments_dev || !image_dev || !var_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    if (spp <= 0) return fail(RT_ERR_INVALID, "spp must be positive");
+    int rc = check_band(W, H, y0, y1, 0, 0);
+    if (rc) return rc;
+    CU(cudaSetDevice(device));
+    CU(launch_resolve_clear_moments(reinterpret_cast<float4 *>(accum_dev), reinterpret_cast<double4 *>(moments_dev), W, y0,
+                                    y1, spp, image_dev, var_dev, clear, S(stream)));
     return RT_OK;
 }
 

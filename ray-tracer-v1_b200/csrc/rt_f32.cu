@@ -43,6 +43,37 @@ cudaError_t launch_resolve_clear(float4 *accum, int W, int y0, int y1, int spp, 
     return cudaGetLastError();
 }
 
+// resolve_clear_kernel plus the moments: the variance of the same rows into the (possibly peer-mapped) variance image
+// (variance_of_mean, as rt_resolve_variance), and both buffers' rows cleared for the next frame
+__global__ void resolve_clear_moments_kernel(float4 *accum, double4 *moments, int W, int y0, int y1, int spp, float *image,
+                                             float *var, int clear) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t n = (size_t)(y1 - y0) * W;
+    if (i >= n) return;
+    const size_t o = (size_t)y0 * W + i;
+    const float4 a = accum[o];
+    const double4 q = moments[o];
+    const double s = (double)spp;
+    const double r = floor((double)a.x / s) / 255.0, g = floor((double)a.y / s) / 255.0, b = floor((double)a.z / s) / 255.0;
+    image[3 * o + 0] = (float)(r < 1.0 ? r : 1.0);
+    image[3 * o + 1] = (float)(g < 1.0 ? g : 1.0);
+    image[3 * o + 2] = (float)(b < 1.0 ? b : 1.0);
+    var[3 * o + 0] = variance_of_mean((double)a.x, q.x, q.w);
+    var[3 * o + 1] = variance_of_mean((double)a.y, q.y, q.w);
+    var[3 * o + 2] = variance_of_mean((double)a.z, q.z, q.w);
+    if (clear) {
+        accum[o] = make_float4(0.f, 0.f, 0.f, 0.f);
+        moments[o] = make_double4(0.0, 0.0, 0.0, 0.0);
+    }
+}
+cudaError_t launch_resolve_clear_moments(float4 *accum, double4 *moments, int W, int y0, int y1, int spp, float *image,
+                                         float *var, int clear, cudaStream_t st) {
+    const size_t n = (size_t)(y1 - y0) * W;
+    if (n == 0) return cudaSuccess;
+    resolve_clear_moments_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(accum, moments, W, y0, y1, spp, image, var, clear);
+    return cudaGetLastError();
+}
+
 // epoch flags in peer memory.  Signal: every write this stream issued before (kernel boundary) is ordered before the
 // flag by the system fence + release store.  Wait: acquire loads until every flag has reached the epoch.
 __global__ void peer_signal_kernel(PeerFlagTable flags, int n, unsigned epoch) {

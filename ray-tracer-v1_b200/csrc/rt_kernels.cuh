@@ -306,6 +306,20 @@ RT_DEV void flag_post(unsigned *flag, unsigned epoch) {
     asm volatile("st.release.sys.global.u32 [%0], %1;" :: "l"(flag), "r"(epoch) : "memory");
 }
 RT_DEV bool a_count_ok(int spp_total) { return spp_total > 0; }
+
+// variance of a pixel's mean in colour levels^2, from the sum S and the sum of squares Q of its k samples:
+// (Q - S^2/k) / (k (k-1)), evaluated as (k Q - S^2) / (k^2 (k-1)) -- the numerator is exact while k Q and S^2 stay below
+// 2^53 (integer colours), so a pixel whose samples all agree gets exactly 0; 0 where k < 2.  Every site that resolves a
+// variance (resolve_variance_kernel, the fused sinks of path_kernel, resolve_clear_moments_kernel) calls this one
+// expression, so their results agree bit for bit.
+RT_DEV float variance_of_mean(double S, double Q, double k) {
+    double v = 0.0;
+    if (k >= 2.0) {
+        v = __ddiv_rn(__dsub_rn(__dmul_rn(k, Q), __dmul_rn(S, S)), __dmul_rn(__dmul_rn(k, k), k - 1.0));
+        v = v > 0.0 ? v : 0.0;
+    }
+    return (float)v;
+}
 #define RT_FLAG_ADDED 0
 #define RT_FLAG_DONE 16
 #define RT_FLAG_GO 32
@@ -340,15 +354,16 @@ template <typename T> RT_DEV V3<T> path_camera_ray(const PathDev<T> &pp, int x, 
 // s+1 together.  Everything outside the sphere loop (camera ray, Philox, fold) runs once per sample at full lane
 // occupancy.
 // kIntFold: integer fold through the div255 table (all leaf colours integer-valued), else the double-division fold.
-// kMoments: also store the second moments of the pixel's samples, moments[o] = (sum r^2, sum g^2, sum b^2, n) (the
-// trailing parameter is empty otherwise, so the plain kernels keep their parameter offsets).  Exact: an integer-fold
-// colour is <= 65535, so its square fits a uint32 and a uint64 sum of 65536 of them stays below 2^53; the double fold
-// sums its squares in double.
+// kMoments: also the second moments of the pixel's samples, (sum r^2, sum g^2, sum b^2, n), into the sink of MomentsDev
+// that matches pp.sink: moments.local[o] like accum, the variance of the resolved pixel into moments.var (image sink), or
+// added into the owner's moments.peer[k] (scatter-add sink).  The trailing parameter is empty otherwise, so the plain
+// kernels keep their parameter offsets.  Exact: an integer-fold colour is <= 65535, so its square fits a uint32 and a
+// uint64 sum of 65536 of them stays below 2^53; the double fold sums its squares in double.
 template <typename T, int kMode, bool kIntFold, bool kMoments>
 __global__ void __launch_bounds__(256, (sizeof(T) == 4 ? (kMode == 3 ? RT_PATH_MIN_BLOCKS_PKC : RT_PATH_MIN_BLOCKS) : 1))
 path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned long long *stats,
             const __grid_constant__ typename std::conditional<kMode == 3, PkConst, PkNone>::type pkc,
-            typename std::conditional<kMoments, double4 *, PkNone>::type moments) {
+            const __grid_constant__ typename std::conditional<kMoments, MomentsDev, PkNone>::type moments) {
     RT_MODE_DECL;
     using PK = typename std::conditional<kMode == 3, PkConst, PkNone>::type;
     extern __shared__ __align__(32) unsigned char smem[];
@@ -665,6 +680,13 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                 const double r = floor((double)a0 / s) / 255.0, g = floor((double)a1 / s) / 255.0, b = floor((double)a2 / s) / 255.0;
                 float *px = pp.image + 3 * o;
                 px[0] = (float)(r < 1.0 ? r : 1.0); px[1] = (float)(g < 1.0 ? g : 1.0); px[2] = (float)(b < 1.0 ? b : 1.0);
+                if constexpr (kMoments) {
+                    // the variance rt_resolve_variance would give: S as the float accum would hold it, k = ns = spp_total
+                    float *pv = moments.var + 3 * o;
+                    pv[0] = variance_of_mean((double)(float)a0, (double)q0, (double)ns);
+                    pv[1] = variance_of_mean((double)(float)a1, (double)q1, (double)ns);
+                    pv[2] = variance_of_mean((double)(float)a2, (double)q2, (double)ns);
+                }
                 to_accum = false;
             } else if (pp.sink == 2) {
                 // sample sharding: one 16-byte system-scope reduction into the accumulators of the pixel's owner
@@ -675,6 +697,15 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                 float4 *dst = pp.peer_accum[k] + o;
                 asm volatile("red.relaxed.sys.global.add.v4.f32 [%0], {%1, %2, %3, %4};"
                              :: "l"(dst), "f"((float)a0), "f"((float)a1), "f"((float)a2), "f"((float)ns) : "memory");
+                if constexpr (kMoments) {
+                    // the squares beside them: no vector f64 reduction exists, so four scalar ones; integer-valued
+                    // doubles below 2^53 (DESIGN.md 4.8a), exact in any order
+                    double *qd = reinterpret_cast<double *>(moments.peer[k] + o);
+                    asm volatile("red.relaxed.sys.global.add.f64 [%0], %1;" :: "l"(qd), "d"((double)q0) : "memory");
+                    asm volatile("red.relaxed.sys.global.add.f64 [%0], %1;" :: "l"(qd + 1), "d"((double)q1) : "memory");
+                    asm volatile("red.relaxed.sys.global.add.f64 [%0], %1;" :: "l"(qd + 2), "d"((double)q2) : "memory");
+                    asm volatile("red.relaxed.sys.global.add.f64 [%0], %1;" :: "l"(qd + 3), "d"((double)ns) : "memory");
+                }
                 to_accum = false;
             }
         }
@@ -688,10 +719,10 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
             if constexpr (kMoments) {
                 double4 m = make_double4((double)q0, (double)q1, (double)q2, (double)ns);
                 if (pp.accumulate) {
-                    const double4 old = moments[o];
+                    const double4 old = moments.local[o];
                     m.x += old.x; m.y += old.y; m.z += old.z; m.w += old.w;
                 }
-                moments[o] = m;
+                moments.local[o] = m;
             }
         }
     }
@@ -711,7 +742,8 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     if (lane_ == 0) {
         // every warp of the launch passes here exactly once, after its last fetch: the last one re-arms the counters
         // and, under the frame protocol, publishes this rank's part (its peer writes, and through the fence + counter
-        // chain those of every other warp, are ordered before the release stores)
+        // chain those of every other warp, are ordered before the release stores; the system fence orders the kMoments
+        // f64 reductions into the owners' moments as it orders the f32 ones into their accumulators)
         if (sync) __threadfence_system(); else __threadfence();
         if (atomicAdd(pp.sched + 1, 1u) == (gridDim.x << 3) - 1u) {
             if (sync) {
@@ -742,6 +774,18 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
                     float *px = pp.image + 3 * o;
                     px[0] = (float)(r < 1.0 ? r : 1.0); px[1] = (float)(g < 1.0 ? g : 1.0); px[2] = (float)(b < 1.0 ? b : 1.0);
                     __stcg(own + o, make_float4(0.f, 0.f, 0.f, 0.f));
+                    if constexpr (kMoments) {
+                        // the own band of the moments -> rank 0's variance image, as rt_resolve_variance would
+                        // resolve the reduced frame; cleared for the frame after next like the sums
+                        double2 *qo = reinterpret_cast<double2 *>(moments.peer[pp.rank] + o);
+                        const double2 qa = __ldcg(qo), qb = __ldcg(qo + 1);
+                        RT_ASSERT(qb.y == (double)pp.spp_total);
+                        float *pv = moments.var + 3 * o;
+                        pv[0] = variance_of_mean((double)a.x, qa.x, qb.y);
+                        pv[1] = variance_of_mean((double)a.y, qa.y, qb.y);
+                        pv[2] = variance_of_mean((double)a.z, qb.x, qb.y);
+                        __stcg(qo, make_double2(0.0, 0.0)); __stcg(qo + 1, make_double2(0.0, 0.0));
+                    }
                 }
                 __syncthreads();
                 if (threadIdx.x == 0) {
@@ -1046,9 +1090,8 @@ __global__ void resolve_kernel(const typename M<T>::v4 *accum, int W, int y0, in
     image[3 * o + 2] = (float)(b < 1.0 ? b : 1.0);
 }
 
-// variance of the pixel's mean in colour levels^2, from the sums S (accum) and the sums of squares Q (moments) of its n
-// samples: (Q - S^2/n) / (n (n-1)), evaluated as (n Q - S^2) / (n^2 (n-1)) -- the numerator is exact while n Q and S^2
-// stay below 2^53 (integer colours), so a pixel whose samples all agree gets exactly 0; 0 where n < 2
+// variance of the pixel's mean in colour levels^2 (variance_of_mean) from the sums S (accum) and the sums of squares Q
+// (moments) of its n samples
 template <typename T>
 __global__ void resolve_variance_kernel(const typename M<T>::v4 *accum, const double4 *moments, int W, int y0, int y1,
                                         float *var) {
@@ -1060,14 +1103,7 @@ __global__ void resolve_variance_kernel(const typename M<T>::v4 *accum, const do
     const double4 q = moments[o];
     const double k = q.w, S[3] = {(double)a.x, (double)a.y, (double)a.z}, Q[3] = {q.x, q.y, q.z};
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        double v = 0.0;
-        if (k >= 2.0) {
-            v = __ddiv_rn(__dsub_rn(__dmul_rn(k, Q[c]), __dmul_rn(S[c], S[c])), __dmul_rn(__dmul_rn(k, k), k - 1.0));
-            v = v > 0.0 ? v : 0.0;
-        }
-        var[3 * o + c] = (float)v;
-    }
+    for (int c = 0; c < 3; ++c) var[3 * o + c] = variance_of_mean(S[c], Q[c], k);
 }
 
 // ------------------------------------------------------------------ batched primitives
@@ -1565,28 +1601,28 @@ cudaError_t launch_whitted(const SceneDev<T> &sc, const WhittedDev<T> &wp, void 
 
 template <typename T>
 cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathLaunch &pl, void *accum,
-                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, double *moments) {
+                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, const MomentsDev *moments) {
     if (pp.y1 <= pp.y0 || pp.W <= 0) return cudaSuccess;
     const long long tiles_total = (long long)pp.gx * pp.gy + (long long)pp.gx2 * pp.gy2;
     dim3 grid(1), block(256);
     using v4 = typename M<T>::v4;
     const size_t sm = pl.smem;
     cudaError_t e = cudaSuccess;
-    double4 *const mom = reinterpret_cast<double4 *>(moments);
+    const MomentsDev *const mom = moments;
     // one launch of path_kernel<T, M_, F_, Q_>; SMOPT_: the shared memory to opt in to, PKC_: the parameter-block
-    // scene (kMode 3), MOM_: the moments buffer (Q_ = true)
+    // scene (kMode 3), MOM_: the moments sinks (Q_ = true)
 #define RT_PATH_LAUNCH(M_, F_, Q_, SMOPT_, PKC_, MOM_)                                                               \
     { e = allow_smem(path_kernel<T, M_, F_, Q_>, SMOPT_); if (e != cudaSuccess) return e;                          \
       grid.x = persistent_ctas(path_kernel<T, M_, F_, Q_>, sm, tiles_total);                                       \
       if (pp.max_ctas > 0 && grid.x > (unsigned)pp.max_ctas) grid.x = (unsigned)pp.max_ctas;                        \
       path_kernel<T, M_, F_, Q_><<<grid, block, sm, st>>>(sc, pp, (v4 *)accum, stats, PKC_, MOM_); }
 #define RT_PATH_CASE(M_, F_)                                                                                       \
-    { if (mom) RT_PATH_LAUNCH(M_, F_, true, sm, PkNone(), mom) else RT_PATH_LAUNCH(M_, F_, false, sm, PkNone(), PkNone()) }
+    { if (mom) RT_PATH_LAUNCH(M_, F_, true, sm, PkNone(), *mom) else RT_PATH_LAUNCH(M_, F_, false, sm, PkNone(), PkNone()) }
     if (pl.mode == 3) {
         if constexpr (sizeof(T) == 4) {
             // + the static arrays: opt in above 48 KB in all
 #define RT_PATH_CASE3(F_)                                                                                          \
-    { if (mom) RT_PATH_LAUNCH(3, F_, true, sm ? sm + 8192 : 0, *pkc, mom)                                          \
+    { if (mom) RT_PATH_LAUNCH(3, F_, true, sm ? sm + 8192 : 0, *pkc, *mom)                                          \
       else RT_PATH_LAUNCH(3, F_, false, sm ? sm + 8192 : 0, *pkc, PkNone()) }
             if (pp.int_fold) RT_PATH_CASE3(true) else RT_PATH_CASE3(false)
 #undef RT_PATH_CASE3
@@ -1727,7 +1763,7 @@ cudaError_t launch_env_step(const SceneDev<T> &sc, const EnvDev<T> &e, const flo
     template cudaError_t launch_whitted<T>(const SceneDev<T> &, const WhittedDev<T> &, void *, int *,                   \
                                            unsigned long long *, cudaStream_t, unsigned *, unsigned *, unsigned *);     \
     template cudaError_t launch_path<T>(const SceneDev<T> &, const PathDev<T> &, const PathLaunch &, void *,           \
-                                        unsigned long long *, cudaStream_t, const PkConst *, double *);                 \
+                                        unsigned long long *, cudaStream_t, const PkConst *, const MomentsDev *);       \
     template cudaError_t launch_resolve<T>(const void *, int, int, int, int, float *, cudaStream_t);                    \
     template cudaError_t launch_resolve_variance<T>(const void *, const double *, int, int, int, float *, cudaStream_t); \
     template cudaError_t launch_trajectories<T>(const SceneDev<T> &, int, int, int, uint64_t, float *, float *, float *,  \

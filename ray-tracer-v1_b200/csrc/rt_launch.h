@@ -139,11 +139,18 @@ cudaError_t launch_whitted(const SceneDev<T> &sc, const WhittedDev<T> &wp, void 
 // samples of a pixel with FP32 reductions in no fixed order)
 // kernel variant (kMode) and dynamic shared memory of a path-kernel launch (plan_path_launch, rt_api.cu)
 struct PathLaunch { int mode; size_t smem; };
+// where the kMoments path kernels put the second moments (sum r^2, sum g^2, sum b^2, n): the kernel's trailing parameter,
+// not fields of PathDev, whose layout the plain kernels' instruction schedule depends on
+struct MomentsDev {
+    double4 *local;              // RT_SINK_ACCUM: [H,W,4] doubles, stored like accum
+    double4 *peer[16];           // RT_SINK_SCATTER_ADD: the owners' [H,W,4] moments (own at [rank], peer mappings elsewhere)
+    float *var;                  // RT_SINK_IMAGE, and RT_SINK_SCATTER_ADD under sync: rank 0's [H,W,3] variance image
+};
 template <typename T>
 cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathLaunch &pl, void *accum,
-                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, double *moments);
+                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, const MomentsDev *moments);
 // pkc: host copy of the FP32 pair arrays, read by kMode 3; pp.sched: two zeroed device counters owned by this launch;
-// moments: NULL, or [H,W,4] doubles that receive (sum r^2, sum g^2, sum b^2, n) like accum (the kMoments kernels)
+// moments: NULL (plain kernels), or the moments sinks of the kMoments kernels
 template <typename T>
 cudaError_t launch_trajectories(const SceneDev<T> &sc, int n_traj, int max_steps, int max_bounces, uint64_t seed, float *obs,
                                 float *action, float *next_obs, float *reward, uint8_t *hit, int *length,
@@ -155,6 +162,9 @@ template <typename T>
 cudaError_t launch_resolve(const void *accum, int W, int y0, int y1, int spp, float *image, cudaStream_t st);
 // rt_f32.cu: resolve + clear, peer flags
 cudaError_t launch_resolve_clear(float4 *accum, int W, int y0, int y1, int spp, float *image, int clear, cudaStream_t st);
+// the same with the moments: also the variance of rows [y0,y1) into var (rt_resolve_variance), and clear both buffers' rows
+cudaError_t launch_resolve_clear_moments(float4 *accum, double4 *moments, int W, int y0, int y1, int spp, float *image,
+                                         float *var, int clear, cudaStream_t st);
 struct PeerFlagTable { unsigned *p[32]; };      // flag addresses ride in the kernel's parameter block
 cudaError_t launch_peer_signal(const PeerFlagTable &flags, int n, unsigned epoch, cudaStream_t st);
 cudaError_t launch_peer_wait(const unsigned *flags, int n, unsigned epoch, long long timeout_cycles, int *timed_out,

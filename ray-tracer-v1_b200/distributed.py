@@ -7,6 +7,8 @@ The path shards three ways (SURVEY.md section 8e); each needs at most ONE collec
 * samples  -- sample ranges of every pixel, one per rank (C4: chandelier at high spp).  One NCCL reduce(sum) of the
               FP32 [H,W,4] accumulation buffers to rank 0, then the ``// spp`` resolve there.  Per-sample colours are
               integers, so FP32 sums are exact below 2^24 and the reduced frame is bit-identical to the unsharded one.
+              With ``variance=True`` the float64 second moments are reduced the same way (integer-valued doubles below
+              2^53: exact), so the variance image is bit-identical too.
 * env      -- environment slices (C5): no collective at all, see ray_tracer_env.BatchedRayTracerEnv.shard.
 
 Because the Philox stream is keyed by the GLOBAL (pixel, sample, bounce), a sharded frame equals the unsharded frame
@@ -256,9 +258,26 @@ class ShardedPathRenderer:
             self._frame = 0
             self._key = (W, H)
 
-    def _to_host(self, src, slot, release=None):
-        """Queue the device->host copy of ``src`` on the copy stream (after everything the current stream has queued)
-        into pinned slot ``slot``; ``release`` (optional) runs on the copy stream after the copy."""
+    def _ensure_host_vars(self, W, H):
+        """Pinned, double-buffered host slots of the variance image (first variance frame of a size only)."""
+        if getattr(self, "_host_var_key", None) != (W, H):
+            self.host_vars = [self.torch.empty((H, W, 3), dtype=self.torch.float32, pin_memory=True) for _ in (0, 1)]
+            self._host_var_key = (W, H)
+
+    def _ensure_variance(self, W, H):
+        """float64 second moments [H,W,4] and double-buffered variance images, allocated by the first variance frame."""
+        torch = self.torch
+        if getattr(self, "_var_key", None) != (W, H):
+            dev = torch.device("cuda", self.device)
+            self.moments = torch.zeros((H, W, 4), dtype=torch.float64, device=dev)
+            self.vars = [torch.zeros((H, W, 3), dtype=torch.float32, device=dev) for _ in (0, 1)]
+            self._var_key = (W, H)
+        self._ensure_host_vars(W, H)
+
+    def _to_host(self, src, slot, release=None, var=None):
+        """Queue the device->host copy of ``src`` (and of the variance image ``var``, if given) on the copy stream (after
+        everything the current stream has queued) into pinned slot ``slot``; ``release`` (optional) runs on the copy
+        stream after the copies.  -> (PendingFrame of the image, PendingFrame of the variance or None)."""
         torch = self.torch
         ready = torch.cuda.Event()
         ready.record()
@@ -266,25 +285,47 @@ class ShardedPathRenderer:
         cs.wait_event(ready)
         with torch.cuda.stream(cs):
             self.host_images[slot].copy_(src, non_blocking=True)
+            if var is not None:
+                self.host_vars[slot].copy_(var, non_blocking=True)
             # the frame is on the host once the COPY is done: the event must not sit behind the release launch, which
             # (a kernel) cannot start while the next frame's persistent kernel holds every SM -- it would report the
             # frame a whole frame late and stall a caller that reads frame f before it issues frame f + 2
             self._copied[slot].record(cs)
             if release is not None:
                 release(cs.cuda_stream)
-        self.d2h_bytes = self.host_images[slot].numel() * 4
-        return PendingFrame(self.host_images[slot], self._copied[slot])
+        self.d2h_bytes = self.host_images[slot].numel() * 4 * (1 if var is None else 2)
+        return (PendingFrame(self.host_images[slot], self._copied[slot]),
+                None if var is None else PendingFrame(self.host_vars[slot], self._copied[slot]))
 
-    def render(self, cam, W, H, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, mode="tiles", to_host=False):
+    def _deliver(self, image, var, slot, to_host, release=None):
+        """Rank 0's (image, variance or None) in the form ``to_host`` asks for."""
+        if not to_host:
+            return image, var
+        pi, pv = self._to_host(image, slot, release, var)
+        if to_host == "async":
+            return pi, pv
+        return pi.result(), (None if pv is None else pv.result())
+
+    def render(self, cam, W, H, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, mode="tiles", to_host=False,
+               variance=False):
         """Render one frame cooperatively.  Returns (image, stats) on rank 0 -- image a CUDA tensor [H,W,3] float32, a
         numpy view of pinned host memory when ``to_host`` is True, or a ``PendingFrame`` when ``to_host == "async"``
         (the copy runs on a second stream while the next frame renders) -- and (None, stats) elsewhere.  stats = this
-        rank's uint64[8] counter block as a CUDA int64 tensor (not reduced: callers sum what they need)."""
+        rank's uint64[8] counter block as a CUDA int64 tensor (not reduced: callers sum what they need).
+
+        ``variance=True`` (the same on every rank of a frame): also the variance of each pixel's mean in colour
+        levels^2, [H,W,3] float32, bit-identical to ``render_path(..., variance=True)`` of the unsharded frame.  The
+        call then returns (image, stats, var) on rank 0, var of the same kind as image, and (None, stats, None)
+        elsewhere."""
         torch, nat, sc = self.torch, self.nat, self.scene
         self._ensure(W, H)
+        if variance:
+            self._ensure_variance(W, H)
         self._frame += 1
         slot = self._frame & 1
         self.image = self.images[slot]
+        var = self.vars[slot] if variance else None
+        moments = self.moments if variance else None
         torch.cuda.current_stream().wait_event(self._copied[slot])         # slot's previous copy-out has finished
         rows = (0, H)
         samples = (0, spp)
@@ -298,24 +339,34 @@ class ShardedPathRenderer:
         self.stats.zero_()
         if mode == "samples" and samples[0] == samples[1]:
             self.accum.zero_()
+            if variance:
+                moments.zero_()
         p = sc.path_params(cam, W, H, spp, max_bounces, mirror_threshold, seed=seed, fov=fov, rows=rows, samples=samples)
-        sc.render_path(p, self.accum, self.precision, stats=self.stats)
+        sc.render_path(p, self.accum, self.precision, stats=self.stats, moments=moments)
         self.launches = 1
         if mode == "tiles":
             sc.resolve(self.accum, W, H, spp, self.image, self.precision, rows=rows)
             self.launches += 1
+            if variance:
+                sc.resolve_variance(self.accum, moments, W, H, var, self.precision, rows=rows)
+                self.launches += 1
             gather_row_bands(self.image, bands, self.group)
+            if variance:
+                gather_row_bands(var, bands, self.group)
         else:
             reduce_sample_sums(self.accum, self.group)
+            if variance:
+                reduce_sample_sums(moments, self.group)
             if self.rank == 0:
                 sc.resolve(self.accum, W, H, spp, self.image, self.precision)
                 self.launches += 1
+                if variance:
+                    sc.resolve_variance(self.accum, moments, W, H, var, self.precision)
+                    self.launches += 1
         if self.rank != 0:
-            return None, self.stats
-        if to_host:
-            pending = self._to_host(self.image, slot)
-            return (pending if to_host == "async" else pending.result()), self.stats
-        return self.image, self.stats
+            return (None, self.stats, None) if variance else (None, self.stats)
+        image, var = self._deliver(self.image, var, slot, to_host)
+        return (image, self.stats, var) if variance else (image, self.stats)
 
     # ---- fused sinks over NVLink peer memory ------------------------------------------------------------------
     def _ensure_fabric(self, W, H):
@@ -336,9 +387,24 @@ class ShardedPathRenderer:
         if not hasattr(self, "host_image") or self._key != (W, H):
             self._ensure(W, H)
         self._fab_key = (W, H)
+        self._fab_var = False
+
+    def _ensure_fabric_variance(self, W, H):
+        """Peer-mapped, double-buffered second moments (one [H,W,4] float64 per rank) and variance images (rank 0's),
+        allocated by the first variance frame.  Collective, like the frame itself; freshly zeroed, and the epochs and
+        flags of the existing buffers are left as they are."""
+        if self._fab_var:
+            return
+        torch, fab = self.torch, self.fabric
+        fab.alloc("moments0", H * W * 32); fab.alloc("moments1", H * W * 32)
+        fab.alloc("var0", H * W * 3 * 4); fab.alloc("var1", H * W * 3 * 4)
+        self._fused_vars = [torch.as_tensor(_DevArray(fab.ptrs[f"var{k}"][self.rank], (H, W, 3), "<f4"),
+                                            device=torch.device("cuda", self.device)) for k in (0, 1)]
+        self._ensure_host_vars(W, H)
+        self._fab_var = True
 
     def render_fused(self, cam, W, H, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, mode="tiles", to_host=False,
-                     kernel_events=None, in_kernel=True):
+                     kernel_events=None, in_kernel=True, variance=False):
         """The same frame as ``render`` with the collective fused into the path kernel: no NCCL call on the data path.
 
         tiles    every rank renders interleaved 8-row stripes (tile_stripes) and its path kernel stores the resolved
@@ -354,12 +420,19 @@ class ShardedPathRenderer:
         PROVIDED its consumer is queued on the current stream before the next ``render_fused`` call (the "consumed"
         signal of frame f is published by rank 0's stream at the start of frame f+1, i.e. after everything queued in
         between; with ``to_host`` it follows the copy-out on the copy stream).  kernel_events = (start, end) CUDA
-        events recorded around the path kernel alone (bench.py's roofline)."""
+        events recorded around the path kernel alone (bench.py's roofline).
+
+        ``variance=True``: the per-pixel variance travels through the same sinks -- tiles: the path kernel also stores
+        each resolved pixel's variance into rank 0's variance image; samples: it also adds the squared colours into the
+        owner's float64 moments, which the band resolve turns into rank 0's variance image.  Returns (image, stats,
+        var) as ``render`` does.  Like ``mode``, ``variance`` must be the same on every rank for a given frame."""
         nat, sc, torch = self.nat, self.scene, self.torch
-        self._ensure_fabric(W, H)
-        fab, rank, world = self.fabric, self.rank, self.world
         if mode not in ("tiles", "samples"):
             raise ValueError("mode must be 'tiles' or 'samples'")
+        self._ensure_fabric(W, H)
+        if variance:
+            self._ensure_fabric_variance(W, H)
+        fab, rank, world = self.fabric, self.rank, self.world
         self._epoch += 1
         e, buf = self._epoch, self._epoch & 1
         everyone = list(range(world))
@@ -382,6 +455,13 @@ class ShardedPathRenderer:
             sink.band_y[world] = H
         sink.world = world
         sink.image = fab.ptrs[f"image{buf}"][0]
+        msink = None
+        if variance:
+            msink = nat.PathMomentsSink()
+            msink.var = fab.ptrs[f"var{buf}"][0]
+            if mode == "samples":
+                for k in range(world):
+                    msink.moments[k] = fab.ptrs[f"moments{buf}"][k]
         pending_go, self._pending_go = getattr(self, "_pending_go", 0), 0
         if in_kernel:
             sink.sync, sink.rank, sink.epoch, sink.spp_total = 1, rank, e, spp
@@ -391,7 +471,7 @@ class ShardedPathRenderer:
             sink.timed_out = self._timed_out.data_ptr()
             if kernel_events:
                 kernel_events[0].record()
-            sc.render_path_sink(p, sink, stats=self.stats)                     # ONE launch: the frame is complete on rank 0 when it ends
+            sc.render_path_sink(p, sink, stats=self.stats, moments_sink=msink)   # ONE launch: the frame is complete on rank 0 when it ends
             if kernel_events:
                 kernel_events[1].record()
             self.launches = 1
@@ -402,7 +482,7 @@ class ShardedPathRenderer:
             if mode == "tiles":
                 if kernel_events:
                     kernel_events[0].record()
-                sc.render_path_sink(p, sink, stats=self.stats)
+                sc.render_path_sink(p, sink, stats=self.stats, moments_sink=msink)
                 if kernel_events:
                     kernel_events[1].record()
                 self.launches = 3 + (2 if rank == 0 else 0)
@@ -410,30 +490,36 @@ class ShardedPathRenderer:
                 if kernel_events:
                     kernel_events[0].record()
                 if s1 > s0:
-                    sc.render_path_sink(p, sink, stats=self.stats)
+                    sc.render_path_sink(p, sink, stats=self.stats, moments_sink=msink)
                 if kernel_events:
                     kernel_events[1].record()
                 fab.signal("flags", rank, everyone, e)                         # my sums have been added everywhere
                 fab.wait("flags", 0, world, e, self._timed_out)                # everyone's sums are in my band
                 y0, y1 = bands[rank]
-                nat.check(nat.lib().rt_resolve_clear(self.device, fab.ptrs[f"accum{buf}"][rank], W, H, y0, y1, spp,
-                                                     fab.ptrs[f"image{buf}"][0], 1, None))
+                if variance:
+                    nat.check(nat.lib().rt_resolve_clear_moments(self.device, fab.ptrs[f"accum{buf}"][rank],
+                                                                 fab.ptrs[f"moments{buf}"][rank], W, H, y0, y1, spp,
+                                                                 fab.ptrs[f"image{buf}"][0], fab.ptrs[f"var{buf}"][0], 1,
+                                                                 None))
+                else:
+                    nat.check(nat.lib().rt_resolve_clear(self.device, fab.ptrs[f"accum{buf}"][rank], W, H, y0, y1, spp,
+                                                         fab.ptrs[f"image{buf}"][0], 1, None))
                 self.launches = 6 + (2 if rank == 0 else 0)     # wait, path, signal, wait, resolve, signal (+ wait, signal)
             fab.signal("flags", 16 + rank, [0], e)                             # my part of rank 0's image is written
             if rank == 0:
                 fab.wait("flags", 16, world, e, self._timed_out)
-        out = None
+        out = var = None
         if rank == 0:
-            out = self._fused_images[buf]
+            out, var = self._fused_images[buf], (self._fused_vars[buf] if variance else None)
             if to_host:
                 # the copy-out runs on the copy stream; the "consumed" signal follows it there
-                pending = self._to_host(out, buf, release=lambda st: fab.signal("flags", 32, everyone, e, stream=st))
-                out = pending if to_host == "async" else pending.result()
+                out, var = self._deliver(out, var, buf, to_host,
+                                         release=lambda st: fab.signal("flags", 32, everyone, e, stream=st))
             else:
                 # the caller's consumer of this CUDA image comes AFTER this call: publish "consumed" at the start of the
                 # next frame on this stream (in the kernel's own prologue), never right away
                 self._pending_go = e
-        return out, self.stats
+        return (out, self.stats, var) if variance else (out, self.stats)
 
     def fused_timed_out(self):
         return bool(int(self._timed_out.item())) if getattr(self, "_timed_out", None) is not None else False

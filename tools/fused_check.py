@@ -4,6 +4,10 @@ for bit, device-timed side by side.
 
     python tools/fused_check.py                                   # 1 GPU (peers = self)
     torchrun --nproc-per-node N --master-addr 127.0.0.1 tools/fused_check.py [--spp 64]
+
+--variance: per-pixel variance through every path instead.  For each mode, rank 0's variance from render and from
+render_fused (single launch and chain) is compared bit for bit with the 1-GPU render_path(..., variance=True), each
+image with the same call without variance, and plain and variance frames of every path are timed alternately.
 """
 import argparse
 import json
@@ -29,6 +33,7 @@ def main():
     ap.add_argument("--h", type=int, default=1080)
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--scene", default="complex")
+    ap.add_argument("--variance", action="store_true", help="check and time the per-pixel variance of every path")
     args = ap.parse_args()
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
     torch.cuda.set_device(local)
@@ -47,6 +52,16 @@ def main():
         torch.cuda.synchronize()
 
     out = {"world": world, "scene": args.scene, "spp": spp}
+    if args.variance:
+        out["variance"] = True
+        check_variance(args, r, spec, fs, rank, world, sync, out)
+        out["timed_out"] = r.fused_timed_out()
+        if rank == 0:
+            print(json.dumps(out), flush=True)
+        r.close()
+        if world > 1:
+            dist.destroy_process_group()
+        return
     for mode in ("tiles", "samples"):
         ref, _ = r.render(spec.camera, W, H, spp, depth, thr, seed=3, mode=mode)
         ref = ref.clone() if rank == 0 else None
@@ -80,6 +95,46 @@ def main():
     r.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+def check_variance(args, r, spec, fs, rank, world, sync, out):
+    """Bit-exactness of every path's variance against one GPU, and plain vs variance ms/frame of every path."""
+    W, H, spp = args.w, args.h, args.spp
+    depth, thr = spec.max_bounces, spec.mirror_threshold
+    cam = spec.camera
+    ref_var = None
+    if rank == 0:
+        from ray_tracer_v1_b200.renderers import render_path
+        _, _, ref_var = render_path(fs, cam, W, H, spp, depth, thr, seed=3, variance=True)
+    paths = {"nccl": r.render, "fused": r.render_fused,
+             "chain": lambda *a, **k: r.render_fused(*a, in_kernel=False, **k)}
+    for mode in ("tiles", "samples"):
+        for name, fn in paths.items():
+            img, _ = fn(cam, W, H, spp, depth, thr, seed=3, mode=mode)
+            img = img.clone() if rank == 0 else None
+            img_v, _, var = fn(cam, W, H, spp, depth, thr, seed=3, mode=mode, variance=True)
+            sync()
+            if rank == 0:
+                out[f"{mode}_{name}_var_identical"] = bool(np.array_equal(var.cpu().numpy(), ref_var))
+                out[f"{mode}_{name}_image_identical"] = bool(torch.equal(img, img_v))
+        for name, fn in paths.items():
+            for variance in (False, True):                  # warm both kernels
+                fn(cam, W, H, spp, depth, thr, seed=10, mode=mode, variance=variance)
+            sync()
+            times = {False: [], True: []}
+            for i in range(2 * args.reps):                    # alternate plain and variance frames
+                variance = bool(i & 1)
+                a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                a.record()
+                fn(cam, W, H, spp, depth, thr, seed=20 + i, mode=mode, variance=variance)
+                b.record()
+                sync()
+                times[variance].append(a.elapsed_time(b))
+            for variance, key in ((False, "ms"), (True, "var_ms")):
+                t = torch.tensor([float(np.median(times[variance]))], device="cuda")
+                if world > 1:
+                    dist.all_reduce(t, op=dist.ReduceOp.MAX)
+                out[f"{mode}_{name}_{key}"] = round(float(t), 3)
 
 
 if __name__ == "__main__":
