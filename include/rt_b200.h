@@ -188,6 +188,27 @@ int rt_render_path(rt_scene *scene, int precision, const rt_path_params *p, void
  * bit-identical to rt_render_path's. */
 int rt_render_path_moments(rt_scene *scene, int precision, const rt_path_params *p, void *accum_dev,
                            double *moments_dev, uint64_t *stats_dev, void *stream);
+/* Adaptive Algorithm B frame over rows [y0,y1): every pixel gets samples [0, min_spp); then, at the checkpoints
+ * c0 = min_spp, c(r+1) = min(2 c(r), max_spp = p->s1), a pixel that received samples up to c(r) and whose variance of
+ * the mean (what rt_resolve_variance gives, levels^2) exceeds tolerance^2 in some channel gets samples [c(r), c(r+1)).
+ * tolerance is in colour levels (0-255 scale); a negative one takes every pixel to max_spp.  Each pixel equals, bit for
+ * bit, the uniform frame rendered with its own final sample count n (accum, moments, image, variance).
+ * accum_dev / moments_dev as rt_render_path_moments (overwritten in the band); list_dev: uint32 scratch of
+ * (y1-y0)*W + 1 words (the active pixels and their count); image_dev [H,W,3] float32 = min(1, floor(S/n)/255);
+ * var_dev (optional) [H,W,3] float32 variance of the mean; counts_dev (optional) [H,W] int32 = n.  stats_dev sums
+ * over the rounds (sphere / AABB tests depend on how the rounds group the pixels).
+ * The call synchronises the stream once per round to read the active count; the final resolve is enqueued on the
+ * stream when it returns.  Integer colours only (RT_ERR_UNSUPPORTED otherwise), and in FP32 max_colour * max_spp < 2^24
+ * (max_colour 255 for byte colours, else 65535).  RT_ERR_INVALID for p->s0 != 0, p->accumulate, min_spp outside
+ * [2, max_spp], a NaN tolerance, max_spp > 65536 or unknown schedule bits. */
+typedef struct rt_adaptive_params {
+    int32_t min_spp;
+    int32_t reserved_;
+    double tolerance;
+} rt_adaptive_params;
+int rt_render_path_adaptive(rt_scene *scene, int precision, const rt_path_params *p, const rt_adaptive_params *a,
+                            void *accum_dev, double *moments_dev, uint32_t *list_dev, float *image_dev, float *var_dev,
+                            int32_t *counts_dev, uint64_t *stats_dev, void *stream);
 /* TraditionalRenderer.trace_ray_traditional(ray, bounce_count) (FB/fb_vs_traditional_chandelier.py:431-521) for n
  * explicit rays at once: rays_dev [n,6] doubles = origin, direction AS GIVEN (Ray() has normalised it); the path starts
  * at recursion depth bounce_count (a call with bounce_count >= max_bounces returns (2,2,5)); ray i draws its bounce

@@ -65,6 +65,12 @@ class PathParams(C.Structure):
                 ("schedule", C.c_int32), ("ksplit", C.c_int32), ("reserved_", C.c_int32)]
 
 
+class AdaptiveParams(C.Structure):
+    """rt_adaptive_params: samples [0, min_spp) for every pixel, then doubling rounds for the pixels whose variance of the
+    mean exceeds ``tolerance``^2 (colour levels, 0-255 scale; negative: every pixel to max_spp)."""
+    _fields_ = [("min_spp", C.c_int32), ("reserved_", C.c_int32), ("tolerance", C.c_double)]
+
+
 class SimpleParams(C.Structure):
     _fields_ = [("cam", C.c_double * 3), ("W", C.c_int32), ("H", C.c_int32), ("fov_rad", C.c_double),
                 ("sun_pos", C.c_double * 3), ("sun_col", C.c_double * 3), ("sun_id", C.c_int32), ("max_bounces", C.c_int32),
@@ -129,6 +135,8 @@ SIGNATURES = {
     "rt_render_whitted": (C.c_int, [vp, C.c_int, C.POINTER(WhittedParams), vp, vp, vp, vp]),
     "rt_render_path": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), vp, vp, vp]),
     "rt_render_path_moments": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), vp, vp, vp, vp]),
+    "rt_render_path_adaptive": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), C.POINTER(AdaptiveParams), vp, vp, vp, vp, vp,
+                                          vp, vp, vp]),
     "rt_trace_paths": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), C.c_int32, vp, vp, C.c_int32, vp, vp, vp]),
     "rt_resolve": (C.c_int, [C.c_int, C.c_int, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
     "rt_resolve_variance": (C.c_int, [C.c_int, C.c_int, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
@@ -475,6 +483,17 @@ class DeviceScene:
         else:
             check(lib().rt_render_path_moments(self.handle, precision, C.byref(params), _ptr(accum), _ptr(moments),
                                                _ptr(stats), stream))
+
+    def render_path_adaptive(self, params, min_spp, tolerance, accum, moments, pixel_list, image, precision=F32, var=None,
+                             counts=None, stats=None, stream=None):
+        """Adaptive frame (``rt_render_path_adaptive``): ``params.s1`` is max_spp; every pixel of the band gets
+        ``min_spp`` samples, then doubling rounds for the pixels whose variance of the mean exceeds ``tolerance``^2.
+        ``pixel_list``: uint32 scratch of (y1 - y0) * W + 1 words.  Resolves into ``image`` (and ``var`` float32
+        [H,W,3], ``counts`` int32 [H,W] when given) on the stream; synchronises the stream once per round."""
+        a = AdaptiveParams()
+        a.min_spp, a.tolerance = int(min_spp), float(tolerance)
+        check(lib().rt_render_path_adaptive(self.handle, precision, C.byref(params), C.byref(a), _ptr(accum), _ptr(moments),
+                                            _ptr(pixel_list), _ptr(image), _ptr(var), _ptr(counts), _ptr(stats), stream))
 
     def trace_paths(self, rays, max_bounces, mirror_threshold, bounce_count=0, seed=0, ray_ids=None, samples=(0, 1),
                     precision=F64):

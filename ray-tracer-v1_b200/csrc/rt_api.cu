@@ -76,6 +76,7 @@ struct rt_scene {
     mutable std::atomic<unsigned> sched_next{0}; // launches rotate through the slots, so launches in flight never share a pair
     PkConst pkc;                  // host copy of the FP32 sphere pairs of a small scene (path kernel parameter block)
     bool pkc_ok = false;
+    uint32_t *adaptive_count = nullptr;  // pinned word: an adaptive frame reads each round's active-pixel count into it
 };
 
 struct rt_env {
@@ -345,7 +346,7 @@ static inline cudaStream_t S(void *stream) { return reinterpret_cast<cudaStream_
 
 // ------------------------------------------------------------------ library / device
 RT_EXPORT const char *rt_last_error(void) { return g_err.c_str(); }
-RT_EXPORT int rt_version(void) { return 102; }
+RT_EXPORT int rt_version(void) { return 103; }
 
 RT_EXPORT int rt_device_count(int *count) {
     if (!count) return fail(RT_ERR_INVALID, "count is NULL");
@@ -514,6 +515,7 @@ RT_EXPORT int rt_scene_destroy(rt_scene *scene) {
     if (scene->sched_dev) cudaFree(scene->sched_dev);
     if (scene->heavy_dev) cudaFree(scene->heavy_dev);
     if (scene->stage) cudaFreeHost(scene->stage);
+    if (scene->adaptive_count) cudaFreeHost(scene->adaptive_count);
     if (scene->staged) cudaEventDestroy(scene->staged);
     for (rt_scene::Grid &g : scene->grids) grid_free(g);
     scene->grids.clear();
@@ -673,11 +675,14 @@ template <typename T> static void path_camera(PathDev<T> &pp, const rt_path_para
 // Cuts one path-kernel launch into work units: sets the band (y0, tile_step, col_*, seg_w), the sample split, both tile
 // grids and fold_tab of pp (which holds W, y1 and int_fold of the request) and returns the kernel variant and its dynamic
 // shared memory.  Every rank of a frame plans from the same numbers, so the launches of a frame tile it exactly.
+// list_count >= 0: a list launch of an adaptive frame over that many listed pixels -- the same sample split and kernel
+// choice with pixels = list_count, on one tile grid of ceil(list_count / (32 >> ksplit_log2)) units.
 template <typename T>
 static PathLaunch plan_path_launch(PathDev<T> &pp, const SceneDev<T> &sc, const rt_path_params *p, const rt_path_sink *sink,
-                                   bool xr, bool byte_colours, bool allow_pkc, int sms) {
+                                   bool xr, bool byte_colours, bool allow_pkc, int sms, long long list_count = -1) {
     const int ns = p->s1 - p->s0;
     const bool image = sink && sink->mode == RT_SINK_IMAGE;
+    const bool list = list_count >= 0;
     long long pixels = 0;
     // interleave: the 2-D interleave (rt_path_sink::col_split), one column segment of every stripe; false when a segment
     // does not hold whole work units of both tile grids (32 / 16 / 8 / 4 pixels wide for 1-2 / 4 / 8-16 / 32 lanes per pixel)
@@ -690,7 +695,7 @@ static PathLaunch plan_path_launch(PathDev<T> &pp, const SceneDev<T> &sc, const 
         }
         const int rows = pp.y1 - pp.y0, step = pp.tile_step;
         const int owned = ((rows + 7) / 8 + step - 1) / step;             // 8-row stripes of this launch
-        pixels = (long long)pp.seg_w * ((rows + step - 1) / step);
+        pixels = list ? list_count : (long long)pp.seg_w * ((rows + step - 1) / step);
         // sample split (automatic): k lanes per pixel so that a lane keeps about 8 samples -- measured best at 8, 16, 32
         // and 64 samples per launch (k = 1, 2, 4, 8: tighter camera-ray cones against per-unit overhead) -- and, for small
         // frames, more lanes per pixel until there are ~4 warp tiles per resident warp (every lane keeps >= 2 samples)
@@ -710,10 +715,16 @@ static PathLaunch plan_path_launch(PathDev<T> &pp, const SceneDev<T> &sc, const 
                 // hierarchy the units are short already)
                 int lk2 = lk + 2 < 5 ? lk + 2 : 5;
                 while (lk2 > lk && (ns >> lk2) < 2) --lk2;
-                if (sc.bvh.nodes == 0 && lk2 > lk) pp.ksplit2_log2 = lk2;
+                if (sc.bvh.nodes == 0 && lk2 > lk && !list) pp.ksplit2_log2 = lk2;
             }
         }
         pp.ksplit_log2 = lk;
+        if (list) {
+            const long long units = (list_count + (32 >> lk) - 1) >> (5 - lk);
+            pp.gx = (int)((units + 7) / 8); pp.gy = 1;
+            pp.gx2 = pp.gy2 = pp.stripe2 = 0;
+            return true;
+        }
         const int lk2 = pp.ksplit2_log2 > lk ? pp.ksplit2_log2 : lk, pw = unit_pw_log2(lk), pw2 = unit_pw_log2(lk2);
         const int ctw = 4 << pw, cth = 2 << ((5 - lk) - pw), ctw2 = 4 << pw2, cth2 = 2 << ((5 - lk2) - pw2);
         // coarse tile grid: stripes of 8 rows (8 / cth CTA rows each); without interleaving the last stripe may be cut short
@@ -750,7 +761,8 @@ static PathLaunch plan_path_launch(PathDev<T> &pp, const SceneDev<T> &sc, const 
 template <typename T>
 static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_path_params *p, void *accum, uint64_t *stats,
                          cudaStream_t st, const rt_path_sink *sink = nullptr, const ExplicitRays *xr = nullptr,
-                         double *moments = nullptr, const rt_path_moments_sink *msink = nullptr) {
+                         double *moments = nullptr, const rt_path_moments_sink *msink = nullptr,
+                         const uint32_t *list = nullptr, unsigned list_count = 0) {
     // bit 1: no camera-ray candidate lists, bit 2: no parameter-block kernel (include/rt_b200.h)
     if (p->schedule & ~6) return fail(RT_ERR_INVALID, "unknown schedule bits");
     PathDev<T> pp;
@@ -830,11 +842,16 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
     int sms = 0;
     if (device_attr(sc->device, cudaDevAttrMultiProcessorCount, &sms) != cudaSuccess || sms <= 0) sms = 148;
     const PathLaunch pl = plan_path_launch<T>(pp, view, p, sink, xr != nullptr, sc->byte_colours,
-                                              sizeof(T) == 4 && sc->pkc_ok && !(p->schedule & 4) && !xr, sms);
+                                              sizeof(T) == 4 && sc->pkc_ok && !(p->schedule & 4) && !xr, sms,
+                                              list ? (long long)list_count : -1);
     if (!sc->sched_dev) return fail(RT_ERR_INVALID, "scene has no scheduler counters (upload failed?)");
     pp.sched = sc->sched_dev + 4 * (sc->sched_next.fetch_add(1u) % RT_SCHED_SLOTS);      // {next unit, warps done, CTAs resolved, -}
+    MomentsListDev ml;
+    std::memset(&ml, 0, sizeof ml);
+    static_cast<MomentsDev &>(ml) = md;
+    ml.list = list; ml.count = list_count;
     CU(launch_path<T>(view, pp, pl, accum, reinterpret_cast<unsigned long long *>(stats), st, &sc->pkc,
-                      (moments || msink) ? &md : nullptr));
+                      (moments || msink) ? &md : nullptr, list ? &ml : nullptr));
     return RT_OK;
 }
 
@@ -860,6 +877,66 @@ RT_EXPORT int rt_render_path_moments(rt_scene *scene, int precision, const rt_pa
     if (precision == RT_F64) return render_path_t<double>(scene, scene->d.view, p, accum_dev, stats_dev, S(stream), nullptr, nullptr, moments_dev);
     if (precision == RT_F32) return render_path_t<float>(scene, scene->f.view, p, accum_dev, stats_dev, S(stream), nullptr, nullptr, moments_dev);
     return fail(RT_ERR_INVALID, "unknown precision");
+}
+
+// Adaptive frame: round 0 renders samples [0, min_spp) of every pixel of the band; after each round the select kernel
+// lists the pixels still above the tolerance, the host reads their count, and a list launch takes them to the next
+// checkpoint min(2c, s1).  Every decision is a function of exact sums, so each pixel equals the uniform frame rendered
+// at its own final count.
+template <typename T>
+static int render_path_adaptive_t(rt_scene *sc, const SceneDev<T> &view, const rt_path_params *p, const rt_adaptive_params *a,
+                                  void *accum, double *moments, uint32_t *list, float *image, float *var, int32_t *counts,
+                                  uint64_t *stats, cudaStream_t st) {
+    uint32_t *count_dev = list + (size_t)(p->y1 - p->y0) * p->W;
+    if (!sc->adaptive_count) CU(cudaMallocHost((void **)&sc->adaptive_count, sizeof(uint32_t)));
+    // a negative tolerance keeps every pixel to max_spp (a variance is never negative)
+    const double thr = a->tolerance < 0.0 ? -1.0 : a->tolerance * a->tolerance;
+    rt_path_params q = *p;
+    q.s0 = 0; q.s1 = a->min_spp;
+    int rc = render_path_t<T>(sc, view, &q, accum, stats, st, nullptr, nullptr, moments);
+    if (rc) return rc;
+    q.accumulate = 1;
+    for (int c = a->min_spp; c < p->s1;) {
+        CU(cudaMemsetAsync(count_dev, 0, sizeof(uint32_t), st));
+        CU(launch_adaptive_select<T>(accum, moments, p->W, p->y0, p->y1, c, thr, list, count_dev, st));
+        CU(cudaMemcpyAsync(sc->adaptive_count, count_dev, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        const unsigned active = *sc->adaptive_count;
+        if (active == 0u) break;
+        q.s0 = c; q.s1 = c < p->s1 - c ? 2 * c : p->s1;
+        rc = render_path_t<T>(sc, view, &q, accum, stats, st, nullptr, nullptr, moments, nullptr, list, active);
+        if (rc) return rc;
+        c = q.s1;
+    }
+    CU(launch_adaptive_resolve<T>(accum, moments, p->W, p->y0, p->y1, image, var, counts, st));
+    return RT_OK;
+}
+
+RT_EXPORT int rt_render_path_adaptive(rt_scene *scene, int precision, const rt_path_params *p, const rt_adaptive_params *a,
+                                      void *accum_dev, double *moments_dev, uint32_t *list_dev, float *image_dev,
+                                      float *var_dev, int32_t *counts_dev, uint64_t *stats_dev, void *stream) {
+    if (!scene || !p || !a || !accum_dev || !moments_dev || !list_dev || !image_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    int rc = check_band(p->W, p->H, p->y0, p->y1, p->s0, p->s1);
+    if (rc) return rc;
+    if (p->max_bounces > RT_PATH_MAX_DEPTH) return fail(RT_ERR_UNSUPPORTED, "max_bounces above 32 is not supported by the path kernel");
+    if (p->schedule & ~6) return fail(RT_ERR_INVALID, "unknown schedule bits");
+    if (p->s0 != 0) return fail(RT_ERR_INVALID, "adaptive frames start at sample 0 (s0 must be 0)");
+    if (p->accumulate) return fail(RT_ERR_INVALID, "adaptive frames do not accumulate into earlier sums (accumulate must be 0)");
+    if (p->s1 > 65536) return fail(RT_ERR_INVALID, "max_spp (s1) above 65536");
+    if (a->min_spp < 2 || a->min_spp > p->s1) return fail(RT_ERR_INVALID, "min_spp must be in [2, max_spp]");
+    if (std::isnan(a->tolerance)) return fail(RT_ERR_INVALID, "tolerance is NaN");
+    if (precision != RT_F32 && precision != RT_F64) return fail(RT_ERR_INVALID, "unknown precision");
+    if (!scene->int_colours) return fail(RT_ERR_UNSUPPORTED, "adaptive frames need integer colours");
+    // the float accum of FP32 stays exact across rounds while every sum stays below 2^24
+    const double max_colour = scene->byte_colours ? 255.0 : 65535.0;
+    if (precision == RT_F32 && max_colour * (double)p->s1 >= 16777216.0)
+        return fail(RT_ERR_UNSUPPORTED, "max_colour * max_spp >= 2^24: FP32 sums would not stay exact across rounds");
+    CU(cudaSetDevice(scene->device));
+    if (precision == RT_F64)
+        return render_path_adaptive_t<double>(scene, scene->d.view, p, a, accum_dev, moments_dev, list_dev, image_dev, var_dev,
+                                              counts_dev, stats_dev, S(stream));
+    return render_path_adaptive_t<float>(scene, scene->f.view, p, a, accum_dev, moments_dev, list_dev, image_dev, var_dev,
+                                         counts_dev, stats_dev, S(stream));
 }
 
 RT_EXPORT int rt_trace_paths(rt_scene *scene, int precision, const rt_path_params *p, int32_t n, const double *rays_dev,

@@ -359,11 +359,15 @@ template <typename T> RT_DEV V3<T> path_camera_ray(const PathDev<T> &pp, int x, 
 // added into the owner's moments.peer[k] (scatter-add sink).  The trailing parameter is empty otherwise, so the plain
 // kernels keep their parameter offsets.  Exact: an integer-fold colour is <= 65535, so its square fits a uint32 and a
 // uint64 sum of 65536 of them stays below 2^53; the double fold sums its squares in double.
-template <typename T, int kMode, bool kIntFold, bool kMoments>
+// kList (with kIntFold and kMoments only): a list launch of an adaptive frame (rt_render_path_adaptive) traces only the
+// pixels of moments.list, adding into their accum and moments: unit u takes entries [u (32 >> lk), (u + 1) (32 >> lk)).
+template <typename T, int kMode, bool kIntFold, bool kMoments, bool kList = false>
 __global__ void __launch_bounds__(256, (sizeof(T) == 4 ? (kMode == 3 ? RT_PATH_MIN_BLOCKS_PKC : RT_PATH_MIN_BLOCKS) : 1))
 path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned long long *stats,
             const __grid_constant__ typename std::conditional<kMode == 3, PkConst, PkNone>::type pkc,
-            const __grid_constant__ typename std::conditional<kMoments, MomentsDev, PkNone>::type moments) {
+            const __grid_constant__ typename std::conditional<kMoments, typename std::conditional<kList, MomentsListDev, MomentsDev>::type,
+                                                              PkNone>::type moments) {
+    static_assert(!kList || (kIntFold && kMoments), "list launches fold in integers and keep the moments");
     RT_MODE_DECL;
     using PK = typename std::conditional<kMode == 3, PkConst, PkNone>::type;
     extern __shared__ __align__(32) unsigned char smem[];
@@ -491,9 +495,16 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     // 2-D interleave: in stripe s the launch owns the column segment (col_first + s) mod col_step
     const int xs = (pp.col_step > 1 ? ((pp.col_first + (by >> cps_sh) + stripe0) % pp.col_step) * pp.seg_w : 0) +
                    (((bx << 2) + (wt & 3)) << pw_sh);             // first column of the warp's pixel block
-    const int x = xs + (pl & ((1 << pw_sh) - 1));
-    const int y = ys + (pl >> pw_sh);
-    const bool has_pixel = x < pp.W && y < pp.y1;
+    int x = xs + (pl & ((1 << pw_sh) - 1));
+    int y = ys + (pl >> pw_sh);
+    bool has_pixel = x < pp.W && y < pp.y1;
+    if constexpr (kList) {
+        const unsigned e = u_ * (32u >> lk) + (unsigned)pl;
+        has_pixel = e < moments.count;
+        const unsigned q = has_pixel ? __ldg(moments.list + e) : 0u;
+        y = (int)(q / (unsigned)pp.W); x = (int)(q - (unsigned)y * (unsigned)pp.W);
+        RT_ASSERT(!has_pixel || (y >= pp.y0 && y < pp.y1));
+    }
     const uint32_t pixel = (uint32_t)(y * pp.W + x);
     // integer-valued sums: exact in uint32 (int fold: colours <= 65535, samples per launch <= 65536) / in double
     typename std::conditional<kIntFold, unsigned, double>::type a0 = 0, a1 = 0, a2 = 0;
@@ -502,9 +513,17 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
     unsigned long long cand = ~0ull;
     bool first_trip = false;                          // warp-uniform: every live lane is about to trace its camera ray
     if constexpr (kMode == 3) if (pp.primary_cull) {
-        const int bw = 1 << pw_sh, bh = 1 << ph_sh;   // the warp's pixel block
-        const int x0 = xs;
-        const int y0 = ys;
+        int bw = 1 << pw_sh, bh = 1 << ph_sh;         // the warp's pixel block
+        int x0 = xs;
+        int y0 = ys;
+        if constexpr (kList) {
+            // list launch: the bounding box of the unit's pixels (a scattered unit only widens the cone)
+            const unsigned xlo = __reduce_min_sync(0xffffffffu, has_pixel ? (unsigned)x : 0xffffffffu);
+            const unsigned ylo = __reduce_min_sync(0xffffffffu, has_pixel ? (unsigned)y : 0xffffffffu);
+            const unsigned xhi = __reduce_max_sync(0xffffffffu, has_pixel ? (unsigned)x : 0u);
+            const unsigned yhi = __reduce_max_sync(0xffffffffu, has_pixel ? (unsigned)y : 0u);
+            if (xlo <= xhi) { x0 = (int)xlo; y0 = (int)ylo; bw = (int)(xhi - xlo) + 1; bh = (int)(yhi - ylo) + 1; }
+        }
         const V3<T> d0 = path_camera_ray<T>(pp, x0, y0, T(0.5) * T(bw), T(0.5) * T(bh));
         const float ex = 0.5f * (float)bw * (2.f / (float)pp.W) * (float)pp.aspect * (float)pp.half_w;
         const float ey = 0.5f * (float)bh * (2.f / (float)pp.H) * (float)pp.half_h;
@@ -1106,6 +1125,59 @@ __global__ void resolve_variance_kernel(const typename M<T>::v4 *accum, const do
     for (int c = 0; c < 3; ++c) var[3 * o + c] = variance_of_mean(S[c], Q[c], k);
 }
 
+// ------------------------------------------------------------------ adaptive frames (rt_render_path_adaptive)
+// After the round that took every active pixel of rows [y0, y1) to c samples: a pixel stays active when it was active
+// in that round (n == c) and the variance of its mean (variance_of_mean, the float rt_resolve_variance gives, compared in
+// double) exceeds thr in some channel.  Active pixels y * W + x are appended to list with one atomic per warp; a warp
+// covers an 8x4 tile (tile_pixel), so neighbours stay adjacent in the list.  *count is zero on entry.
+template <typename T>
+__global__ void adaptive_select_kernel(const typename M<T>::v4 *accum, const double4 *moments, int W, int y0, int y1, int c,
+                                       double thr, uint32_t *list, uint32_t *count) {
+    int x, y_rel;
+    tile_pixel(x, y_rel);
+    const int y = y0 + y_rel;
+    bool active = false;
+    if (x < W && y < y1) {
+        const size_t o = (size_t)y * W + x;
+        const typename M<T>::v4 a = accum[o];
+        const double4 q = moments[o];
+        RT_ASSERT(q.w == (double)a.w);
+        if ((double)a.w == (double)c)
+            active = (double)variance_of_mean((double)a.x, q.x, q.w) > thr || (double)variance_of_mean((double)a.y, q.y, q.w) > thr ||
+                     (double)variance_of_mean((double)a.z, q.z, q.w) > thr;
+    }
+    const unsigned ballot = __ballot_sync(0xffffffffu, active), lane = threadIdx.x & 31;
+    if (ballot == 0u) return;
+    unsigned base = 0;
+    if (lane == 0) base = atomicAdd(count, (unsigned)__popc(ballot));
+    base = __shfl_sync(0xffffffffu, base, 0);
+    if (active) list[base + (unsigned)__popc(ballot & ((1u << lane) - 1u))] = (uint32_t)(y * W + x);
+}
+
+// the adaptive frame's resolve: each pixel by its own sample count n = accum.w -- image min(1, floor(S/n)/255) as
+// resolve_kernel, the variance as resolve_variance_kernel (var optional), n into counts (optional)
+template <typename T>
+__global__ void adaptive_resolve_kernel(const typename M<T>::v4 *accum, const double4 *moments, int W, int y0, int y1,
+                                        float *image, float *var, int *counts) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t n = (size_t)(y1 - y0) * W;
+    if (i >= n) return;
+    const size_t o = (size_t)y0 * W + i;
+    const typename M<T>::v4 a = accum[o];
+    const double s = (double)a.w;
+    double r = floor((double)a.x / s) / 255.0, g = floor((double)a.y / s) / 255.0, b = floor((double)a.z / s) / 255.0;
+    image[3 * o + 0] = (float)(r < 1.0 ? r : 1.0);
+    image[3 * o + 1] = (float)(g < 1.0 ? g : 1.0);
+    image[3 * o + 2] = (float)(b < 1.0 ? b : 1.0);
+    if (var) {
+        const double4 q = moments[o];
+        var[3 * o + 0] = variance_of_mean((double)a.x, q.x, q.w);
+        var[3 * o + 1] = variance_of_mean((double)a.y, q.y, q.w);
+        var[3 * o + 2] = variance_of_mean((double)a.z, q.z, q.w);
+    }
+    if (counts) counts[o] = (int)a.w;
+}
+
 // ------------------------------------------------------------------ batched primitives
 template <typename T>
 __global__ void sphere_disc_kernel(int m, const double *rays, const double *spheres, int point, double *out) {
@@ -1601,7 +1673,8 @@ cudaError_t launch_whitted(const SceneDev<T> &sc, const WhittedDev<T> &wp, void 
 
 template <typename T>
 cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathLaunch &pl, void *accum,
-                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, const MomentsDev *moments) {
+                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, const MomentsDev *moments,
+                        const MomentsListDev *listed) {
     if (pp.y1 <= pp.y0 || pp.W <= 0) return cudaSuccess;
     const long long tiles_total = (long long)pp.gx * pp.gy + (long long)pp.gx2 * pp.gy2;
     dim3 grid(1), block(256);
@@ -1609,21 +1682,29 @@ cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathL
     const size_t sm = pl.smem;
     cudaError_t e = cudaSuccess;
     const MomentsDev *const mom = moments;
-    // one launch of path_kernel<T, M_, F_, Q_>; SMOPT_: the shared memory to opt in to, PKC_: the parameter-block
-    // scene (kMode 3), MOM_: the moments sinks (Q_ = true)
-#define RT_PATH_LAUNCH(M_, F_, Q_, SMOPT_, PKC_, MOM_)                                                               \
-    { e = allow_smem(path_kernel<T, M_, F_, Q_>, SMOPT_); if (e != cudaSuccess) return e;                          \
-      grid.x = persistent_ctas(path_kernel<T, M_, F_, Q_>, sm, tiles_total);                                       \
+    // one launch of path_kernel<T, M_, F_, Q_, L_>; SMOPT_: the shared memory to opt in to, PKC_: the parameter-block
+    // scene (kMode 3), MOM_: the moments sinks (Q_ = true) with the pixel list (L_ = true)
+#define RT_PATH_LAUNCH(M_, F_, Q_, L_, SMOPT_, PKC_, MOM_)                                                           \
+    { e = allow_smem(path_kernel<T, M_, F_, Q_, L_>, SMOPT_); if (e != cudaSuccess) return e;                      \
+      grid.x = persistent_ctas(path_kernel<T, M_, F_, Q_, L_>, sm, tiles_total);                                   \
       if (pp.max_ctas > 0 && grid.x > (unsigned)pp.max_ctas) grid.x = (unsigned)pp.max_ctas;                        \
-      path_kernel<T, M_, F_, Q_><<<grid, block, sm, st>>>(sc, pp, (v4 *)accum, stats, PKC_, MOM_); }
+      path_kernel<T, M_, F_, Q_, L_><<<grid, block, sm, st>>>(sc, pp, (v4 *)accum, stats, PKC_, MOM_); }
+    if (listed) {                                     // list launches: integer fold only (rt_render_path_adaptive)
+        if (!pp.int_fold) return cudaErrorInvalidValue;
+        if (pl.mode == 3) { if constexpr (sizeof(T) == 4) RT_PATH_LAUNCH(3, true, true, true, sm ? sm + 8192 : 0, *pkc, *listed) }
+        else if (pl.mode == 0) RT_PATH_LAUNCH(0, true, true, true, sm, PkNone(), *listed)
+        else if (pl.mode == 1) RT_PATH_LAUNCH(1, true, true, true, sm, PkNone(), *listed)
+        else RT_PATH_LAUNCH(2, true, true, true, sm, PkNone(), *listed)
+        return cudaGetLastError();
+    }
 #define RT_PATH_CASE(M_, F_)                                                                                       \
-    { if (mom) RT_PATH_LAUNCH(M_, F_, true, sm, PkNone(), *mom) else RT_PATH_LAUNCH(M_, F_, false, sm, PkNone(), PkNone()) }
+    { if (mom) RT_PATH_LAUNCH(M_, F_, true, false, sm, PkNone(), *mom) else RT_PATH_LAUNCH(M_, F_, false, false, sm, PkNone(), PkNone()) }
     if (pl.mode == 3) {
         if constexpr (sizeof(T) == 4) {
             // + the static arrays: opt in above 48 KB in all
 #define RT_PATH_CASE3(F_)                                                                                          \
-    { if (mom) RT_PATH_LAUNCH(3, F_, true, sm ? sm + 8192 : 0, *pkc, *mom)                                          \
-      else RT_PATH_LAUNCH(3, F_, false, sm ? sm + 8192 : 0, *pkc, PkNone()) }
+    { if (mom) RT_PATH_LAUNCH(3, F_, true, false, sm ? sm + 8192 : 0, *pkc, *mom)                                   \
+      else RT_PATH_LAUNCH(3, F_, false, false, sm ? sm + 8192 : 0, *pkc, PkNone()) }
             if (pp.int_fold) RT_PATH_CASE3(true) else RT_PATH_CASE3(false)
 #undef RT_PATH_CASE3
         }
@@ -1677,6 +1758,27 @@ cudaError_t launch_resolve_variance(const void *accum, const double *moments, in
     if (n == 0) return cudaSuccess;
     resolve_variance_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const typename M<T>::v4 *)accum,
                                                                           (const double4 *)moments, W, y0, y1, var);
+    return cudaGetLastError();
+}
+
+template <typename T>
+cudaError_t launch_adaptive_select(const void *accum, const double *moments, int W, int y0, int y1, int c, double thr,
+                                   uint32_t *list, uint32_t *count, cudaStream_t st) {
+    if (y1 <= y0 || W <= 0) return cudaSuccess;
+    const dim3 grid((unsigned)((W + 31) / 32), (unsigned)((y1 - y0 + 7) / 8));
+    adaptive_select_kernel<T><<<grid, 256, 0, st>>>((const typename M<T>::v4 *)accum, (const double4 *)moments, W, y0, y1,
+                                                    c, thr, list, count);
+    return cudaGetLastError();
+}
+
+template <typename T>
+cudaError_t launch_adaptive_resolve(const void *accum, const double *moments, int W, int y0, int y1, float *image,
+                                    float *var, int *counts, cudaStream_t st) {
+    const size_t n = (size_t)(y1 - y0) * W;
+    if (n == 0) return cudaSuccess;
+    adaptive_resolve_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const typename M<T>::v4 *)accum,
+                                                                          (const double4 *)moments, W, y0, y1, image, var,
+                                                                          counts);
     return cudaGetLastError();
 }
 
@@ -1763,9 +1865,14 @@ cudaError_t launch_env_step(const SceneDev<T> &sc, const EnvDev<T> &e, const flo
     template cudaError_t launch_whitted<T>(const SceneDev<T> &, const WhittedDev<T> &, void *, int *,                   \
                                            unsigned long long *, cudaStream_t, unsigned *, unsigned *, unsigned *);     \
     template cudaError_t launch_path<T>(const SceneDev<T> &, const PathDev<T> &, const PathLaunch &, void *,           \
-                                        unsigned long long *, cudaStream_t, const PkConst *, const MomentsDev *);       \
+                                        unsigned long long *, cudaStream_t, const PkConst *, const MomentsDev *,        \
+                                        const MomentsListDev *);                                                        \
     template cudaError_t launch_resolve<T>(const void *, int, int, int, int, float *, cudaStream_t);                    \
     template cudaError_t launch_resolve_variance<T>(const void *, const double *, int, int, int, float *, cudaStream_t); \
+    template cudaError_t launch_adaptive_select<T>(const void *, const double *, int, int, int, int, double, uint32_t *,  \
+                                                   uint32_t *, cudaStream_t);                                           \
+    template cudaError_t launch_adaptive_resolve<T>(const void *, const double *, int, int, int, float *, float *, int *, \
+                                                    cudaStream_t);                                                      \
     template cudaError_t launch_trajectories<T>(const SceneDev<T> &, int, int, int, uint64_t, float *, float *, float *,  \
                                                 float *, uint8_t *, int *, uint8_t *, unsigned long long *, cudaStream_t); \
     template cudaError_t launch_simple<T>(const SceneDev<T> &, const SimpleDev<T> &, int4 *, float *,                   \

@@ -146,11 +146,18 @@ struct MomentsDev {
     double4 *peer[16];           // RT_SINK_SCATTER_ADD: the owners' [H,W,4] moments (own at [rank], peer mappings elsewhere)
     float *var;                  // RT_SINK_IMAGE, and RT_SINK_SCATTER_ADD under sync: rank 0's [H,W,3] variance image
 };
+// the trailing parameter of a list launch (kList): the moments sinks plus the pixels y * W + x to trace and their number
+struct MomentsListDev : MomentsDev {
+    const uint32_t *list;
+    unsigned count;
+};
 template <typename T>
 cudaError_t launch_path(const SceneDev<T> &sc, const PathDev<T> &pp, const PathLaunch &pl, void *accum,
-                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, const MomentsDev *moments);
+                        unsigned long long *stats, cudaStream_t st, const PkConst *pkc, const MomentsDev *moments,
+                        const MomentsListDev *listed);
 // pkc: host copy of the FP32 pair arrays, read by kMode 3; pp.sched: two zeroed device counters owned by this launch;
-// moments: NULL (plain kernels), or the moments sinks of the kMoments kernels
+// moments: NULL (plain kernels), or the moments sinks of the kMoments kernels; listed: NULL, or a list launch (integer
+// fold, accumulate, RT_SINK_ACCUM), which takes its moments sink from there
 template <typename T>
 cudaError_t launch_trajectories(const SceneDev<T> &sc, int n_traj, int max_steps, int max_bounces, uint64_t seed, float *obs,
                                 float *action, float *next_obs, float *reward, uint8_t *hit, int *length,
@@ -201,6 +208,15 @@ cudaError_t launch_wf_finish(const SceneDev<T> &sc, const WaveDev<T> &w, void *a
 // variance of each pixel's mean from accum and moments (rt_resolve_variance): rows [y0, y1) of var [H,W,3]
 template <typename T>
 cudaError_t launch_resolve_variance(const void *accum, const double *moments, int W, int y0, int y1, float *var, cudaStream_t st);
+// adaptive frames (rt_render_path_adaptive): the pixels of rows [y0, y1) with accum.w == c whose variance of the mean
+// exceeds thr in some channel, appended to list; *count must be zero before the launch and holds their number after it
+template <typename T>
+cudaError_t launch_adaptive_select(const void *accum, const double *moments, int W, int y0, int y1, int c, double thr,
+                                   uint32_t *list, uint32_t *count, cudaStream_t st);
+// image (and optionally var and the sample counts) of rows [y0, y1), each pixel resolved by its own count accum.w
+template <typename T>
+cudaError_t launch_adaptive_resolve(const void *accum, const double *moments, int W, int y0, int y1, float *image,
+                                    float *var, int *counts, cudaStream_t st);
 
 // FFMA issue-rate micro-benchmark (rt_f32.cu): `iters` trips of 16 independent FFMA per thread
 cudaError_t launch_fp32_peak(int blocks, int threads, int iters, float *sink, cudaStream_t st);

@@ -24,6 +24,9 @@ class FrameContext:
         self.host_image = self.host_stats = None
         self.moments = self.var = None      # variance frames only: [H,W,4] float64 moments, [H,W,3] float32 variance
         self.host_var_ring, self.host_var = [], None
+        # adaptive frames only: the active-pixel list ((H*W + 1) uint32) and the [H,W] int32 sample counts
+        self.pixel_list = self.counts = None
+        self.host_counts_ring, self.host_counts = [], None
         self.h2d_bytes = 0          # bytes of the last scene upload
         self.d2h_bytes = 0          # bytes of the last read-back
 
@@ -46,10 +49,10 @@ class FrameContext:
 
     # ---- buffers ---------------------------------------------------------------------------------------------
     def _buffers(self):
-        return [self.accum, self.image, self.stats, self.hit, self.host_stats, self.moments, self.var] + \
-            list(getattr(self, "host_ring", [])) + list(self.host_var_ring)
+        return [self.accum, self.image, self.stats, self.hit, self.host_stats, self.moments, self.var, self.pixel_list,
+                self.counts] + list(getattr(self, "host_ring", [])) + list(self.host_var_ring) + list(self.host_counts_ring)
 
-    def ensure(self, W, H, precision=nat.F32, want_hit=False, want_variance=False):
+    def ensure(self, W, H, precision=nat.F32, want_hit=False, want_variance=False, want_adaptive=False):
         key = (int(W), int(H), precision)
         if self._key != key:
             for b in self._buffers():
@@ -68,6 +71,8 @@ class FrameContext:
             self.hit = None
             self.moments = self.var = None
             self.host_var_ring = []
+            self.pixel_list = self.counts = None
+            self.host_counts_ring = []
             self._key = key
         if want_hit and self.hit is None:
             self.hit = nat.DeviceBuffer((H, W), np.int32, self.device)
@@ -76,6 +81,11 @@ class FrameContext:
             self.moments = nat.DeviceBuffer((H, W, 4), np.float64, self.device)
             self.var = nat.DeviceBuffer((H, W, 3), np.float32, self.device)
             self.host_var_ring = [nat.PinnedArray((H, W, 3), np.float32) for _ in range(self.HOST_RING)]
+        if want_adaptive and self.pixel_list is None:
+            # allocated on the first adaptive frame
+            self.pixel_list = nat.DeviceBuffer(H * W + 1, np.uint32, self.device)
+            self.counts = nat.DeviceBuffer((H, W), np.int32, self.device)
+            self.host_counts_ring = [nat.PinnedArray((H, W), np.int32) for _ in range(self.HOST_RING)]
 
     # ---- frames ----------------------------------------------------------------------------------------------
     def render_path(self, cam, W, H, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, precision=nat.F32, rows=None,
@@ -168,6 +178,20 @@ class FrameContext:
             return self.host_image.array, self.host_stats.array, self.host_var.array
         return self.host_image.array, self.host_stats.array
 
+    def render_path_adaptive(self, cam, W, H, max_spp, max_bounces, mirror_threshold, min_spp, tolerance, seed=0, fov=60.0,
+                             precision=nat.F32, stream=None):
+        """Adaptive Algorithm B frame (``rt_render_path_adaptive``): every pixel gets ``min_spp`` samples, then the pixels
+        whose variance of the mean still exceeds ``tolerance``^2 (colour levels) get doubling rounds up to ``max_spp``.
+        Returns (image [H,W,3] float32, stats u64[8], variance [H,W,3] float32, sample counts [H,W] int32), views of
+        pinned host rings like the image of ``render_path``.  The call synchronises the stream once per round."""
+        self.ensure(W, H, precision, want_variance=True, want_adaptive=True)
+        p = self.scene.path_params(cam, W, H, max_spp, max_bounces, mirror_threshold, seed=seed, fov=fov)
+        self.stats.fill(0, stream)
+        self.scene.render_path_adaptive(p, min_spp, tolerance, self.accum, self.moments, self.pixel_list, self.image,
+                                        precision, var=self.var, counts=self.counts, stats=self.stats, stream=stream)
+        image, stats = self.read_back(W, H, (0, H), stream, variance=True, counts=True)
+        return image, stats, self.host_var.array, self.host_counts.array
+
     def render_whitted(self, cam, X, Y, spp=1, max_bounces=1, shadow_max_bounces=0, miss=None, seed=0, prenorm=False,
                        precision=nat.F32, rows=None, samples=None, read_back=True, stream=None):
         W, H = len(X), len(Y)
@@ -182,9 +206,10 @@ class FrameContext:
             return None, None
         return self.read_back(W, H, (p.y0, p.y1), stream)
 
-    def read_back(self, W, H, rows, stream=None, variance=False):
+    def read_back(self, W, H, rows, stream=None, variance=False, counts=False):
         """D2H of the resolved rows (float32) + the stats block into pinned memory; synchronises the stream.  variance:
-        the rows of the variance image too, into ``self.host_var`` (the pinned ring slot of this frame)."""
+        the rows of the variance image too, into ``self.host_var`` (the pinned ring slot of this frame); counts: those
+        of the int32 sample counts of an adaptive frame, into ``self.host_counts``."""
         L = nat.lib()
         y0, y1 = rows
         self._ring_at = (self._ring_at + 1) % self.HOST_RING
@@ -196,9 +221,14 @@ class FrameContext:
             self.host_var = self.host_var_ring[self._ring_at]
             if nbytes:
                 nat.check(L.rt_memcpy_d2h(self.device, self.host_var.ptr + off, self.var.ptr + off, nbytes, stream))
+        if counts:
+            self.host_counts = self.host_counts_ring[self._ring_at]
+            if nbytes:
+                nat.check(L.rt_memcpy_d2h(self.device, self.host_counts.ptr + off // 3, self.counts.ptr + off // 3, nbytes // 3,
+                                          stream))
         nat.check(L.rt_memcpy_d2h(self.device, self.host_stats.ptr, self.stats.ptr, 64, stream))
         nat.check(L.rt_stream_sync(self.device, stream))
-        self.d2h_bytes = nbytes * (2 if variance else 1) + 64
+        self.d2h_bytes = nbytes * (2 if variance else 1) + (nbytes // 3 if counts else 0) + 64
         return self.host_image.array, self.host_stats.array
 
     def close(self):
@@ -207,7 +237,8 @@ class FrameContext:
                 b.free()
         self.host_ring = []
         self.host_var_ring = []
-        self.moments = self.var = None
+        self.host_counts_ring = []
+        self.moments = self.var = self.pixel_list = self.counts = None
         if getattr(self, "_copy_stream", None) is not None:
             nat.lib().rt_stream_destroy(self.device, self._copy_stream)
             self._copy_stream = None

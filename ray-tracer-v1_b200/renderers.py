@@ -126,6 +126,11 @@ class TraditionalRenderer:
     # True: render() also sets self.variance, the float32 [H,W,3] variance of each pixel's mean in colour levels^2,
     # estimated from the frame's own samples in the same launch (a view of a pinned ring, like the image)
     track_variance = False
+    # adaptive sampling: with a tolerance (colour levels, 0-255 scale) render() treats samples_per_pixel as the maximum,
+    # gives every pixel adaptive_min_spp samples and doubles the samples of the pixels whose variance of the mean still
+    # exceeds tolerance^2 (FrameContext.render_path_adaptive); it then also sets self.sample_counts, int32 [H,W]
+    adaptive_tolerance = None
+    adaptive_min_spp = 16
 
     def __init__(self, device=0, precision="f32", seed=None):
         self.scene = []
@@ -194,9 +199,16 @@ class TraditionalRenderer:
         if self._ctx is None:
             self._ctx = FrameContext(self.device)
         self._ctx.set_scene(self.flat_scene())          # re-flattened every render: the scene list is mutable
-        out = self._ctx.render_path(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
-                                    self.mirror_threshold, seed=seed, fov=self.fov, precision=_precision(self.precision),
-                                    variance=self.track_variance)
+        if self.adaptive_tolerance is not None:
+            out = self._ctx.render_path_adaptive(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
+                                                 self.mirror_threshold, min(self.adaptive_min_spp, samples_per_pixel),
+                                                 self.adaptive_tolerance, seed=seed, fov=self.fov,
+                                                 precision=_precision(self.precision))
+            self.sample_counts = out[3] if self.reuse_output else out[3].copy()
+        else:
+            out = self._ctx.render_path(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
+                                        self.mirror_threshold, seed=seed, fov=self.fov, precision=_precision(self.precision),
+                                        variance=self.track_variance)
         view, st = out[:2]
         if self.track_variance:
             self.variance = out[2] if self.reuse_output else out[2].copy()
