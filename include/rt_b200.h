@@ -227,6 +227,25 @@ int rt_resolve(int device, int precision, const void *accum_dev, int32_t W, int3
  * sample count; 0 where n < 2.  Rows [y0,y1) only. */
 int rt_resolve_variance(int device, int precision, const void *accum_dev, const double *moments_dev, int32_t W,
                         int32_t H, int32_t y0, int32_t y1, float *var_dev, void *stream);
+/* Variance-guided non-local-means filter of a whole Algorithm B frame (DESIGN §4.8c).  Inputs: accum_dev [H,W,4]
+ * (float / double per precision; per-pixel sample counts n >= 1 may differ, so adaptive frames are valid) and var_dev
+ * [H,W,3] float32, the variance of each pixel's mean as rt_resolve_variance gives it.  With u = S/n (levels, rounded to
+ * float32, not clamped), V = var, eps = 255^2 * 1e-10 and reads clamped into the frame (each pixel of a pair on its own):
+ *   delta(p,q) = 1/3 sum_c [(u_p - u_q)^2 - (V_p + min(V_p, V_q))] / [eps + k^2 (V_p + V_q)]
+ *   D(p,o)     = mean of delta(p+t, p+t+o) over t in [-patch_radius, patch_radius]^2, o in [-radius, radius]^2
+ *   out_p      = sum_o exp(-max(0, D)) u_{p+o} / sum_o exp(-max(0, D))
+ * image_dev [H,W,3] float32 = min(1, floor(out) / 255), the lattice of rt_resolve.  FP32 arithmetic for both
+ * precisions, fixed summation order: the same input gives the same bits.  Enqueued on the stream.  RT_ERR_INVALID for
+ * a NULL pointer, W or H < 1, an unknown precision, radius outside [0,15], patch_radius outside [0,5], or k not finite
+ * or not > 0.  Defaults: radius 10, patch_radius 3, k 0.45. */
+typedef struct rt_denoise_params {
+    int32_t radius;         /* search window half-width r: (2r+1)^2 offsets */
+    int32_t patch_radius;   /* patch half-width f: distances are averaged over (2f+1)^2 pixel pairs */
+    float k;                /* how many standard deviations of noise a difference may have and still count as similar */
+    int32_t reserved_;
+} rt_denoise_params;
+int rt_denoise(int device, int precision, const void *accum_dev, const float *var_dev, int32_t W, int32_t H,
+               const rt_denoise_params *d, float *image_dev, void *stream);
 
 /* ---- "Algorithm C" frame: SimplifiedFBRenderer.render_original_style / trace_ray_simple /
  *      calculate_lighting_exact_original in traditional mode (fb_usage_prob = 0): FB/output6.py:197-306, :434-654.

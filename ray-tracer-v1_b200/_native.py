@@ -71,6 +71,11 @@ class AdaptiveParams(C.Structure):
     _fields_ = [("min_spp", C.c_int32), ("reserved_", C.c_int32), ("tolerance", C.c_double)]
 
 
+class DenoiseParams(C.Structure):
+    """rt_denoise_params: the variance-guided non-local-means filter's search radius, patch radius and k."""
+    _fields_ = [("radius", C.c_int32), ("patch_radius", C.c_int32), ("k", C.c_float), ("reserved_", C.c_int32)]
+
+
 class SimpleParams(C.Structure):
     _fields_ = [("cam", C.c_double * 3), ("W", C.c_int32), ("H", C.c_int32), ("fov_rad", C.c_double),
                 ("sun_pos", C.c_double * 3), ("sun_col", C.c_double * 3), ("sun_id", C.c_int32), ("max_bounces", C.c_int32),
@@ -140,6 +145,7 @@ SIGNATURES = {
     "rt_trace_paths": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), C.c_int32, vp, vp, C.c_int32, vp, vp, vp]),
     "rt_resolve": (C.c_int, [C.c_int, C.c_int, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
     "rt_resolve_variance": (C.c_int, [C.c_int, C.c_int, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
+    "rt_denoise": (C.c_int, [C.c_int, C.c_int, vp, vp, C.c_int32, C.c_int32, C.POINTER(DenoiseParams), vp, vp]),
     "rt_wf_create": (C.c_int, [vp, C.c_int, C.c_int32, C.c_int32, C.POINTER(vp)]),
     "rt_wf_destroy": (C.c_int, [vp]),
     "rt_wf_begin": (C.c_int, [vp, C.POINTER(PathParams), C.c_double, vp, vp]),
@@ -531,6 +537,15 @@ class DeviceScene:
         y0, y1 = (0, H) if rows is None else rows
         check(lib().rt_resolve_variance(self.device, precision, _ptr(accum), _ptr(moments), int(W), int(H), int(y0), int(y1),
                                         _ptr(var), stream))
+
+    def denoise(self, accum, var, W, H, image, precision=F32, radius=10, patch_radius=3, k=0.45, stream=None):
+        """accum [H,W,4] + var [H,W,3] float32 (``resolve_variance``) -> image [H,W,3] float32: the whole frame filtered
+        by the variance-guided non-local-means filter (``rt_denoise``), on rt_resolve's lattice.  Per-pixel sample counts
+        may differ (adaptive frames)."""
+        d = DenoiseParams()
+        d.radius, d.patch_radius, d.k = int(radius), int(patch_radius), float(k)
+        check(lib().rt_denoise(self.device, precision, _ptr(accum), _ptr(var), int(W), int(H), C.byref(d), _ptr(image),
+                               stream))
 
     def render_whitted_host(self, params, precision=F32, want_accum=True, want_hit=True):
         """Host-buffer entry: -> (image [H,W,3] f32, sums [H,W,4], hit [H,W] i32, stats u64[8])."""

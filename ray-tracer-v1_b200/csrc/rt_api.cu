@@ -346,7 +346,7 @@ static inline cudaStream_t S(void *stream) { return reinterpret_cast<cudaStream_
 
 // ------------------------------------------------------------------ library / device
 RT_EXPORT const char *rt_last_error(void) { return g_err.c_str(); }
-RT_EXPORT int rt_version(void) { return 103; }
+RT_EXPORT int rt_version(void) { return 104; }
 
 RT_EXPORT int rt_device_count(int *count) {
     if (!count) return fail(RT_ERR_INVALID, "count is NULL");
@@ -1084,6 +1084,22 @@ RT_EXPORT int rt_resolve_variance(int device, int precision, const void *accum_d
     if (precision == RT_F64) CU(launch_resolve_variance<double>(accum_dev, moments_dev, W, y0, y1, var_dev, S(stream)));
     else if (precision == RT_F32) CU(launch_resolve_variance<float>(accum_dev, moments_dev, W, y0, y1, var_dev, S(stream)));
     else return fail(RT_ERR_INVALID, "unknown precision");
+    return RT_OK;
+}
+
+RT_EXPORT int rt_denoise(int device, int precision, const void *accum_dev, const float *var_dev, int32_t W, int32_t H,
+                         const rt_denoise_params *d, float *image_dev, void *stream) {
+    if (!accum_dev || !var_dev || !d || !image_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    if (W < 1 || H < 1) return fail(RT_ERR_INVALID, "W and H must be at least 1");
+    if (precision != RT_F32 && precision != RT_F64) return fail(RT_ERR_INVALID, "unknown precision");
+    if (d->radius < 0 || d->radius > 15) return fail(RT_ERR_INVALID, "radius must be in [0, 15]");
+    if (d->patch_radius < 0 || d->patch_radius > 5) return fail(RT_ERR_INVALID, "patch_radius must be in [0, 5]");
+    if (!std::isfinite(d->k) || !(d->k > 0.0f)) return fail(RT_ERR_INVALID, "k must be finite and > 0");
+    CU(cudaSetDevice(device));
+    if (precision == RT_F64)
+        CU(launch_denoise<double>(accum_dev, var_dev, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
+    else
+        CU(launch_denoise<float>(accum_dev, var_dev, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
     return RT_OK;
 }
 

@@ -1,0 +1,154 @@
+// rt_denoise.cu -- variance-guided non-local-means filter of an Algorithm B frame (rt_denoise, DESIGN §4.8c).
+// Both accum precisions are instantiated here, in one translation unit with the default contraction flags: the filter's
+// arithmetic is FP32 for either, so both must compile it the same way (rt_f64.cu is built with -fmad=false).
+//
+// For pixel p with mean u_p = S_p / n_p (levels) and variance of the mean V_p (levels^2), per offset o in [-r, r]^2:
+//   delta(p, q) = 1/3 sum_c [(u_p,c - u_q,c)^2 - (V_p,c + min(V_p,c, V_q,c))] / [eps + k^2 (V_p,c + V_q,c)]
+//   D(p, o)     = mean of delta(p + t, p + t + o) over t in [-f, f]^2,   w = exp(-max(0, D))
+//   out_p       = sum_o w u_{p+o} / sum_o w   -> image = min(1, floor(out) / 255)
+// every read at (x, y) clamped into the frame, the two pixels of a pair independently.
+#include "rt_launch.h"
+
+namespace rt {
+
+namespace {
+constexpr int kTile = 16;                       // output tile side: one CTA of kTile^2 threads per tile
+constexpr int kThreads = kTile * kTile;
+constexpr int kMaxR = 15, kMaxF = 5;            // the ABI's limits on radius and patch_radius
+constexpr int kMaxRegion = kTile + 2 * kMaxF;   // side of the region whose deltas a patch sum reads
+constexpr int kRegionSlots = (kMaxRegion * kMaxRegion + kThreads - 1) / kThreads;        // region positions per thread
+constexpr int kRowSlots = (kMaxRegion * kTile + kThreads - 1) / kThreads;                // row sums per thread
+constexpr float kEps = 255.0f * 255.0f * 1e-10f;
+}  // namespace
+
+// dynamic shared memory: the halo of u and V (6 planes of L^2 floats, L = kTile + 2(r + f)), the deltas of the
+// (kTile + 2f)^2 region, and their row sums ((kTile + 2f) rows x kTile columns)
+static size_t denoise_smem(int r, int f) {
+    const size_t L = kTile + 2 * (r + f), R = kTile + 2 * f;
+    return (6 * L * L + R * R + R * kTile) * sizeof(float);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const typename M<T>::v4 *__restrict__ accum,
+                                                               const float *__restrict__ var, int W, int H, int r, int f,
+                                                               float k2, float *__restrict__ image) {
+    extern __shared__ float smem[];
+    const int L = kTile + 2 * (r + f), LL = L * L, R = kTile + 2 * f, RR = R * R;
+    float *su = smem, *sv = smem + 3 * LL;      // su[c * LL + i], sv[c * LL + i]
+    float *sd = sv + 3 * LL, *sr = sd + RR;
+    const int tid = threadIdx.x;
+    const int x0 = blockIdx.x * kTile - (r + f), y0 = blockIdx.y * kTile - (r + f);
+
+    // halo, with clamped reads: entry (i, j) holds pixel (clamp(x0 + j), clamp(y0 + i))
+    for (int i = tid; i < LL; i += kThreads) {
+        const int x = min(max(x0 + i % L, 0), W - 1), y = min(max(y0 + i / L, 0), H - 1);
+        const size_t o = (size_t)y * W + x;
+        const typename M<T>::v4 a = accum[o];
+        RT_ASSERT(a.w >= 1);
+        const double n = (double)a.w;
+        su[i] = (float)((double)a.x / n);
+        su[LL + i] = (float)((double)a.y / n);
+        su[2 * LL + i] = (float)((double)a.z / n);
+        sv[i] = var[3 * o + 0];
+        sv[LL + i] = var[3 * o + 1];
+        sv[2 * LL + i] = var[3 * o + 2];
+    }
+    __syncthreads();
+
+    // the region positions this thread computes deltas for: their first pixel stays in registers for every offset
+    int hp[kRegionSlots];
+    float up[kRegionSlots][3], vp[kRegionSlots][3];
+#pragma unroll
+    for (int s = 0; s < kRegionSlots; ++s) {
+        const int j = tid + s * kThreads;
+        hp[s] = j < RR ? (j / R + r) * L + (j % R + r) : 0;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            up[s][c] = su[c * LL + hp[s]];
+            vp[s][c] = sv[c * LL + hp[s]];
+        }
+    }
+    // row sums: row j / kTile of the region, columns [j % kTile, j % kTile + 2f]
+    int rs[kRowSlots];
+#pragma unroll
+    for (int s = 0; s < kRowSlots; ++s) {
+        const int j = tid + s * kThreads;
+        rs[s] = (j / kTile) * R + j % kTile;
+    }
+    const int px = tid % kTile, py = tid / kTile;
+    const int hc = (py + r + f) * L + (px + r + f);           // this thread's output pixel in the halo
+    const int P = 2 * f + 1;
+    const float inv_area = 1.0f / (float)(P * P);
+    float sw = 0.f, s0 = 0.f, s1 = 0.f, s2 = 0.f;
+
+    for (int oy = -r; oy <= r; ++oy) {
+        for (int ox = -r; ox <= r; ++ox) {
+            const int d = oy * L + ox;
+#pragma unroll
+            for (int s = 0; s < kRegionSlots; ++s) {
+                const int j = tid + s * kThreads;
+                if (j < RR) {
+                    const int q = hp[s] + d;
+                    float acc = 0.f;
+#pragma unroll
+                    for (int c = 0; c < 3; ++c) {
+                        const float uq = su[c * LL + q], vq = sv[c * LL + q];
+                        const float du = up[s][c] - uq, vs = vp[s][c] + vq;
+                        const float num = du * du - (vp[s][c] + fminf(vp[s][c], vq));
+                        acc += __fdividef(num, kEps + k2 * vs);
+                    }
+                    sd[j] = acc * (1.0f / 3.0f);
+                }
+            }
+            __syncthreads();
+#pragma unroll
+            for (int s = 0; s < kRowSlots; ++s) {
+                const int j = tid + s * kThreads;
+                if (j < R * kTile) {
+                    float acc = 0.f;
+                    for (int t = 0; t < P; ++t) acc += sd[rs[s] + t];
+                    sr[j] = acc;
+                }
+            }
+            __syncthreads();
+            float D = 0.f;
+            for (int t = 0; t < P; ++t) D += sr[(py + t) * kTile + px];
+            const float w = __expf(-fmaxf(0.f, D * inv_area));
+            const int q = hc + d;
+            sw += w;
+            s0 = fmaf(w, su[q], s0);
+            s1 = fmaf(w, su[LL + q], s1);
+            s2 = fmaf(w, su[2 * LL + q], s2);
+        }
+    }
+
+    const int x = blockIdx.x * kTile + px, y = blockIdx.y * kTile + py;
+    if (x >= W || y >= H) return;
+    // o = 0 has weight 1, so sw >= 1; the lattice is rt_resolve's: min(1, floor(value) / 255) rounded from double
+    const float vals[3] = {s0 / sw, s1 / sw, s2 / sw};
+    const size_t o = (size_t)y * W + x;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const double v = floor((double)vals[c]) / 255.0;
+        image[3 * o + c] = (float)(v < 1.0 ? v : 1.0);
+    }
+}
+
+template <typename T>
+cudaError_t launch_denoise(const void *accum, const float *var, int W, int H, int r, int f, float k, float *image,
+                           cudaStream_t st) {
+    if (r < 0 || r > kMaxR || f < 0 || f > kMaxF) return cudaErrorInvalidValue;
+    const size_t smem = denoise_smem(r, f);
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(denoise_nlm_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    const dim3 grid((unsigned)((W + kTile - 1) / kTile), (unsigned)((H + kTile - 1) / kTile));
+    denoise_nlm_kernel<T><<<grid, kThreads, smem, st>>>((const typename M<T>::v4 *)accum, var, W, H, r, f, k * k, image);
+    return cudaGetLastError();
+}
+
+template cudaError_t launch_denoise<float>(const void *, const float *, int, int, int, int, float, float *, cudaStream_t);
+template cudaError_t launch_denoise<double>(const void *, const float *, int, int, int, int, float, float *, cudaStream_t);
+
+}  // namespace rt

@@ -218,6 +218,12 @@ template <typename T>
 cudaError_t launch_adaptive_resolve(const void *accum, const double *moments, int W, int y0, int y1, float *image,
                                     float *var, int *counts, cudaStream_t st);
 
+// variance-guided non-local-means filter of a whole frame (rt_denoise.cu): accum [H,W,4] of T and var [H,W,3] ->
+// image [H,W,3]; search radius r in [0, 15], patch radius f in [0, 5] (cudaErrorInvalidValue otherwise)
+template <typename T>
+cudaError_t launch_denoise(const void *accum, const float *var, int W, int H, int r, int f, float k, float *image,
+                           cudaStream_t st);
+
 // FFMA issue-rate micro-benchmark (rt_f32.cu): `iters` trips of 16 independent FFMA per thread
 cudaError_t launch_fp32_peak(int blocks, int threads, int iters, float *sink, cudaStream_t st);
 

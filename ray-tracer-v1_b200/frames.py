@@ -89,24 +89,36 @@ class FrameContext:
 
     # ---- frames ----------------------------------------------------------------------------------------------
     def render_path(self, cam, W, H, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, precision=nat.F32, rows=None,
-                    samples=None, resolve=True, read_back=True, stream=None, variance=False):
+                    samples=None, resolve=True, read_back=True, stream=None, variance=False, denoise=False):
         """Algorithm B over rows x samples of this rank.  Returns (host image view or None, stats u64[8] or None).
 
         variance=True: the launch also stores the second moments of every pixel's samples (``self.moments``), and the
         result gains a third item, the float32 [H,W,3] variance of each pixel's mean in colour levels^2 -- a view of a
-        pinned host ring like the image (None when not read back; ``self.var`` holds it in HBM when resolved)."""
-        self.ensure(W, H, precision, want_variance=variance)
+        pinned host ring like the image (None when not read back; ``self.var`` holds it in HBM when resolved).
+
+        denoise=True: the frame is rendered with its moments, its variance is resolved, and the image is the variance-guided
+        non-local-means filter of the frame (``rt_denoise`` with the library defaults) in place of the resolved one; the
+        return shape is the one ``variance`` selects.  The filter reads every row, so the whole frame is rendered in one
+        launch and read back once after the filter: the banded read-back overlap (``BANDS``) does not apply, and
+        ``rows`` must cover the frame."""
+        if denoise and (not resolve or (rows is not None and (int(rows[0]), int(rows[1])) != (0, int(H)))):
+            raise ValueError("denoise filters the whole frame: it needs every row and resolve=True")
+        self.ensure(W, H, precision, want_variance=variance or denoise)
         L = nat.lib()
         p = self.scene.path_params(cam, W, H, spp, max_bounces, mirror_threshold, seed=seed, fov=fov, rows=rows,
                                    samples=samples)
         self.stats.fill(0, stream)
-        moments = self.moments if variance else None
-        bands = self._bands(W, p.y0, p.y1, p.s1 - p.s0) if (resolve and read_back) else None
+        moments = self.moments if (variance or denoise) else None
+        bands = self._bands(W, p.y0, p.y1, p.s1 - p.s0) if (resolve and read_back and not denoise) else None
         if bands:
             return self._render_path_banded(p, bands, W, H, precision, stream, variance)
         self.scene.render_path(p, self.accum, precision, stats=self.stats, stream=stream, moments=moments)
         self.launches = 1
-        if resolve:
+        if denoise:
+            self.scene.resolve_variance(self.accum, self.moments, W, H, self.var, precision, stream=stream)
+            self.scene.denoise(self.accum, self.var, W, H, self.image, precision, stream=stream)
+            self.launches += 2
+        elif resolve:
             self.scene.resolve(self.accum, W, H, p.s1 - p.s0, self.image, precision, rows=(p.y0, p.y1), stream=stream)
             self.launches += 1
             if variance:
@@ -179,16 +191,20 @@ class FrameContext:
         return self.host_image.array, self.host_stats.array
 
     def render_path_adaptive(self, cam, W, H, max_spp, max_bounces, mirror_threshold, min_spp, tolerance, seed=0, fov=60.0,
-                             precision=nat.F32, stream=None):
+                             precision=nat.F32, stream=None, denoise=False):
         """Adaptive Algorithm B frame (``rt_render_path_adaptive``): every pixel gets ``min_spp`` samples, then the pixels
         whose variance of the mean still exceeds ``tolerance``^2 (colour levels) get doubling rounds up to ``max_spp``.
         Returns (image [H,W,3] float32, stats u64[8], variance [H,W,3] float32, sample counts [H,W] int32), views of
-        pinned host rings like the image of ``render_path``.  The call synchronises the stream once per round."""
+        pinned host rings like the image of ``render_path``.  The call synchronises the stream once per round.
+        denoise=True: the image is the frame filtered by ``rt_denoise`` (library defaults), each pixel's mean and variance
+        taken at its own sample count."""
         self.ensure(W, H, precision, want_variance=True, want_adaptive=True)
         p = self.scene.path_params(cam, W, H, max_spp, max_bounces, mirror_threshold, seed=seed, fov=fov)
         self.stats.fill(0, stream)
         self.scene.render_path_adaptive(p, min_spp, tolerance, self.accum, self.moments, self.pixel_list, self.image,
                                         precision, var=self.var, counts=self.counts, stats=self.stats, stream=stream)
+        if denoise:
+            self.scene.denoise(self.accum, self.var, W, H, self.image, precision, stream=stream)
         image, stats = self.read_back(W, H, (0, H), stream, variance=True, counts=True)
         return image, stats, self.host_var.array, self.host_counts.array
 

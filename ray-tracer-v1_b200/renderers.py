@@ -131,6 +131,9 @@ class TraditionalRenderer:
     # exceeds tolerance^2 (FrameContext.render_path_adaptive); it then also sets self.sample_counts, int32 [H,W]
     adaptive_tolerance = None
     adaptive_min_spp = 16
+    # True: render() returns the frame filtered by the variance-guided non-local-means filter (rt_denoise, library
+    # defaults; DESIGN §4.8c), from the frame's own per-pixel variance; combines with track_variance and adaptive_tolerance
+    denoise = False
 
     def __init__(self, device=0, precision="f32", seed=None):
         self.scene = []
@@ -203,12 +206,12 @@ class TraditionalRenderer:
             out = self._ctx.render_path_adaptive(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
                                                  self.mirror_threshold, min(self.adaptive_min_spp, samples_per_pixel),
                                                  self.adaptive_tolerance, seed=seed, fov=self.fov,
-                                                 precision=_precision(self.precision))
+                                                 precision=_precision(self.precision), denoise=self.denoise)
             self.sample_counts = out[3] if self.reuse_output else out[3].copy()
         else:
             out = self._ctx.render_path(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
                                         self.mirror_threshold, seed=seed, fov=self.fov, precision=_precision(self.precision),
-                                        variance=self.track_variance)
+                                        variance=self.track_variance, denoise=self.denoise)
         view, st = out[:2]
         if self.track_variance:
             self.variance = out[2] if self.reuse_output else out[2].copy()
