@@ -246,6 +246,37 @@ typedef struct rt_denoise_params {
 } rt_denoise_params;
 int rt_denoise(int device, int precision, const void *accum_dev, const float *var_dev, int32_t W, int32_t H,
                const rt_denoise_params *d, float *image_dev, void *stream);
+/* First-hit features of an Algorithm B frame (DESIGN §4.8d), the AOVs of a path tracer and the inputs of a feature-guided
+ * filter.  For every pixel of rows [y0,y1) of p and samples [s0,s1) it traces exactly the camera rays rt_render_path
+ * traces (p's cam, W, H, fov_deg and seed; the other fields are ignored) to their nearest hit, following no mirror or
+ * glass: albedo = the sphere's colour / 255 (emissive spheres too), normal = (hit point - centre) / radius,
+ * depth = the hit distance t; all 0 on a miss.  Outputs, float32, rows [y0,y1) only: albedo_dev [H,W,3], normal_dev
+ * [H,W,3] and depth_dev [H,W], each the mean over the samples, and fvar_dev [H,W,3], the variance of the mean of albedo,
+ * normal and depth, (sum f^2 - (sum f)^2 / n) / (n (n - 1)) averaged over the feature's channels (0 for n < 2).  Sums are
+ * doubles added in sample order: the same request gives the same bits.  Enqueued on the stream.  RT_ERR_INVALID for a
+ * NULL pointer, a bad band, s1 <= s0 or an unknown precision. */
+int rt_render_features(rt_scene *scene, int precision, const rt_path_params *p, float *albedo_dev, float *normal_dev,
+                       float *depth_dev, float *fvar_dev, void *stream);
+/* rt_denoise with the feature term of Rousselle, Manzi and Zwicker 2013 (DESIGN §4.8d), from rt_render_features' buffers.
+ * For feature j (albedo, normal: 3 channels, depth: 1) with mean f_j, variance Var_j and, reads clamped into the frame,
+ *   G_j,p     = mean_c [((f(x+1,y) - f(x-1,y)) / 2)^2 + ((f(x,y+1) - f(x,y-1)) / 2)^2]
+ *   Phi_j(p,q)= [mean_c (f_j,p - f_j,q)^2 - (Var_j,p + min(Var_j,p, Var_j,q))] / [k_f^2 max(tau, Var_j,p, G_j,p)]
+ *   w         = min(w_c, exp(-max(0, max_j Phi_j)))          (w_c = rt_denoise's weight exp(-max(0, D)))
+ * and out_p = sum_o w u_{p+o} / sum_o w, on the same lattice.  Features can only lower a colour weight: k_f -> infinity
+ * gives rt_denoise's image.  Validation as rt_denoise, and RT_ERR_INVALID for a NULL feature pointer, k_f not finite or
+ * not > 0, or tau not finite or < 0.  Defaults (measured, DESIGN §4.8d): radius 10, patch_radius 3, k 1.0, k_f 1.2,
+ * tau 1e-3. */
+typedef struct rt_denoise_features_params {
+    int32_t radius;         /* as rt_denoise_params */
+    int32_t patch_radius;
+    float k;
+    float k_f;              /* how many standard deviations a feature difference may have and still count as similar */
+    float tau;              /* floor of the feature denominators (squared feature units) */
+    int32_t reserved_;
+} rt_denoise_features_params;
+int rt_denoise_features(int device, int precision, const void *accum_dev, const float *var_dev, const float *albedo_dev,
+                        const float *normal_dev, const float *depth_dev, const float *fvar_dev, int32_t W, int32_t H,
+                        const rt_denoise_features_params *d, float *image_dev, void *stream);
 
 /* ---- "Algorithm C" frame: SimplifiedFBRenderer.render_original_style / trace_ray_simple /
  *      calculate_lighting_exact_original in traditional mode (fb_usage_prob = 0): FB/output6.py:197-306, :434-654.

@@ -76,6 +76,12 @@ class DenoiseParams(C.Structure):
     _fields_ = [("radius", C.c_int32), ("patch_radius", C.c_int32), ("k", C.c_float), ("reserved_", C.c_int32)]
 
 
+class DenoiseFeaturesParams(C.Structure):
+    """rt_denoise_features_params: rt_denoise_params plus the feature term's k_f and tau."""
+    _fields_ = [("radius", C.c_int32), ("patch_radius", C.c_int32), ("k", C.c_float), ("k_f", C.c_float),
+                ("tau", C.c_float), ("reserved_", C.c_int32)]
+
+
 class SimpleParams(C.Structure):
     _fields_ = [("cam", C.c_double * 3), ("W", C.c_int32), ("H", C.c_int32), ("fov_rad", C.c_double),
                 ("sun_pos", C.c_double * 3), ("sun_col", C.c_double * 3), ("sun_id", C.c_int32), ("max_bounces", C.c_int32),
@@ -146,6 +152,9 @@ SIGNATURES = {
     "rt_resolve": (C.c_int, [C.c_int, C.c_int, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
     "rt_resolve_variance": (C.c_int, [C.c_int, C.c_int, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
     "rt_denoise": (C.c_int, [C.c_int, C.c_int, vp, vp, C.c_int32, C.c_int32, C.POINTER(DenoiseParams), vp, vp]),
+    "rt_render_features": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), vp, vp, vp, vp, vp]),
+    "rt_denoise_features": (C.c_int, [C.c_int, C.c_int, vp, vp, vp, vp, vp, vp, C.c_int32, C.c_int32,
+                                      C.POINTER(DenoiseFeaturesParams), vp, vp]),
     "rt_wf_create": (C.c_int, [vp, C.c_int, C.c_int32, C.c_int32, C.POINTER(vp)]),
     "rt_wf_destroy": (C.c_int, [vp]),
     "rt_wf_begin": (C.c_int, [vp, C.POINTER(PathParams), C.c_double, vp, vp]),
@@ -538,14 +547,33 @@ class DeviceScene:
         check(lib().rt_resolve_variance(self.device, precision, _ptr(accum), _ptr(moments), int(W), int(H), int(y0), int(y1),
                                         _ptr(var), stream))
 
-    def denoise(self, accum, var, W, H, image, precision=F32, radius=10, patch_radius=3, k=0.45, stream=None):
+    def denoise(self, accum, var, W, H, image, precision=F32, radius=10, patch_radius=3, k=None, stream=None,
+                features=None, k_f=1.2, tau=1e-3):
         """accum [H,W,4] + var [H,W,3] float32 (``resolve_variance``) -> image [H,W,3] float32: the whole frame filtered
         by the variance-guided non-local-means filter (``rt_denoise``), on rt_resolve's lattice.  Per-pixel sample counts
-        may differ (adaptive frames)."""
-        d = DenoiseParams()
-        d.radius, d.patch_radius, d.k = int(radius), int(patch_radius), float(k)
-        check(lib().rt_denoise(self.device, precision, _ptr(accum), _ptr(var), int(W), int(H), C.byref(d), _ptr(image),
-                               stream))
+        may differ (adaptive frames).  ``features`` = (albedo, normal, depth, fvar) as ``render_features`` gives them:
+        the filter with the feature term (``rt_denoise_features``), with ``k_f`` and ``tau``.  k defaults to 0.45
+        without features and 1.0 with them (the defaults measured in DESIGN §4.8c and §4.8d)."""
+        if k is None:
+            k = 0.45 if features is None else 1.0
+        if features is None:
+            d = DenoiseParams()
+            d.radius, d.patch_radius, d.k = int(radius), int(patch_radius), float(k)
+            check(lib().rt_denoise(self.device, precision, _ptr(accum), _ptr(var), int(W), int(H), C.byref(d), _ptr(image),
+                                   stream))
+            return
+        albedo, normal, depth, fvar = features
+        d = DenoiseFeaturesParams()
+        d.radius, d.patch_radius, d.k, d.k_f, d.tau = int(radius), int(patch_radius), float(k), float(k_f), float(tau)
+        check(lib().rt_denoise_features(self.device, precision, _ptr(accum), _ptr(var), _ptr(albedo), _ptr(normal),
+                                        _ptr(depth), _ptr(fvar), int(W), int(H), C.byref(d), _ptr(image), stream))
+
+    def render_features(self, params, albedo, normal, depth, fvar, precision=F32, stream=None):
+        """First-hit features of rows [y0, y1) over samples [s0, s1) of ``params`` (``rt_render_features``): the camera
+        rays ``render_path`` traces, to their nearest hit.  Means into albedo [H,W,3], normal [H,W,3] and depth [H,W],
+        and the variance of the mean of each feature into fvar [H,W,3], all float32; asynchronous."""
+        check(lib().rt_render_features(self.handle, precision, C.byref(params), _ptr(albedo), _ptr(normal), _ptr(depth),
+                                       _ptr(fvar), stream))
 
     def render_whitted_host(self, params, precision=F32, want_accum=True, want_hit=True):
         """Host-buffer entry: -> (image [H,W,3] f32, sums [H,W,4], hit [H,W] i32, stats u64[8])."""

@@ -346,7 +346,7 @@ static inline cudaStream_t S(void *stream) { return reinterpret_cast<cudaStream_
 
 // ------------------------------------------------------------------ library / device
 RT_EXPORT const char *rt_last_error(void) { return g_err.c_str(); }
-RT_EXPORT int rt_version(void) { return 104; }
+RT_EXPORT int rt_version(void) { return 105; }
 
 RT_EXPORT int rt_device_count(int *count) {
     if (!count) return fail(RT_ERR_INVALID, "count is NULL");
@@ -672,6 +672,12 @@ template <typename T> static void path_camera(PathDev<T> &pp, const rt_path_para
     pp.inv_W = (T)(1.0 / (double)p->W); pp.inv_H = (T)(1.0 / (double)p->H);
 }
 
+// the Philox key of the frame and its round keys
+template <typename T> static void path_keys(PathDev<T> &pp, const rt_path_params *p) {
+    pp.k0 = (uint32_t)p->seed; pp.k1 = (uint32_t)(p->seed >> 32);
+    for (uint32_t r = 0; r < 10; ++r) { pp.rk[2 * r] = pp.k0 + r * 0x9E3779B9u; pp.rk[2 * r + 1] = pp.k1 + r * 0xBB67AE85u; }
+}
+
 // Cuts one path-kernel launch into work units: sets the band (y0, tile_step, col_*, seg_w), the sample split, both tile
 // grids and fold_tab of pp (which holds W, y1 and int_fold of the request) and returns the kernel variant and its dynamic
 // shared memory.  Every rank of a frame plans from the same numbers, so the launches of a frame tile it exactly.
@@ -771,8 +777,7 @@ static int render_path_t(const rt_scene *sc, const SceneDev<T> &view, const rt_p
     path_camera(pp, p);
     pp.y0 = p->y0; pp.y1 = p->y1; pp.s0 = p->s0; pp.s1 = p->s1; pp.max_bounces = p->max_bounces;
     pp.mirror_threshold = (T)p->mirror_threshold;
-    pp.k0 = (uint32_t)p->seed; pp.k1 = (uint32_t)(p->seed >> 32);
-    for (uint32_t r = 0; r < 10; ++r) { pp.rk[2 * r] = pp.k0 + r * 0x9E3779B9u; pp.rk[2 * r + 1] = pp.k1 + r * 0xBB67AE85u; }
+    path_keys(pp, p);
     pp.accumulate = p->accumulate;
     pp.int_fold = sc->int_colours && (p->s1 - p->s0) <= 65536;
     pp.primary_cull = (p->schedule & 2) == 0;
@@ -939,6 +944,30 @@ RT_EXPORT int rt_render_path_adaptive(rt_scene *scene, int precision, const rt_p
                                          counts_dev, stats_dev, S(stream));
 }
 
+template <typename T>
+static int render_features_t(const SceneDev<T> &view, const rt_path_params *p, float *albedo, float *normal, float *depth,
+                             float *fvar, cudaStream_t st) {
+    PathDev<T> pp;
+    std::memset(&pp, 0, sizeof pp);
+    path_camera(pp, p);
+    path_keys(pp, p);
+    pp.y0 = p->y0; pp.y1 = p->y1; pp.s0 = p->s0; pp.s1 = p->s1;
+    CU(launch_features<T>(view, pp, albedo, normal, depth, fvar, st));
+    return RT_OK;
+}
+
+RT_EXPORT int rt_render_features(rt_scene *scene, int precision, const rt_path_params *p, float *albedo_dev,
+                                 float *normal_dev, float *depth_dev, float *fvar_dev, void *stream) {
+    if (!scene || !p || !albedo_dev || !normal_dev || !depth_dev || !fvar_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    int rc = check_band(p->W, p->H, p->y0, p->y1, p->s0, p->s1);
+    if (rc) return rc;
+    if (p->s1 <= p->s0) return fail(RT_ERR_INVALID, "empty sample range: s1 must be greater than s0");
+    if (precision != RT_F32 && precision != RT_F64) return fail(RT_ERR_INVALID, "unknown precision");
+    CU(cudaSetDevice(scene->device));
+    if (precision == RT_F64) return render_features_t<double>(scene->d.view, p, albedo_dev, normal_dev, depth_dev, fvar_dev, S(stream));
+    return render_features_t<float>(scene->f.view, p, albedo_dev, normal_dev, depth_dev, fvar_dev, S(stream));
+}
+
 RT_EXPORT int rt_trace_paths(rt_scene *scene, int precision, const rt_path_params *p, int32_t n, const double *rays_dev,
                              const int32_t *ray_ids_dev, int32_t bounce_count, void *accum_dev, uint64_t *stats_dev, void *stream) {
     if (!scene || !p || !accum_dev || (n > 0 && !rays_dev)) return fail(RT_ERR_INVALID, "NULL argument");
@@ -1100,6 +1129,28 @@ RT_EXPORT int rt_denoise(int device, int precision, const void *accum_dev, const
         CU(launch_denoise<double>(accum_dev, var_dev, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
     else
         CU(launch_denoise<float>(accum_dev, var_dev, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
+    return RT_OK;
+}
+
+RT_EXPORT int rt_denoise_features(int device, int precision, const void *accum_dev, const float *var_dev,
+                                  const float *albedo_dev, const float *normal_dev, const float *depth_dev,
+                                  const float *fvar_dev, int32_t W, int32_t H, const rt_denoise_features_params *d,
+                                  float *image_dev, void *stream) {
+    if (!accum_dev || !var_dev || !d || !image_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    if (!albedo_dev || !normal_dev || !depth_dev || !fvar_dev) return fail(RT_ERR_INVALID, "NULL feature buffer");
+    if (W < 1 || H < 1) return fail(RT_ERR_INVALID, "W and H must be at least 1");
+    if (precision != RT_F32 && precision != RT_F64) return fail(RT_ERR_INVALID, "unknown precision");
+    if (d->radius < 0 || d->radius > 15) return fail(RT_ERR_INVALID, "radius must be in [0, 15]");
+    if (d->patch_radius < 0 || d->patch_radius > 5) return fail(RT_ERR_INVALID, "patch_radius must be in [0, 5]");
+    if (!std::isfinite(d->k) || !(d->k > 0.0f)) return fail(RT_ERR_INVALID, "k must be finite and > 0");
+    if (!std::isfinite(d->k_f) || !(d->k_f > 0.0f)) return fail(RT_ERR_INVALID, "k_f must be finite and > 0");
+    if (!std::isfinite(d->tau) || !(d->tau >= 0.0f)) return fail(RT_ERR_INVALID, "tau must be finite and >= 0");
+    CU(cudaSetDevice(device));
+    const DenoiseFeatures feat = {albedo_dev, normal_dev, depth_dev, fvar_dev, d->k_f * d->k_f, d->tau};
+    if (precision == RT_F64)
+        CU(launch_denoise_features<double>(accum_dev, var_dev, feat, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
+    else
+        CU(launch_denoise_features<float>(accum_dev, var_dev, feat, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
     return RT_OK;
 }
 

@@ -7,6 +7,14 @@
 //   D(p, o)     = mean of delta(p + t, p + t + o) over t in [-f, f]^2,   w = exp(-max(0, D))
 //   out_p       = sum_o w u_{p+o} / sum_o w   -> image = min(1, floor(out) / 255)
 // every read at (x, y) clamped into the frame, the two pixels of a pair independently.
+//
+// kFeatures (rt_denoise_features, DESIGN §4.8d) adds the feature term of Rousselle, Manzi and Zwicker 2013, per pixel and
+// without a patch.  For feature j (albedo, normal: 3 channels; depth: 1) with mean f_j, variance of the mean Var_j and
+// gradient G_j,p = mean_c [((f(x+1,y) - f(x-1,y)) / 2)^2 + ((f(x,y+1) - f(x,y-1)) / 2)^2] (reads clamped):
+//   Phi_j(p, q) = [mean_c (f_j,p - f_j,q)^2 - (Var_j,p + min(Var_j,p, Var_j,q))] / [k_f^2 max(tau, Var_j,p, G_j,p)]
+//   w = min(w_c, exp(-max(0, max_j Phi_j))) = exp(-max(0, D, max_j Phi_j))
+// The features of p and its denominators stay in registers; the (kTile + 2r)^2 halo of the 7 feature channels and the
+// 3 variances is staged beside the colour halo.
 #include "rt_launch.h"
 
 namespace rt {
@@ -23,21 +31,39 @@ constexpr float kEps = 255.0f * 255.0f * 1e-10f;
 
 // dynamic shared memory: the halo of u and V (6 planes of L^2 floats, L = kTile + 2(r + f)), the deltas of the
 // (kTile + 2f)^2 region, and their row sums ((kTile + 2f) rows x kTile columns)
-static size_t denoise_smem(int r, int f) {
-    const size_t L = kTile + 2 * (r + f), R = kTile + 2 * f;
-    return (6 * L * L + R * R + R * kTile) * sizeof(float);
+// kFeatures: + the feature halo, 10 planes of LF^2 floats, LF = kTile + 2r
+static size_t denoise_smem(int r, int f, bool features) {
+    const size_t L = kTile + 2 * (r + f), R = kTile + 2 * f, LF = kTile + 2 * r;
+    return (6 * L * L + R * R + R * kTile + (features ? 10 * LF * LF : 0)) * sizeof(float);
 }
 
-template <typename T>
-__global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const typename M<T>::v4 *__restrict__ accum,
-                                                               const float *__restrict__ var, int W, int H, int r, int f,
-                                                               float k2, float *__restrict__ image) {
+// The filter of one CTA; kFeatures: with the feature term.  Two kernels below call it, so that the colour-only one keeps
+// its parameter block.  tid = threadIdx.x, read in the kernel, where its range (__launch_bounds__) is known.
+template <typename T, bool kFeatures>
+RT_DEV void denoise_nlm(const typename M<T>::v4 *__restrict__ accum, const float *__restrict__ var, int W, int H, int r,
+                        int f, float k2, float *__restrict__ image, const DenoiseFeatures &feat, const int tid) {
     extern __shared__ float smem[];
     const int L = kTile + 2 * (r + f), LL = L * L, R = kTile + 2 * f, RR = R * R;
     float *su = smem, *sv = smem + 3 * LL;      // su[c * LL + i], sv[c * LL + i]
     float *sd = sv + 3 * LL, *sr = sd + RR;
-    const int tid = threadIdx.x;
     const int x0 = blockIdx.x * kTile - (r + f), y0 = blockIdx.y * kTile - (r + f);
+    // kFeatures: sf[j * LFF + i], planes 0-2 albedo, 3-5 normal, 6 depth, 7-9 the variances of albedo, normal, depth
+    const int LF = kTile + 2 * r, LFF = LF * LF;
+    float *sf = sr + R * kTile;
+    if constexpr (kFeatures) {
+        const int fx0 = blockIdx.x * kTile - r, fy0 = blockIdx.y * kTile - r;
+        for (int i = tid; i < LFF; i += kThreads) {
+            const int x = min(max(fx0 + i % LF, 0), W - 1), y = min(max(fy0 + i / LF, 0), H - 1);
+            const size_t o = (size_t)y * W + x;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                sf[c * LFF + i] = feat.albedo[3 * o + c];
+                sf[(3 + c) * LFF + i] = feat.normal[3 * o + c];
+                sf[(7 + c) * LFF + i] = feat.fvar[3 * o + c];
+            }
+            sf[6 * LFF + i] = feat.depth[o];
+        }
+    }
 
     // halo, with clamped reads: entry (i, j) holds pixel (clamp(x0 + j), clamp(y0 + i))
     for (int i = tid; i < LL; i += kThreads) {
@@ -80,6 +106,32 @@ __global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const typename M<
     const int P = 2 * f + 1;
     const float inv_area = 1.0f / (float)(P * P);
     float sw = 0.f, s0 = 0.f, s1 = 0.f, s2 = 0.f;
+    // kFeatures: p's features, variances and 1 / (k_f^2 max(tau, Var_j,p, G_j,p)); G from clamped global reads
+    float fp[7], vfp[3], inv_den[3];
+    const int hcf = (py + r) * LF + (px + r);                // this thread's output pixel in the feature halo
+    if constexpr (kFeatures) {
+#pragma unroll
+        for (int c = 0; c < 7; ++c) fp[c] = sf[c * LFF + hcf];
+#pragma unroll
+        for (int j = 0; j < 3; ++j) vfp[j] = sf[(7 + j) * LFF + hcf];
+        const int xc = min(blockIdx.x * kTile + px, W - 1), yc = min(blockIdx.y * kTile + py, H - 1);
+        const size_t oxm = (size_t)yc * W + max(xc - 1, 0), oxp = (size_t)yc * W + min(xc + 1, W - 1);
+        const size_t oym = (size_t)max(yc - 1, 0) * W + xc, oyp = (size_t)min(yc + 1, H - 1) * W + xc;
+        float g[3] = {0.f, 0.f, 0.f};
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            float gx = 0.5f * (feat.albedo[3 * oxp + c] - feat.albedo[3 * oxm + c]);
+            float gy = 0.5f * (feat.albedo[3 * oyp + c] - feat.albedo[3 * oym + c]);
+            g[0] += gx * gx + gy * gy;
+            gx = 0.5f * (feat.normal[3 * oxp + c] - feat.normal[3 * oxm + c]);
+            gy = 0.5f * (feat.normal[3 * oyp + c] - feat.normal[3 * oym + c]);
+            g[1] += gx * gx + gy * gy;
+        }
+        const float gx = 0.5f * (feat.depth[oxp] - feat.depth[oxm]), gy = 0.5f * (feat.depth[oyp] - feat.depth[oym]);
+        g[0] *= 1.0f / 3.0f; g[1] *= 1.0f / 3.0f; g[2] = gx * gx + gy * gy;
+#pragma unroll
+        for (int j = 0; j < 3; ++j) inv_den[j] = 1.0f / (feat.kf2 * fmaxf(feat.tau, fmaxf(vfp[j], g[j])));
+    }
 
     for (int oy = -r; oy <= r; ++oy) {
         for (int ox = -r; ox <= r; ++ox) {
@@ -113,7 +165,25 @@ __global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const typename M<
             __syncthreads();
             float D = 0.f;
             for (int t = 0; t < P; ++t) D += sr[(py + t) * kTile + px];
-            const float w = __expf(-fmaxf(0.f, D * inv_area));
+            float e = D * inv_area;
+            if constexpr (kFeatures) {
+                // fmaxf drops a NaN (0 * inf with tau = 0 between equal features): such a feature does not lower w
+                const int qf = hcf + oy * LF + ox;
+                float da = 0.f, dm = 0.f;
+#pragma unroll
+                for (int c = 0; c < 3; ++c) {
+                    const float a = fp[c] - sf[c * LFF + qf], b = fp[3 + c] - sf[(3 + c) * LFF + qf];
+                    da = fmaf(a, a, da);
+                    dm = fmaf(b, b, dm);
+                }
+                const float dz = fp[6] - sf[6 * LFF + qf];
+                const float va = sf[7 * LFF + qf], vm = sf[8 * LFF + qf], vz = sf[9 * LFF + qf];
+                const float pa = (da * (1.0f / 3.0f) - (vfp[0] + fminf(vfp[0], va))) * inv_den[0];
+                const float pm = (dm * (1.0f / 3.0f) - (vfp[1] + fminf(vfp[1], vm))) * inv_den[1];
+                const float pz = (dz * dz - (vfp[2] + fminf(vfp[2], vz))) * inv_den[2];
+                e = fmaxf(e, fmaxf(fmaxf(pa, pm), pz));
+            }
+            const float w = __expf(-fmaxf(0.f, e));
             const int q = hc + d;
             sw += w;
             s0 = fmaf(w, su[q], s0);
@@ -135,20 +205,52 @@ __global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const typename M<
 }
 
 template <typename T>
-cudaError_t launch_denoise(const void *accum, const float *var, int W, int H, int r, int f, float k, float *image,
-                           cudaStream_t st) {
+__global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const typename M<T>::v4 *__restrict__ accum,
+                                                               const float *__restrict__ var, int W, int H, int r, int f,
+                                                               float k2, float *__restrict__ image) {
+    denoise_nlm<T, false>(accum, var, W, H, r, f, k2, image, DenoiseFeatures{}, threadIdx.x);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kThreads) denoise_nlm_features_kernel(const typename M<T>::v4 *__restrict__ accum,
+                                                                        const float *__restrict__ var, int W, int H, int r,
+                                                                        int f, float k2, float *__restrict__ image,
+                                                                        const __grid_constant__ DenoiseFeatures feat) {
+    denoise_nlm<T, true>(accum, var, W, H, r, f, k2, image, feat, threadIdx.x);
+}
+
+template <typename K, typename... A>
+static cudaError_t launch_nlm(K kernel, bool features, int W, int H, int r, int f, cudaStream_t st, const A &...args) {
     if (r < 0 || r > kMaxR || f < 0 || f > kMaxF) return cudaErrorInvalidValue;
-    const size_t smem = denoise_smem(r, f);
+    const size_t smem = denoise_smem(r, f, features);
     if (smem > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(denoise_nlm_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
     const dim3 grid((unsigned)((W + kTile - 1) / kTile), (unsigned)((H + kTile - 1) / kTile));
-    denoise_nlm_kernel<T><<<grid, kThreads, smem, st>>>((const typename M<T>::v4 *)accum, var, W, H, r, f, k * k, image);
+    kernel<<<grid, kThreads, smem, st>>>(args...);
     return cudaGetLastError();
+}
+
+template <typename T>
+cudaError_t launch_denoise(const void *accum, const float *var, int W, int H, int r, int f, float k, float *image,
+                           cudaStream_t st) {
+    return launch_nlm(denoise_nlm_kernel<T>, false, W, H, r, f, st, (const typename M<T>::v4 *)accum, var, W, H, r, f,
+                      k * k, image);
+}
+
+template <typename T>
+cudaError_t launch_denoise_features(const void *accum, const float *var, const DenoiseFeatures &feat, int W, int H, int r,
+                                    int f, float k, float *image, cudaStream_t st) {
+    return launch_nlm(denoise_nlm_features_kernel<T>, true, W, H, r, f, st, (const typename M<T>::v4 *)accum, var, W, H,
+                      r, f, k * k, image, feat);
 }
 
 template cudaError_t launch_denoise<float>(const void *, const float *, int, int, int, int, float, float *, cudaStream_t);
 template cudaError_t launch_denoise<double>(const void *, const float *, int, int, int, int, float, float *, cudaStream_t);
+template cudaError_t launch_denoise_features<float>(const void *, const float *, const DenoiseFeatures &, int, int, int, int,
+                                                    float, float *, cudaStream_t);
+template cudaError_t launch_denoise_features<double>(const void *, const float *, const DenoiseFeatures &, int, int, int,
+                                                     int, float, float *, cudaStream_t);
 
 }  // namespace rt

@@ -349,6 +349,14 @@ template <typename T> RT_DEV V3<T> path_camera_ray(const PathDev<T> &pp, int x, 
     return d;
 }
 
+// The camera ray of a sample of pixel (x, y), rng begun at the key (pixel, sample): Philox slot 0 jitters it inside the
+// pixel.  path_kernel and feature_kernel both call it, so the features see exactly the rays the frame traces.
+template <typename T> RT_DEV V3<T> path_sample_ray(const PathDev<T> &pp, PathRng &rng, int x, int y) {
+    uint32_t wa, wb;
+    rng.pair_rk(0u, wa, wb, pp.rk);
+    return path_camera_ray<T>(pp, x, y, u01<T>(wa), u01<T>(wb));
+}
+
 // One thread per pixel, looping over its samples; 8x4-pixel warps in lock-step: the warp traces sample s of all its
 // 32 pixels together, one nearest-hit query per trip, until every lane's path has ended, then folds and starts sample
 // s+1 together.  Everything outside the sphere loop (camera ray, Philox, fold) runs once per sample at full lane
@@ -562,9 +570,7 @@ path_kernel(SceneDev<T> sc, PathDev<T> pp, typename M<T>::v4 *accum, unsigned lo
             }
             rng.begin(pixel, (uint32_t)smp, pp.k0, pp.k1);
             if constexpr (kMode == 3) if (pp.primary_cull) n_tests += (unsigned)__popcll(cand);
-            uint32_t wa, wb;
-            rng.pair_rk(0u, wa, wb, pp.rk);
-            D = path_camera_ray<T>(pp, x, y, u01<T>(wa), u01<T>(wb));
+            D = path_sample_ray<T>(pp, rng, x, y);
             n_rays++;                                 // trace_ray_traditional call count, chandelier.py:432
         };
         int fold_from = 0;                            // deepest-first fold stops at the level the path started on
@@ -1226,6 +1232,63 @@ __global__ void __launch_bounds__(256) trace_rays_kernel(SceneDev<T> sc, int m, 
     }
 }
 
+// First-hit features of an Algorithm B frame (rt_render_features, DESIGN §4.8d).  One thread per pixel of rows [y0, y1),
+// 32 x 8 pixels per CTA.  For samples [s0, s1) it traces the camera rays path_kernel traces (path_sample_ray) to their
+// nearest hit: albedo = colour / 255, normal = (p - centre) / r, depth = t; all 0 on a miss.  Per pixel: the mean of
+// every channel and, per feature, the variance of the mean averaged over its channels.  The sums are doubles added in
+// sample order by one thread, so the result does not depend on the launch.
+template <typename T, int kMode>
+__global__ void __launch_bounds__(256) feature_kernel(SceneDev<T> sc, PathDev<T> pp, float *albedo, float *normal,
+                                                      float *depth, float *fvar) {
+    RT_MODE_DECL;
+    extern __shared__ __align__(32) unsigned char smem[];
+    Staged<T> S;
+    stage_scene<T, kShared>(sc, smem, S);
+    const int x = blockIdx.x * 32 + (threadIdx.x & 31), y = pp.y0 + blockIdx.y * 8 + (threadIdx.x >> 5);
+    if (x >= pp.W || y >= pp.y1) return;
+    const uint32_t pixel = (uint32_t)(y * pp.W + x);
+    const V3<T> cam = mk<T>(pp.cam[0], pp.cam[1], pp.cam[2]);
+    PathRng rng;
+    unsigned n_tests = 0, n_boxes = 0;
+    double s[7] = {0, 0, 0, 0, 0, 0, 0}, q[7] = {0, 0, 0, 0, 0, 0, 0};   // albedo 0-2, normal 3-5, depth 6
+    for (int smp = pp.s0; smp < pp.s1; ++smp) {
+        rng.begin(pixel, (uint32_t)smp, pp.k0, pp.k1);
+        const V3<T> D = path_sample_ray<T>(pp, rng, x, y);
+        T t;
+        const int i = nearest<T, true, kBvh>(S.g, cam, D, RT_NO_ID_DEV, t, n_tests, n_boxes);
+        double f[7] = {0, 0, 0, 0, 0, 0, 0};
+        if (i >= 0) {
+            RT_ASSERT(i < sc.n);
+            const typename M<T>::v4 col = S.g.sv.col[i];
+            const V3<T> n = (cam + D * t - centre_of<T>(S.g.sv.sph[i])) * col.w;          // col.w = 1/r (finish_hit)
+            f[0] = (double)col.x / 255.0; f[1] = (double)col.y / 255.0; f[2] = (double)col.z / 255.0;
+            f[3] = (double)n.x; f[4] = (double)n.y; f[5] = (double)n.z; f[6] = (double)t;
+        }
+#pragma unroll
+        for (int c = 0; c < 7; ++c) { s[c] = __dadd_rn(s[c], f[c]); q[c] = __dadd_rn(q[c], __dmul_rn(f[c], f[c])); }
+    }
+    const int n = pp.s1 - pp.s0;
+    const double dn = (double)n;
+    // variance of the mean of channel c: (sum f^2 - (sum f)^2 / n) / (n (n - 1)), 0 below two samples; rounding can take a
+    // variance below zero, which is clamped
+    double v[7];
+#pragma unroll
+    for (int c = 0; c < 7; ++c) {
+        const double num = __dsub_rn(q[c], __ddiv_rn(__dmul_rn(s[c], s[c]), dn));
+        v[c] = n < 2 ? 0.0 : fmax(0.0, __ddiv_rn(num, __dmul_rn(dn, dn - 1.0)));
+    }
+    const size_t o = (size_t)y * pp.W + x;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        albedo[3 * o + c] = (float)__ddiv_rn(s[c], dn);
+        normal[3 * o + c] = (float)__ddiv_rn(s[3 + c], dn);
+    }
+    depth[o] = (float)__ddiv_rn(s[6], dn);
+    fvar[3 * o + 0] = (float)__ddiv_rn(__dadd_rn(__dadd_rn(v[0], v[1]), v[2]), 3.0);
+    fvar[3 * o + 1] = (float)__ddiv_rn(__dadd_rn(__dadd_rn(v[3], v[4]), v[5]), 3.0);
+    fvar[3 * o + 2] = (float)v[6];
+}
+
 template <typename T, int kMode>
 __global__ void __launch_bounds__(256) shade_hits_kernel(SceneDev<T> sc, int m, const double *hits, int shadow_max_bounces,
                                                          double *rgb) {
@@ -1802,6 +1865,16 @@ cudaError_t launch_trace_rays(const SceneDev<T> &sc, int m, const double *rays, 
 }
 
 template <typename T>
+cudaError_t launch_features(const SceneDev<T> &sc, const PathDev<T> &pp, float *albedo, float *normal, float *depth,
+                            float *fvar, cudaStream_t st) {
+    if (pp.y1 <= pp.y0 || pp.W <= 0 || pp.s1 <= pp.s0) return cudaSuccess;
+    const dim3 grid((unsigned)((pp.W + 31) / 32), (unsigned)((pp.y1 - pp.y0 + 7) / 8));
+    const int mode = mode_for(sc);
+    RT_DISPATCH_MODE(mode, feature_kernel, grid, 256, smem_for(sc), st, sc, pp, albedo, normal, depth, fvar);
+    return cudaGetLastError();
+}
+
+template <typename T>
 cudaError_t launch_shade_hits(const SceneDev<T> &sc, int m, const double *hits, int shadow_max_bounces, double *rgb,
                               cudaStream_t st) {
     if (m <= 0) return cudaSuccess;
@@ -1882,6 +1955,8 @@ cudaError_t launch_env_step(const SceneDev<T> &sc, const EnvDev<T> &e, const flo
                                               const int *, int, int, const double[3], double *, double *,              \
                                               cudaStream_t);                                                            \
     template cudaError_t launch_shade_hits<T>(const SceneDev<T> &, int, const double *, int, double *, cudaStream_t);    \
+    template cudaError_t launch_features<T>(const SceneDev<T> &, const PathDev<T> &, float *, float *, float *, float *, \
+                                            cudaStream_t);                                                              \
     template cudaError_t launch_env_reset<T>(const SceneDev<T> &, const EnvDev<T> &, const int *, const uint8_t *,      \
                                              uint64_t, float *, int *, unsigned long long *, cudaStream_t);             \
     template cudaError_t launch_env_reshade<T>(const SceneDev<T> &, const EnvDev<T> &, cudaStream_t);                   \

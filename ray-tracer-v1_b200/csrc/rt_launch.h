@@ -185,6 +185,11 @@ cudaError_t launch_trace_rays(const SceneDev<T> &sc, int m, const double *rays, 
 template <typename T>
 cudaError_t launch_shade_hits(const SceneDev<T> &sc, int m, const double *hits, int shadow_max_bounces, double *rgb,
                               cudaStream_t st);
+// first-hit features of rows [pp.y0, pp.y1) over samples [pp.s0, pp.s1) (rt_render_features): pp needs the camera, W, H,
+// the band, the sample range and the Philox keys; albedo / normal / fvar [H,W,3], depth [H,W] float32
+template <typename T>
+cudaError_t launch_features(const SceneDev<T> &sc, const PathDev<T> &pp, float *albedo, float *normal, float *depth,
+                            float *fvar, cudaStream_t st);
 template <typename T>
 cudaError_t launch_env_reset(const SceneDev<T> &sc, const EnvDev<T> &e, const int *pixels, const uint8_t *mask,
                              uint64_t seed, float *obs, int *pixels_out, unsigned long long *stats, cudaStream_t st);
@@ -223,6 +228,15 @@ cudaError_t launch_adaptive_resolve(const void *accum, const double *moments, in
 template <typename T>
 cudaError_t launch_denoise(const void *accum, const float *var, int W, int H, int r, int f, float k, float *image,
                            cudaStream_t st);
+// the same filter with the feature term (rt_denoise_features): albedo / normal / fvar [H,W,3] and depth [H,W] float32 as
+// rt_render_features gives them; k_f > 0, tau >= 0
+struct DenoiseFeatures {
+    const float *albedo, *normal, *depth, *fvar;
+    float kf2, tau;                      // k_f^2 and the floor of the feature denominators
+};
+template <typename T>
+cudaError_t launch_denoise_features(const void *accum, const float *var, const DenoiseFeatures &feat, int W, int H, int r,
+                                    int f, float k, float *image, cudaStream_t st);
 
 // FFMA issue-rate micro-benchmark (rt_f32.cu): `iters` trips of 16 independent FFMA per thread
 cudaError_t launch_fp32_peak(int blocks, int threads, int iters, float *sink, cudaStream_t st);

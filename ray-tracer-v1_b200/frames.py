@@ -15,6 +15,9 @@ __all__ = ["FrameContext"]
 
 class FrameContext:
     HOST_RING = 3
+    # feature frames trace their first-hit features over the first min(spp, FEATURE_SPP) samples of the frame: geometry
+    # converges in a few samples (DESIGN §4.8d)
+    FEATURE_SPP = 8
 
     def __init__(self, device=0):
         self.device = device
@@ -27,6 +30,11 @@ class FrameContext:
         # adaptive frames only: the active-pixel list ((H*W + 1) uint32) and the [H,W] int32 sample counts
         self.pixel_list = self.counts = None
         self.host_counts_ring, self.host_counts = [], None
+        # feature frames only: (albedo [H,W,3], normal [H,W,3], depth [H,W], fvar [H,W,3]) float32 in HBM, their pinned
+        # rings, and the host views of the last feature frame read back
+        self.features = None
+        self.host_features_ring = []
+        self.albedo = self.normal = self.depth = self.feature_var = None
         self.h2d_bytes = 0          # bytes of the last scene upload
         self.d2h_bytes = 0          # bytes of the last read-back
 
@@ -50,9 +58,11 @@ class FrameContext:
     # ---- buffers ---------------------------------------------------------------------------------------------
     def _buffers(self):
         return [self.accum, self.image, self.stats, self.hit, self.host_stats, self.moments, self.var, self.pixel_list,
-                self.counts] + list(getattr(self, "host_ring", [])) + list(self.host_var_ring) + list(self.host_counts_ring)
+                self.counts] + list(getattr(self, "host_ring", [])) + list(self.host_var_ring) + \
+            list(self.host_counts_ring) + list(self.features or ()) + [b for r in self.host_features_ring for b in r]
 
-    def ensure(self, W, H, precision=nat.F32, want_hit=False, want_variance=False, want_adaptive=False):
+    def ensure(self, W, H, precision=nat.F32, want_hit=False, want_variance=False, want_adaptive=False,
+               want_features=False):
         key = (int(W), int(H), precision)
         if self._key != key:
             for b in self._buffers():
@@ -73,6 +83,8 @@ class FrameContext:
             self.host_var_ring = []
             self.pixel_list = self.counts = None
             self.host_counts_ring = []
+            self.features = None
+            self.host_features_ring = []
             self._key = key
         if want_hit and self.hit is None:
             self.hit = nat.DeviceBuffer((H, W), np.int32, self.device)
@@ -86,10 +98,22 @@ class FrameContext:
             self.pixel_list = nat.DeviceBuffer(H * W + 1, np.uint32, self.device)
             self.counts = nat.DeviceBuffer((H, W), np.int32, self.device)
             self.host_counts_ring = [nat.PinnedArray((H, W), np.int32) for _ in range(self.HOST_RING)]
+        if want_features and self.features is None:
+            # allocated on the first feature frame
+            shapes = ((H, W, 3), (H, W, 3), (H, W), (H, W, 3))
+            self.features = tuple(nat.DeviceBuffer(s, np.float32, self.device) for s in shapes)
+            self.host_features_ring = [tuple(nat.PinnedArray(s, np.float32) for s in shapes) for _ in range(self.HOST_RING)]
+
+    def _render_features(self, cam, W, H, spp, seed, fov, precision, rows, s0, stream):
+        """The first-hit features of rows over samples [s0, s0 + min(spp, FEATURE_SPP)) into ``self.features``."""
+        p = self.scene.path_params(cam, W, H, spp, 1, 0.0, seed=seed, fov=fov, rows=rows,
+                                   samples=(s0, s0 + min(int(spp), self.FEATURE_SPP)))
+        self.scene.render_features(p, *self.features, precision=precision, stream=stream)
 
     # ---- frames ----------------------------------------------------------------------------------------------
     def render_path(self, cam, W, H, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, precision=nat.F32, rows=None,
-                    samples=None, resolve=True, read_back=True, stream=None, variance=False, denoise=False):
+                    samples=None, resolve=True, read_back=True, stream=None, variance=False, denoise=False,
+                    features=False):
         """Algorithm B over rows x samples of this rank.  Returns (host image view or None, stats u64[8] or None).
 
         variance=True: the launch also stores the second moments of every pixel's samples (``self.moments``), and the
@@ -100,23 +124,33 @@ class FrameContext:
         non-local-means filter of the frame (``rt_denoise`` with the library defaults) in place of the resolved one; the
         return shape is the one ``variance`` selects.  The filter reads every row, so the whole frame is rendered in one
         launch and read back once after the filter: the banded read-back overlap (``BANDS``) does not apply, and
-        ``rows`` must cover the frame."""
+        ``rows`` must cover the frame.
+
+        features=True: the frame's first-hit features (``rt_render_features`` over its first min(spp, FEATURE_SPP)
+        samples) are rendered too and, when read back, exposed as ``self.albedo`` [H,W,3], ``self.normal`` [H,W,3],
+        ``self.depth`` [H,W] and ``self.feature_var`` [H,W,3], views of pinned host rings like the image; with denoise,
+        the filter is the feature-guided one (``rt_denoise_features``, library defaults).  The return shape does not
+        change, and the banded read-back does not apply."""
         if denoise and (not resolve or (rows is not None and (int(rows[0]), int(rows[1])) != (0, int(H)))):
             raise ValueError("denoise filters the whole frame: it needs every row and resolve=True")
-        self.ensure(W, H, precision, want_variance=variance or denoise)
+        self.ensure(W, H, precision, want_variance=variance or denoise, want_features=features)
         L = nat.lib()
         p = self.scene.path_params(cam, W, H, spp, max_bounces, mirror_threshold, seed=seed, fov=fov, rows=rows,
                                    samples=samples)
         self.stats.fill(0, stream)
         moments = self.moments if (variance or denoise) else None
-        bands = self._bands(W, p.y0, p.y1, p.s1 - p.s0) if (resolve and read_back and not denoise) else None
+        bands = self._bands(W, p.y0, p.y1, p.s1 - p.s0) if (resolve and read_back and not denoise and not features) else None
         if bands:
             return self._render_path_banded(p, bands, W, H, precision, stream, variance)
         self.scene.render_path(p, self.accum, precision, stats=self.stats, stream=stream, moments=moments)
         self.launches = 1
+        if features:
+            self._render_features(cam, W, H, p.s1 - p.s0, seed, fov, precision, (p.y0, p.y1), p.s0, stream)
+            self.launches += 1
         if denoise:
             self.scene.resolve_variance(self.accum, self.moments, W, H, self.var, precision, stream=stream)
-            self.scene.denoise(self.accum, self.var, W, H, self.image, precision, stream=stream)
+            self.scene.denoise(self.accum, self.var, W, H, self.image, precision, stream=stream,
+                               features=self.features if features else None)
             self.launches += 2
         elif resolve:
             self.scene.resolve(self.accum, W, H, p.s1 - p.s0, self.image, precision, rows=(p.y0, p.y1), stream=stream)
@@ -127,7 +161,7 @@ class FrameContext:
                 self.launches += 1
         if not read_back:
             return (None, None, None) if variance else (None, None)
-        image, stats = self.read_back(W, H, (p.y0, p.y1), stream, variance=variance and resolve)
+        image, stats = self.read_back(W, H, (p.y0, p.y1), stream, variance=variance and resolve, features=features)
         if variance:
             return image, stats, (self.host_var.array if resolve else None)
         return image, stats
@@ -191,21 +225,25 @@ class FrameContext:
         return self.host_image.array, self.host_stats.array
 
     def render_path_adaptive(self, cam, W, H, max_spp, max_bounces, mirror_threshold, min_spp, tolerance, seed=0, fov=60.0,
-                             precision=nat.F32, stream=None, denoise=False):
+                             precision=nat.F32, stream=None, denoise=False, features=False):
         """Adaptive Algorithm B frame (``rt_render_path_adaptive``): every pixel gets ``min_spp`` samples, then the pixels
         whose variance of the mean still exceeds ``tolerance``^2 (colour levels) get doubling rounds up to ``max_spp``.
         Returns (image [H,W,3] float32, stats u64[8], variance [H,W,3] float32, sample counts [H,W] int32), views of
         pinned host rings like the image of ``render_path``.  The call synchronises the stream once per round.
         denoise=True: the image is the frame filtered by ``rt_denoise`` (library defaults), each pixel's mean and variance
-        taken at its own sample count."""
-        self.ensure(W, H, precision, want_variance=True, want_adaptive=True)
+        taken at its own sample count.
+        features=True: as for ``render_path``, over the first min(max_spp, FEATURE_SPP) samples."""
+        self.ensure(W, H, precision, want_variance=True, want_adaptive=True, want_features=features)
         p = self.scene.path_params(cam, W, H, max_spp, max_bounces, mirror_threshold, seed=seed, fov=fov)
         self.stats.fill(0, stream)
+        if features:
+            self._render_features(cam, W, H, max_spp, seed, fov, precision, (0, H), 0, stream)
         self.scene.render_path_adaptive(p, min_spp, tolerance, self.accum, self.moments, self.pixel_list, self.image,
                                         precision, var=self.var, counts=self.counts, stats=self.stats, stream=stream)
         if denoise:
-            self.scene.denoise(self.accum, self.var, W, H, self.image, precision, stream=stream)
-        image, stats = self.read_back(W, H, (0, H), stream, variance=True, counts=True)
+            self.scene.denoise(self.accum, self.var, W, H, self.image, precision, stream=stream,
+                               features=self.features if features else None)
+        image, stats = self.read_back(W, H, (0, H), stream, variance=True, counts=True, features=features)
         return image, stats, self.host_var.array, self.host_counts.array
 
     def render_whitted(self, cam, X, Y, spp=1, max_bounces=1, shadow_max_bounces=0, miss=None, seed=0, prenorm=False,
@@ -222,10 +260,11 @@ class FrameContext:
             return None, None
         return self.read_back(W, H, (p.y0, p.y1), stream)
 
-    def read_back(self, W, H, rows, stream=None, variance=False, counts=False):
+    def read_back(self, W, H, rows, stream=None, variance=False, counts=False, features=False):
         """D2H of the resolved rows (float32) + the stats block into pinned memory; synchronises the stream.  variance:
         the rows of the variance image too, into ``self.host_var`` (the pinned ring slot of this frame); counts: those
-        of the int32 sample counts of an adaptive frame, into ``self.host_counts``."""
+        of the int32 sample counts of an adaptive frame, into ``self.host_counts``; features: those of the feature
+        buffers, exposed as ``self.albedo``, ``self.normal``, ``self.depth`` and ``self.feature_var``."""
         L = nat.lib()
         y0, y1 = rows
         self._ring_at = (self._ring_at + 1) % self.HOST_RING
@@ -242,9 +281,17 @@ class FrameContext:
             if nbytes:
                 nat.check(L.rt_memcpy_d2h(self.device, self.host_counts.ptr + off // 3, self.counts.ptr + off // 3, nbytes // 3,
                                           stream))
+        if features:
+            host = self.host_features_ring[self._ring_at]
+            for h, d in zip(host, self.features):
+                k = 1 if h.array.ndim == 2 else 3          # depth has one channel
+                if nbytes:
+                    nat.check(L.rt_memcpy_d2h(self.device, h.ptr + off // 3 * k, d.ptr + off // 3 * k, nbytes // 3 * k,
+                                              stream))
+            self.albedo, self.normal, self.depth, self.feature_var = (h.array for h in host)
         nat.check(L.rt_memcpy_d2h(self.device, self.host_stats.ptr, self.stats.ptr, 64, stream))
         nat.check(L.rt_stream_sync(self.device, stream))
-        self.d2h_bytes = nbytes * (2 if variance else 1) + (nbytes // 3 if counts else 0) + 64
+        self.d2h_bytes = nbytes * (2 if variance else 1) + (nbytes // 3 if counts else 0) + (nbytes // 3 * 10 if features else 0) + 64
         return self.host_image.array, self.host_stats.array
 
     def close(self):
@@ -254,7 +301,9 @@ class FrameContext:
         self.host_ring = []
         self.host_var_ring = []
         self.host_counts_ring = []
-        self.moments = self.var = self.pixel_list = self.counts = None
+        self.host_features_ring = []
+        self.moments = self.var = self.pixel_list = self.counts = self.features = None
+        self.albedo = self.normal = self.depth = self.feature_var = None
         if getattr(self, "_copy_stream", None) is not None:
             nat.lib().rt_stream_destroy(self.device, self._copy_stream)
             self._copy_stream = None

@@ -134,6 +134,10 @@ class TraditionalRenderer:
     # True: render() returns the frame filtered by the variance-guided non-local-means filter (rt_denoise, library
     # defaults; DESIGN §4.8c), from the frame's own per-pixel variance; combines with track_variance and adaptive_tolerance
     denoise = False
+    # True: render() also sets self.albedo [H,W,3], self.normal [H,W,3] and self.depth [H,W] (float32), the first-hit
+    # features of the frame's first FrameContext.FEATURE_SPP samples, and a denoised frame uses the feature-guided filter
+    # (rt_denoise_features, library defaults; DESIGN §4.8d); combines with track_variance and adaptive_tolerance
+    track_features = False
 
     def __init__(self, device=0, precision="f32", seed=None):
         self.scene = []
@@ -206,15 +210,19 @@ class TraditionalRenderer:
             out = self._ctx.render_path_adaptive(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
                                                  self.mirror_threshold, min(self.adaptive_min_spp, samples_per_pixel),
                                                  self.adaptive_tolerance, seed=seed, fov=self.fov,
-                                                 precision=_precision(self.precision), denoise=self.denoise)
+                                                 precision=_precision(self.precision), denoise=self.denoise,
+                                                 features=self.track_features)
             self.sample_counts = out[3] if self.reuse_output else out[3].copy()
         else:
             out = self._ctx.render_path(_xyz(self.camera_position), width, height, samples_per_pixel, max_bounces,
                                         self.mirror_threshold, seed=seed, fov=self.fov, precision=_precision(self.precision),
-                                        variance=self.track_variance, denoise=self.denoise)
+                                        variance=self.track_variance, denoise=self.denoise, features=self.track_features)
         view, st = out[:2]
         if self.track_variance:
             self.variance = out[2] if self.reuse_output else out[2].copy()
+        if self.track_features:
+            c = self._ctx
+            self.albedo, self.normal, self.depth = ((a if self.reuse_output else a.copy()) for a in (c.albedo, c.normal, c.depth))
         # reuse_output (default True): the image is a view of one of the renderer's FrameContext.HOST_RING pinned host
         # buffers -- it stays valid until two more frames have been rendered by THIS renderer, which covers every use
         # in the reference's drivers (plot / save / compare right after render()).  reuse_output = False returns a
