@@ -233,9 +233,11 @@ int rt_resolve_variance(int device, int precision, const void *accum_dev, const 
  * float32, not clamped), V = var, eps = 255^2 * 1e-10 and reads clamped into the frame (each pixel of a pair on its own):
  *   delta(p,q) = 1/3 sum_c [(u_p - u_q)^2 - (V_p + min(V_p, V_q))] / [eps + k^2 (V_p + V_q)]
  *   D(p,o)     = mean of delta(p+t, p+t+o) over t in [-patch_radius, patch_radius]^2, o in [-radius, radius]^2
- *   out_p      = sum_o exp(-max(0, D)) u_{p+o} / sum_o exp(-max(0, D))
- * image_dev [H,W,3] float32 = min(1, floor(out) / 255), the lattice of rt_resolve.  FP32 arithmetic for both
- * precisions, fixed summation order: the same input gives the same bits.  Enqueued on the stream.  RT_ERR_INVALID for
+ *   out_p      = u_p + sum_o exp(-max(0, D)) (u_{p+o} - u_p) / sum_o exp(-max(0, D))
+ * image_dev [H,W,3] float32 = min(1, floor(out) / 255), the lattice of rt_resolve; a window of one colour returns u_p
+ * exactly.  k^2 is formed in double and clamped to FLT_MAX, so any finite k above sqrt(FLT_MAX) acts as k -> infinity.
+ * FP32 arithmetic for both precisions, fixed summation order: the same input gives the same bits.  Enqueued on the
+ * stream.  RT_ERR_INVALID for
  * a NULL pointer, W or H < 1, an unknown precision, radius outside [0,15], patch_radius outside [0,5], or k not finite
  * or not > 0.  Defaults: radius 10, patch_radius 3, k 0.45. */
 typedef struct rt_denoise_params {
@@ -262,8 +264,10 @@ int rt_render_features(rt_scene *scene, int precision, const rt_path_params *p, 
  *   G_j,p     = mean_c [((f(x+1,y) - f(x-1,y)) / 2)^2 + ((f(x,y+1) - f(x,y-1)) / 2)^2]
  *   Phi_j(p,q)= [mean_c (f_j,p - f_j,q)^2 - (Var_j,p + min(Var_j,p, Var_j,q))] / [k_f^2 max(tau, Var_j,p, G_j,p)]
  *   w         = min(w_c, exp(-max(0, max_j Phi_j)))          (w_c = rt_denoise's weight exp(-max(0, D)))
- * and out_p = sum_o w u_{p+o} / sum_o w, on the same lattice.  Features can only lower a colour weight: k_f -> infinity
- * gives rt_denoise's image.  Validation as rt_denoise, and RT_ERR_INVALID for a NULL feature pointer, k_f not finite or
+ * and out_p = u_p + sum_o w (u_{p+o} - u_p) / sum_o w, on the same lattice.  Features can only lower a colour weight: k_f -> infinity
+ * gives rt_denoise's image; k_f^2 is clamped to FLT_MAX as k^2 is.  Where max(tau, Var_j,p, G_j,p) = 0 (tau = 0 and flat
+ * features) Phi_j is +inf for a pair that differs in feature j and is ignored for a pair that does not.  Validation as
+ * rt_denoise, and RT_ERR_INVALID for a NULL feature pointer, k_f not finite or
  * not > 0, or tau not finite or < 0.  Defaults (measured, DESIGN §4.8d): radius 10, patch_radius 3, k 1.0, k_f 1.2,
  * tau 1e-3. */
 typedef struct rt_denoise_features_params {

@@ -1146,7 +1146,7 @@ RT_EXPORT int rt_denoise_features(int device, int precision, const void *accum_d
     if (!std::isfinite(d->k_f) || !(d->k_f > 0.0f)) return fail(RT_ERR_INVALID, "k_f must be finite and > 0");
     if (!std::isfinite(d->tau) || !(d->tau >= 0.0f)) return fail(RT_ERR_INVALID, "tau must be finite and >= 0");
     CU(cudaSetDevice(device));
-    const DenoiseFeatures feat = {albedo_dev, normal_dev, depth_dev, fvar_dev, d->k_f * d->k_f, d->tau};
+    const DenoiseFeatures feat = {albedo_dev, normal_dev, depth_dev, fvar_dev, square_to_float(d->k_f), d->tau};
     if (precision == RT_F64)
         CU(launch_denoise_features<double>(accum_dev, var_dev, feat, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
     else

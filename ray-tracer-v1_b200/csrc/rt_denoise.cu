@@ -5,7 +5,9 @@
 // For pixel p with mean u_p = S_p / n_p (levels) and variance of the mean V_p (levels^2), per offset o in [-r, r]^2:
 //   delta(p, q) = 1/3 sum_c [(u_p,c - u_q,c)^2 - (V_p,c + min(V_p,c, V_q,c))] / [eps + k^2 (V_p,c + V_q,c)]
 //   D(p, o)     = mean of delta(p + t, p + t + o) over t in [-f, f]^2,   w = exp(-max(0, D))
-//   out_p       = sum_o w u_{p+o} / sum_o w   -> image = min(1, floor(out) / 255)
+//   out_p       = u_p + sum_o w (u_{p+o} - u_p) / sum_o w   -> image = min(1, floor(out) / 255)
+// The sum is taken about the centre u_p so that a window of one colour returns u_p exactly: sum_o w u_{p+o} / sum_o w
+// can round just below an integer u_p for fractional weights, and the floor then takes it one level down.
 // every read at (x, y) clamped into the frame, the two pixels of a pair independently.
 //
 // kFeatures (rt_denoise_features, DESIGN §4.8d) adds the feature term of Rousselle, Manzi and Zwicker 2013, per pixel and
@@ -106,6 +108,7 @@ RT_DEV void denoise_nlm(const typename M<T>::v4 *__restrict__ accum, const float
     const int P = 2 * f + 1;
     const float inv_area = 1.0f / (float)(P * P);
     float sw = 0.f, s0 = 0.f, s1 = 0.f, s2 = 0.f;
+    const float uc0 = su[hc], uc1 = su[LL + hc], uc2 = su[2 * LL + hc];
     // kFeatures: p's features, variances and 1 / (k_f^2 max(tau, Var_j,p, G_j,p)); G from clamped global reads
     float fp[7], vfp[3], inv_den[3];
     const int hcf = (py + r) * LF + (px + r);                // this thread's output pixel in the feature halo
@@ -186,16 +189,16 @@ RT_DEV void denoise_nlm(const typename M<T>::v4 *__restrict__ accum, const float
             const float w = __expf(-fmaxf(0.f, e));
             const int q = hc + d;
             sw += w;
-            s0 = fmaf(w, su[q], s0);
-            s1 = fmaf(w, su[LL + q], s1);
-            s2 = fmaf(w, su[2 * LL + q], s2);
+            s0 = fmaf(w, su[q] - uc0, s0);
+            s1 = fmaf(w, su[LL + q] - uc1, s1);
+            s2 = fmaf(w, su[2 * LL + q] - uc2, s2);
         }
     }
 
     const int x = blockIdx.x * kTile + px, y = blockIdx.y * kTile + py;
     if (x >= W || y >= H) return;
     // o = 0 has weight 1, so sw >= 1; the lattice is rt_resolve's: min(1, floor(value) / 255) rounded from double
-    const float vals[3] = {s0 / sw, s1 / sw, s2 / sw};
+    const float vals[3] = {uc0 + s0 / sw, uc1 + s1 / sw, uc2 + s2 / sw};
     const size_t o = (size_t)y * W + x;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
@@ -236,14 +239,14 @@ template <typename T>
 cudaError_t launch_denoise(const void *accum, const float *var, int W, int H, int r, int f, float k, float *image,
                            cudaStream_t st) {
     return launch_nlm(denoise_nlm_kernel<T>, false, W, H, r, f, st, (const typename M<T>::v4 *)accum, var, W, H, r, f,
-                      k * k, image);
+                      square_to_float(k), image);
 }
 
 template <typename T>
 cudaError_t launch_denoise_features(const void *accum, const float *var, const DenoiseFeatures &feat, int W, int H, int r,
                                     int f, float k, float *image, cudaStream_t st) {
     return launch_nlm(denoise_nlm_features_kernel<T>, true, W, H, r, f, st, (const typename M<T>::v4 *)accum, var, W, H,
-                      r, f, k * k, image, feat);
+                      r, f, square_to_float(k), image, feat);
 }
 
 template cudaError_t launch_denoise<float>(const void *, const float *, int, int, int, int, float, float *, cudaStream_t);

@@ -1,6 +1,7 @@
 // rt_launch.h -- kernel parameter blocks and launcher declarations shared by the two kernel translation units
 // (rt_f32.cu: float, FMA-contracted; rt_f64.cu: double, -fmad=false) and the C-ABI layer (rt_api.cu).
 #pragma once
+#include <cfloat>
 #include "rt_common.cuh"
 
 namespace rt {
@@ -234,6 +235,12 @@ struct DenoiseFeatures {
     const float *albedo, *normal, *depth, *fvar;
     float kf2, tau;                      // k_f^2 and the floor of the feature denominators
 };
+// k^2 and k_f^2 for the filter: squared in double and clamped to FLT_MAX, so that a finite k above sqrt(FLT_MAX) keeps
+// the limit k -> infinity (FLT_MAX * 0 = 0 for zero variance; an infinite product gives delta = 0) instead of inf * 0
+inline float square_to_float(float k) {
+    const double k2 = (double)k * k;
+    return k2 < (double)FLT_MAX ? (float)k2 : FLT_MAX;
+}
 template <typename T>
 cudaError_t launch_denoise_features(const void *accum, const float *var, const DenoiseFeatures &feat, int W, int H, int r,
                                     int f, float k, float *image, cudaStream_t st);

@@ -25,7 +25,8 @@ def nat(rt):
 
 
 def nlm_reference(acc, var, radius=10, patch_radius=3, k=0.45):
-    """The filter in float64 -> the filtered mean u_hat [H,W,3] in levels, before the floor."""
+    """The filter in float64 -> the filtered mean u_hat [H,W,3] in levels, before the floor.  The weighted sum is taken
+    about the centre, u_p + sum w (u_q - u_p) / sum w, as the kernel takes it: a window of one colour gives u_p exactly."""
     r, f = radius, patch_radius
     n = acc[..., 3:4].astype(np.float64)
     u = (acc[..., :3].astype(np.float64) / n).astype(np.float32).astype(np.float64)
@@ -47,8 +48,8 @@ def nlm_reference(acc, var, radius=10, patch_radius=3, k=0.45):
             D = sum(rows[t:t + H] for t in range(P)) / (P * P)
             w = np.exp(-np.maximum(0.0, D))[..., None]
             sw += w
-            su += w * at(u, np.arange(H) + oy, np.arange(W) + ox)
-    return su / sw
+            su += w * (at(u, np.arange(H) + oy, np.arange(W) + ox) - u)
+    return u + su / sw
 
 
 def lattice(values):
@@ -56,9 +57,10 @@ def lattice(values):
     return np.minimum(1.0, np.floor(values) / 255.0).astype(np.float32)
 
 
-def check_against_reference(img, u_hat):
+def check_against_reference(img, u_hat, min_far=None):
+    """min_far: the least number of values that must lie far from an integer (default: more than half of them)."""
     far = np.abs(u_hat - np.rint(u_hat)) > 1e-2
-    assert far.mean() > 0.5
+    assert (far.mean() > 0.5) if min_far is None else (far.sum() >= min_far), far.sum()
     assert np.array_equal(img[far], lattice(u_hat)[far])
     got = np.rint(img.astype(np.float64) * 255.0)
     assert np.abs(got - np.minimum(255.0, np.floor(u_hat))).max() <= 1

@@ -120,6 +120,9 @@ def feature_frames():
     z, fs = load_golden("path_chandelier_48x27")
     yield "chandelier+lbvh", fs, z["cam"], 64, 36, True
     yield "2000 spheres", scenes.build_many_spheres_flat(2000, seed=2, emissive_fraction=0.05), (0.0, 2.0, 0.0), 40, 24, True
+    z, fs = load_golden("path_complex_48x27")
+    yield "complex 33x9", fs, z["cam"], 33, 9, False          # one column and one row into a second 32 x 8 CTA
+    yield "complex 1x24", fs, z["cam"], 1, 24, False
 
 
 # FP32 features may differ from the reference only where an FP32 ray flips a hit, at silhouettes: a pixel whose sample
@@ -130,14 +133,16 @@ FP32_FLIP_LIMIT = 0.0
 
 @pytest.mark.parametrize("precision", PRECISIONS)
 def test_features_match_reference(nat, orc, precision):
-    """Every scene-residency mode (shared, shared + LBVH, global + LBVH), a row band and a sample range."""
+    """Every scene-residency mode (shared, shared + LBVH, global + LBVH), frames one pixel past a CTA in x and y and one
+    pixel wide, row bands (one of a single row) and sample ranges (one far from 0)."""
     prec = getattr(nat, precision)
     for name, fs, cam, W, H, lbvh in feature_frames():
         sc = nat.DeviceScene(fs)
         if lbvh:
             sc.build_lbvh()
             assert sc.has_lbvh
-        for rows, samples in (((0, H), (0, 8)), ((5, H - 7), (3, 7)), ((0, H), (2, 3))):
+        bands = [((0, H), (0, 8)), ((0, H), (2, 3)), ((H // 2, H // 2 + 1), (1000, 1004))]
+        for rows, samples in bands + ([((5, H - 7), (3, 7))] if H > 12 else []):
             got = render_features(nat, sc, cam, W, H, 11, prec, rows, samples, fill=0x7F)
             ref = aov_reference(orc, fs, cam, W, H, 11, rows, samples)
             y0, y1 = rows
@@ -206,8 +211,8 @@ def nlm_features_reference(acc, var, feats, radius=10, patch_radius=3, k=1.0, k_
                     e = np.fmax(e, num / den[j])
             w = np.exp(-np.maximum(0.0, e))[..., None]
             sw += w
-            su += w * at(u, Y + oy, X + ox)
-    return su / sw
+            su += w * (at(u, Y + oy, X + ox) - u)
+    return u + su / sw
 
 
 def uniform(nat, sc, frame, spp, prec, seed):
