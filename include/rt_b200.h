@@ -281,6 +281,22 @@ typedef struct rt_denoise_features_params {
 int rt_denoise_features(int device, int precision, const void *accum_dev, const float *var_dev, const float *albedo_dev,
                         const float *normal_dev, const float *depth_dev, const float *fvar_dev, int32_t W, int32_t H,
                         const rt_denoise_features_params *d, float *image_dev, void *stream);
+/* rt_denoise / rt_denoise_features for the output rows [y0, y1) only (DESIGN §4.8e): the building block of a frame
+ * denoised in row bands, one per GPU.  Buffers and indexing stay those of the whole frame ([H,W,.]), as for rt_resolve.
+ * With h = rt_denoise_halo(radius, patch_radius, features), the call reads only rows [max(0, y0 - h), min(H, y1 + h))
+ * of accum_dev, var_dev and the feature buffers -- every read is clamped into that window -- and writes only rows
+ * [y0, y1) of image_dev.  Those rows equal the same rows of the whole-frame call bit for bit, whatever the other rows
+ * of the inputs hold.  Validation as the whole-frame calls, and RT_ERR_INVALID unless 0 <= y0 < y1 <= H. */
+int rt_denoise_rows(int device, int precision, const void *accum_dev, const float *var_dev, int32_t W, int32_t H,
+                    int32_t y0, int32_t y1, const rt_denoise_params *d, float *image_dev, void *stream);
+int rt_denoise_features_rows(int device, int precision, const void *accum_dev, const float *var_dev,
+                             const float *albedo_dev, const float *normal_dev, const float *depth_dev,
+                             const float *fvar_dev, int32_t W, int32_t H, int32_t y0, int32_t y1,
+                             const rt_denoise_features_params *d, float *image_dev, void *stream);
+/* *rows = the halo depth h of the filter: the rows an output row reads lie within h of it.  radius + patch_radius for
+ * rt_denoise (features = 0); max(radius + patch_radius, 1) for rt_denoise_features (features != 0), whose feature
+ * gradient reads y +- 1.  RT_ERR_INVALID for NULL rows, radius outside [0,15] or patch_radius outside [0,5]. */
+int rt_denoise_halo(int32_t radius, int32_t patch_radius, int32_t features, int32_t *rows);
 
 /* ---- "Algorithm C" frame: SimplifiedFBRenderer.render_original_style / trace_ray_simple /
  *      calculate_lighting_exact_original in traditional mode (fb_usage_prob = 0): FB/output6.py:197-306, :434-654.

@@ -155,6 +155,11 @@ SIGNATURES = {
     "rt_render_features": (C.c_int, [vp, C.c_int, C.POINTER(PathParams), vp, vp, vp, vp, vp]),
     "rt_denoise_features": (C.c_int, [C.c_int, C.c_int, vp, vp, vp, vp, vp, vp, C.c_int32, C.c_int32,
                                       C.POINTER(DenoiseFeaturesParams), vp, vp]),
+    "rt_denoise_rows": (C.c_int, [C.c_int, C.c_int, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                  C.POINTER(DenoiseParams), vp, vp]),
+    "rt_denoise_features_rows": (C.c_int, [C.c_int, C.c_int, vp, vp, vp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int32,
+                                           C.c_int32, C.POINTER(DenoiseFeaturesParams), vp, vp]),
+    "rt_denoise_halo": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, c_ip]),
     "rt_wf_create": (C.c_int, [vp, C.c_int, C.c_int32, C.c_int32, C.POINTER(vp)]),
     "rt_wf_destroy": (C.c_int, [vp]),
     "rt_wf_begin": (C.c_int, [vp, C.POINTER(PathParams), C.c_double, vp, vp]),
@@ -260,6 +265,14 @@ def measure_fp32_peak(device=0, repeats=5):
     tf, ms = C.c_double(0), C.c_double(0)
     check(lib().rt_measure_fp32_peak(device, repeats, C.byref(tf), C.byref(ms)))
     return float(tf.value), float(ms.value)
+
+
+def denoise_halo(radius=10, patch_radius=3, features=False):
+    """The halo depth h of the filter (``rt_denoise_halo``): the rows an output row reads lie within h of it, so a row
+    band [y0, y1) of ``DeviceScene.denoise(..., rows=)`` reads only rows [y0 - h, y1 + h) of the frame.  Needs no GPU."""
+    h = C.c_int32(0)
+    check(load_symbols().rt_denoise_halo(int(radius), int(patch_radius), int(bool(features)), C.byref(h)))
+    return int(h.value)
 
 
 def _ptr(x):
@@ -548,25 +561,30 @@ class DeviceScene:
                                         _ptr(var), stream))
 
     def denoise(self, accum, var, W, H, image, precision=F32, radius=10, patch_radius=3, k=None, stream=None,
-                features=None, k_f=1.2, tau=1e-3):
+                features=None, k_f=1.2, tau=1e-3, rows=None):
         """accum [H,W,4] + var [H,W,3] float32 (``resolve_variance``) -> image [H,W,3] float32: the whole frame filtered
         by the variance-guided non-local-means filter (``rt_denoise``), on rt_resolve's lattice.  Per-pixel sample counts
         may differ (adaptive frames).  ``features`` = (albedo, normal, depth, fvar) as ``render_features`` gives them:
         the filter with the feature term (``rt_denoise_features``), with ``k_f`` and ``tau``.  k defaults to 0.45
-        without features and 1.0 with them (the defaults measured in DESIGN §4.8c and §4.8d)."""
+        without features and 1.0 with them (the defaults measured in DESIGN §4.8c and §4.8d).
+        ``rows`` = (y0, y1): only those rows of the image (``rt_denoise_rows`` / ``rt_denoise_features_rows``), equal to
+        the same rows of the whole-frame filter; the inputs are read only within ``denoise_halo`` rows of the band."""
         if k is None:
             k = 0.45 if features is None else 1.0
+        band = () if rows is None else (int(rows[0]), int(rows[1]))
         if features is None:
             d = DenoiseParams()
             d.radius, d.patch_radius, d.k = int(radius), int(patch_radius), float(k)
-            check(lib().rt_denoise(self.device, precision, _ptr(accum), _ptr(var), int(W), int(H), C.byref(d), _ptr(image),
-                                   stream))
+            fn = lib().rt_denoise if rows is None else lib().rt_denoise_rows
+            check(fn(self.device, precision, _ptr(accum), _ptr(var), int(W), int(H), *band, C.byref(d), _ptr(image),
+                     stream))
             return
         albedo, normal, depth, fvar = features
         d = DenoiseFeaturesParams()
         d.radius, d.patch_radius, d.k, d.k_f, d.tau = int(radius), int(patch_radius), float(k), float(k_f), float(tau)
-        check(lib().rt_denoise_features(self.device, precision, _ptr(accum), _ptr(var), _ptr(albedo), _ptr(normal),
-                                        _ptr(depth), _ptr(fvar), int(W), int(H), C.byref(d), _ptr(image), stream))
+        fn = lib().rt_denoise_features if rows is None else lib().rt_denoise_features_rows
+        check(fn(self.device, precision, _ptr(accum), _ptr(var), _ptr(albedo), _ptr(normal), _ptr(depth), _ptr(fvar),
+                 int(W), int(H), *band, C.byref(d), _ptr(image), stream))
 
     def render_features(self, params, albedo, normal, depth, fvar, precision=F32, stream=None):
         """First-hit features of rows [y0, y1) over samples [s0, s1) of ``params`` (``rt_render_features``): the camera

@@ -346,7 +346,7 @@ static inline cudaStream_t S(void *stream) { return reinterpret_cast<cudaStream_
 
 // ------------------------------------------------------------------ library / device
 RT_EXPORT const char *rt_last_error(void) { return g_err.c_str(); }
-RT_EXPORT int rt_version(void) { return 105; }
+RT_EXPORT int rt_version(void) { return 106; }
 
 RT_EXPORT int rt_device_count(int *count) {
     if (!count) return fail(RT_ERR_INVALID, "count is NULL");
@@ -1116,14 +1116,33 @@ RT_EXPORT int rt_resolve_variance(int device, int precision, const void *accum_d
     return RT_OK;
 }
 
-RT_EXPORT int rt_denoise(int device, int precision, const void *accum_dev, const float *var_dev, int32_t W, int32_t H,
-                         const rt_denoise_params *d, float *image_dev, void *stream) {
+// the checks the four filter entries share, in the order rt_denoise and rt_denoise_features made them
+template <typename P>
+static int check_denoise(int precision, const void *accum_dev, const float *var_dev, const P *d, const float *image_dev,
+                         int32_t W, int32_t H, bool feature_missing) {
     if (!accum_dev || !var_dev || !d || !image_dev) return fail(RT_ERR_INVALID, "NULL argument");
+    if (feature_missing) return fail(RT_ERR_INVALID, "NULL feature buffer");
     if (W < 1 || H < 1) return fail(RT_ERR_INVALID, "W and H must be at least 1");
     if (precision != RT_F32 && precision != RT_F64) return fail(RT_ERR_INVALID, "unknown precision");
     if (d->radius < 0 || d->radius > 15) return fail(RT_ERR_INVALID, "radius must be in [0, 15]");
     if (d->patch_radius < 0 || d->patch_radius > 5) return fail(RT_ERR_INVALID, "patch_radius must be in [0, 5]");
     if (!std::isfinite(d->k) || !(d->k > 0.0f)) return fail(RT_ERR_INVALID, "k must be finite and > 0");
+    return RT_OK;
+}
+static int check_denoise_features(const rt_denoise_features_params *d) {
+    if (!std::isfinite(d->k_f) || !(d->k_f > 0.0f)) return fail(RT_ERR_INVALID, "k_f must be finite and > 0");
+    if (!std::isfinite(d->tau) || !(d->tau >= 0.0f)) return fail(RT_ERR_INVALID, "tau must be finite and >= 0");
+    return RT_OK;
+}
+static int check_denoise_rows(int32_t H, int32_t y0, int32_t y1) {
+    if (!(0 <= y0 && y0 < y1 && y1 <= H)) return fail(RT_ERR_INVALID, "rows [y0, y1) must satisfy 0 <= y0 < y1 <= H");
+    return RT_OK;
+}
+
+RT_EXPORT int rt_denoise(int device, int precision, const void *accum_dev, const float *var_dev, int32_t W, int32_t H,
+                         const rt_denoise_params *d, float *image_dev, void *stream) {
+    int rc = check_denoise(precision, accum_dev, var_dev, d, image_dev, W, H, false);
+    if (rc) return rc;
     CU(cudaSetDevice(device));
     if (precision == RT_F64)
         CU(launch_denoise<double>(accum_dev, var_dev, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
@@ -1136,21 +1155,55 @@ RT_EXPORT int rt_denoise_features(int device, int precision, const void *accum_d
                                   const float *albedo_dev, const float *normal_dev, const float *depth_dev,
                                   const float *fvar_dev, int32_t W, int32_t H, const rt_denoise_features_params *d,
                                   float *image_dev, void *stream) {
-    if (!accum_dev || !var_dev || !d || !image_dev) return fail(RT_ERR_INVALID, "NULL argument");
-    if (!albedo_dev || !normal_dev || !depth_dev || !fvar_dev) return fail(RT_ERR_INVALID, "NULL feature buffer");
-    if (W < 1 || H < 1) return fail(RT_ERR_INVALID, "W and H must be at least 1");
-    if (precision != RT_F32 && precision != RT_F64) return fail(RT_ERR_INVALID, "unknown precision");
-    if (d->radius < 0 || d->radius > 15) return fail(RT_ERR_INVALID, "radius must be in [0, 15]");
-    if (d->patch_radius < 0 || d->patch_radius > 5) return fail(RT_ERR_INVALID, "patch_radius must be in [0, 5]");
-    if (!std::isfinite(d->k) || !(d->k > 0.0f)) return fail(RT_ERR_INVALID, "k must be finite and > 0");
-    if (!std::isfinite(d->k_f) || !(d->k_f > 0.0f)) return fail(RT_ERR_INVALID, "k_f must be finite and > 0");
-    if (!std::isfinite(d->tau) || !(d->tau >= 0.0f)) return fail(RT_ERR_INVALID, "tau must be finite and >= 0");
+    int rc = check_denoise(precision, accum_dev, var_dev, d, image_dev, W, H,
+                           !albedo_dev || !normal_dev || !depth_dev || !fvar_dev);
+    if (rc || (rc = check_denoise_features(d))) return rc;
     CU(cudaSetDevice(device));
     const DenoiseFeatures feat = {albedo_dev, normal_dev, depth_dev, fvar_dev, square_to_float(d->k_f), d->tau};
     if (precision == RT_F64)
         CU(launch_denoise_features<double>(accum_dev, var_dev, feat, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
     else
         CU(launch_denoise_features<float>(accum_dev, var_dev, feat, W, H, d->radius, d->patch_radius, d->k, image_dev, S(stream)));
+    return RT_OK;
+}
+
+RT_EXPORT int rt_denoise_rows(int device, int precision, const void *accum_dev, const float *var_dev, int32_t W, int32_t H,
+                              int32_t y0, int32_t y1, const rt_denoise_params *d, float *image_dev, void *stream) {
+    int rc = check_denoise(precision, accum_dev, var_dev, d, image_dev, W, H, false);
+    if (rc || (rc = check_denoise_rows(H, y0, y1))) return rc;
+    CU(cudaSetDevice(device));
+    if (precision == RT_F64)
+        CU(launch_denoise_rows<double>(accum_dev, var_dev, W, H, y0, y1, d->radius, d->patch_radius, d->k, image_dev,
+                                       S(stream)));
+    else
+        CU(launch_denoise_rows<float>(accum_dev, var_dev, W, H, y0, y1, d->radius, d->patch_radius, d->k, image_dev,
+                                      S(stream)));
+    return RT_OK;
+}
+
+RT_EXPORT int rt_denoise_features_rows(int device, int precision, const void *accum_dev, const float *var_dev,
+                                       const float *albedo_dev, const float *normal_dev, const float *depth_dev,
+                                       const float *fvar_dev, int32_t W, int32_t H, int32_t y0, int32_t y1,
+                                       const rt_denoise_features_params *d, float *image_dev, void *stream) {
+    int rc = check_denoise(precision, accum_dev, var_dev, d, image_dev, W, H,
+                           !albedo_dev || !normal_dev || !depth_dev || !fvar_dev);
+    if (rc || (rc = check_denoise_features(d)) || (rc = check_denoise_rows(H, y0, y1))) return rc;
+    CU(cudaSetDevice(device));
+    const DenoiseFeatures feat = {albedo_dev, normal_dev, depth_dev, fvar_dev, square_to_float(d->k_f), d->tau};
+    if (precision == RT_F64)
+        CU(launch_denoise_features_rows<double>(accum_dev, var_dev, feat, W, H, y0, y1, d->radius, d->patch_radius, d->k,
+                                                image_dev, S(stream)));
+    else
+        CU(launch_denoise_features_rows<float>(accum_dev, var_dev, feat, W, H, y0, y1, d->radius, d->patch_radius, d->k,
+                                               image_dev, S(stream)));
+    return RT_OK;
+}
+
+RT_EXPORT int rt_denoise_halo(int32_t radius, int32_t patch_radius, int32_t features, int32_t *rows) {
+    if (!rows) return fail(RT_ERR_INVALID, "NULL argument");
+    if (radius < 0 || radius > 15) return fail(RT_ERR_INVALID, "radius must be in [0, 15]");
+    if (patch_radius < 0 || patch_radius > 5) return fail(RT_ERR_INVALID, "patch_radius must be in [0, 5]");
+    *rows = denoise_halo(radius, patch_radius, features != 0);
     return RT_OK;
 }
 

@@ -39,23 +39,43 @@ static size_t denoise_smem(int r, int f, bool features) {
     return (6 * L * L + R * R + R * kTile + (features ? 10 * LF * LF : 0)) * sizeof(float);
 }
 
-// The filter of one CTA; kFeatures: with the feature term.  Two kernels below call it, so that the colour-only one keeps
-// its parameter block.  tid = threadIdx.x, read in the kernel, where its range (__launch_bounds__) is known.
-template <typename T, bool kFeatures>
+// kBand (rt_denoise_rows, DESIGN §4.8e): the output rows [y0, y1) of the frame; every row the filter reads is clamped
+// into the window [lo, hi) = [max(0, y0 - h), min(H, y1 + h)) instead of [0, H).  For an output row in [y0, y1) every
+// read lies in [y0 - h, y1 + h), where both clamps give the same row, so the band equals those rows of the whole frame.
+struct DenoiseRows {
+    int y0, y1, lo, hi;
+};
+// the frame row of the tile's first row, the first and last rows a read is clamped into, the end of the rows stored;
+// without kBand, exactly the whole-frame kernels' expressions, so that their code does not change
+template <bool kBand>
+RT_DEV unsigned tile_row(const DenoiseRows &band) { return kBand ? band.y0 + blockIdx.y * kTile : blockIdx.y * kTile; }
+template <bool kBand>
+RT_DEV int first_row(const DenoiseRows &band) { return kBand ? band.lo : 0; }
+template <bool kBand>
+RT_DEV int last_row(int H, const DenoiseRows &band) { return kBand ? band.hi - 1 : H - 1; }
+template <bool kBand>
+RT_DEV int end_row(int H, const DenoiseRows &band) { return kBand ? band.y1 : H; }
+
+// The filter of one CTA; kFeatures: with the feature term; kBand: of a row band.  Four kernels below call it, so that
+// the whole-frame ones keep their parameter blocks.  tid = threadIdx.x, read in the kernel, where its range
+// (__launch_bounds__) is known.
+template <typename T, bool kFeatures, bool kBand>
 RT_DEV void denoise_nlm(const typename M<T>::v4 *__restrict__ accum, const float *__restrict__ var, int W, int H, int r,
-                        int f, float k2, float *__restrict__ image, const DenoiseFeatures &feat, const int tid) {
+                        int f, float k2, float *__restrict__ image, const DenoiseFeatures &feat, const DenoiseRows &band,
+                        const int tid) {
     extern __shared__ float smem[];
     const int L = kTile + 2 * (r + f), LL = L * L, R = kTile + 2 * f, RR = R * R;
     float *su = smem, *sv = smem + 3 * LL;      // su[c * LL + i], sv[c * LL + i]
     float *sd = sv + 3 * LL, *sr = sd + RR;
-    const int x0 = blockIdx.x * kTile - (r + f), y0 = blockIdx.y * kTile - (r + f);
+    const int x0 = blockIdx.x * kTile - (r + f), y0 = tile_row<kBand>(band) - (r + f);
     // kFeatures: sf[j * LFF + i], planes 0-2 albedo, 3-5 normal, 6 depth, 7-9 the variances of albedo, normal, depth
     const int LF = kTile + 2 * r, LFF = LF * LF;
     float *sf = sr + R * kTile;
     if constexpr (kFeatures) {
-        const int fx0 = blockIdx.x * kTile - r, fy0 = blockIdx.y * kTile - r;
+        const int fx0 = blockIdx.x * kTile - r, fy0 = tile_row<kBand>(band) - r;
         for (int i = tid; i < LFF; i += kThreads) {
-            const int x = min(max(fx0 + i % LF, 0), W - 1), y = min(max(fy0 + i / LF, 0), H - 1);
+            const int x = min(max(fx0 + i % LF, 0), W - 1);
+            const int y = min(max(fy0 + i / LF, first_row<kBand>(band)), last_row<kBand>(H, band));
             const size_t o = (size_t)y * W + x;
 #pragma unroll
             for (int c = 0; c < 3; ++c) {
@@ -69,7 +89,8 @@ RT_DEV void denoise_nlm(const typename M<T>::v4 *__restrict__ accum, const float
 
     // halo, with clamped reads: entry (i, j) holds pixel (clamp(x0 + j), clamp(y0 + i))
     for (int i = tid; i < LL; i += kThreads) {
-        const int x = min(max(x0 + i % L, 0), W - 1), y = min(max(y0 + i / L, 0), H - 1);
+        const int x = min(max(x0 + i % L, 0), W - 1);
+        const int y = min(max(y0 + i / L, first_row<kBand>(band)), last_row<kBand>(H, band));
         const size_t o = (size_t)y * W + x;
         const typename M<T>::v4 a = accum[o];
         RT_ASSERT(a.w >= 1);
@@ -117,9 +138,10 @@ RT_DEV void denoise_nlm(const typename M<T>::v4 *__restrict__ accum, const float
         for (int c = 0; c < 7; ++c) fp[c] = sf[c * LFF + hcf];
 #pragma unroll
         for (int j = 0; j < 3; ++j) vfp[j] = sf[(7 + j) * LFF + hcf];
-        const int xc = min(blockIdx.x * kTile + px, W - 1), yc = min(blockIdx.y * kTile + py, H - 1);
+        const int xc = min(blockIdx.x * kTile + px, W - 1), yc = min(tile_row<kBand>(band) + py, last_row<kBand>(H, band));
         const size_t oxm = (size_t)yc * W + max(xc - 1, 0), oxp = (size_t)yc * W + min(xc + 1, W - 1);
-        const size_t oym = (size_t)max(yc - 1, 0) * W + xc, oyp = (size_t)min(yc + 1, H - 1) * W + xc;
+        const size_t oym = (size_t)max(yc - 1, first_row<kBand>(band)) * W + xc;
+        const size_t oyp = (size_t)min(yc + 1, last_row<kBand>(H, band)) * W + xc;
         float g[3] = {0.f, 0.f, 0.f};
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
@@ -195,8 +217,8 @@ RT_DEV void denoise_nlm(const typename M<T>::v4 *__restrict__ accum, const float
         }
     }
 
-    const int x = blockIdx.x * kTile + px, y = blockIdx.y * kTile + py;
-    if (x >= W || y >= H) return;
+    const int x = blockIdx.x * kTile + px, y = tile_row<kBand>(band) + py;
+    if (x >= W || y >= end_row<kBand>(H, band)) return;
     // o = 0 has weight 1, so sw >= 1; the lattice is rt_resolve's: min(1, floor(value) / 255) rounded from double
     const float vals[3] = {uc0 + s0 / sw, uc1 + s1 / sw, uc2 + s2 / sw};
     const size_t o = (size_t)y * W + x;
@@ -211,7 +233,7 @@ template <typename T>
 __global__ void __launch_bounds__(kThreads) denoise_nlm_kernel(const typename M<T>::v4 *__restrict__ accum,
                                                                const float *__restrict__ var, int W, int H, int r, int f,
                                                                float k2, float *__restrict__ image) {
-    denoise_nlm<T, false>(accum, var, W, H, r, f, k2, image, DenoiseFeatures{}, threadIdx.x);
+    denoise_nlm<T, false, false>(accum, var, W, H, r, f, k2, image, DenoiseFeatures{}, DenoiseRows{}, threadIdx.x);
 }
 
 template <typename T>
@@ -219,18 +241,36 @@ __global__ void __launch_bounds__(kThreads) denoise_nlm_features_kernel(const ty
                                                                         const float *__restrict__ var, int W, int H, int r,
                                                                         int f, float k2, float *__restrict__ image,
                                                                         const __grid_constant__ DenoiseFeatures feat) {
-    denoise_nlm<T, true>(accum, var, W, H, r, f, k2, image, feat, threadIdx.x);
+    denoise_nlm<T, true, false>(accum, var, W, H, r, f, k2, image, feat, DenoiseRows{}, threadIdx.x);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kThreads) denoise_nlm_rows_kernel(const typename M<T>::v4 *__restrict__ accum,
+                                                                    const float *__restrict__ var, int W, int H, int r,
+                                                                    int f, float k2, float *__restrict__ image,
+                                                                    const DenoiseRows band) {
+    denoise_nlm<T, false, true>(accum, var, W, H, r, f, k2, image, DenoiseFeatures{}, band, threadIdx.x);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kThreads) denoise_nlm_features_rows_kernel(const typename M<T>::v4 *__restrict__ accum,
+                                                                             const float *__restrict__ var, int W, int H,
+                                                                             int r, int f, float k2,
+                                                                             float *__restrict__ image,
+                                                                             const __grid_constant__ DenoiseFeatures feat,
+                                                                             const DenoiseRows band) {
+    denoise_nlm<T, true, true>(accum, var, W, H, r, f, k2, image, feat, band, threadIdx.x);
 }
 
 template <typename K, typename... A>
-static cudaError_t launch_nlm(K kernel, bool features, int W, int H, int r, int f, cudaStream_t st, const A &...args) {
+static cudaError_t launch_nlm(K kernel, bool features, int W, int rows, int r, int f, cudaStream_t st, const A &...args) {
     if (r < 0 || r > kMaxR || f < 0 || f > kMaxF) return cudaErrorInvalidValue;
     const size_t smem = denoise_smem(r, f, features);
     if (smem > 48 * 1024) {
         const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    const dim3 grid((unsigned)((W + kTile - 1) / kTile), (unsigned)((H + kTile - 1) / kTile));
+    const dim3 grid((unsigned)((W + kTile - 1) / kTile), (unsigned)((rows + kTile - 1) / kTile));
     kernel<<<grid, kThreads, smem, st>>>(args...);
     return cudaGetLastError();
 }
@@ -249,11 +289,39 @@ cudaError_t launch_denoise_features(const void *accum, const float *var, const D
                       r, f, square_to_float(k), image, feat);
 }
 
+// the band [y0, y1) and its window: 0 <= y0 < y1 <= H is the caller's to check (rt_api.cu)
+static DenoiseRows band_rows(int H, int y0, int y1, int r, int f, bool features) {
+    const int h = denoise_halo(r, f, features);
+    return DenoiseRows{y0, y1, max(0, y0 - h), min(H, y1 + h)};
+}
+
+template <typename T>
+cudaError_t launch_denoise_rows(const void *accum, const float *var, int W, int H, int y0, int y1, int r, int f, float k,
+                                float *image, cudaStream_t st) {
+    return launch_nlm(denoise_nlm_rows_kernel<T>, false, W, y1 - y0, r, f, st, (const typename M<T>::v4 *)accum, var, W,
+                      H, r, f, square_to_float(k), image, band_rows(H, y0, y1, r, f, false));
+}
+
+template <typename T>
+cudaError_t launch_denoise_features_rows(const void *accum, const float *var, const DenoiseFeatures &feat, int W, int H,
+                                         int y0, int y1, int r, int f, float k, float *image, cudaStream_t st) {
+    return launch_nlm(denoise_nlm_features_rows_kernel<T>, true, W, y1 - y0, r, f, st, (const typename M<T>::v4 *)accum,
+                      var, W, H, r, f, square_to_float(k), image, feat, band_rows(H, y0, y1, r, f, true));
+}
+
 template cudaError_t launch_denoise<float>(const void *, const float *, int, int, int, int, float, float *, cudaStream_t);
 template cudaError_t launch_denoise<double>(const void *, const float *, int, int, int, int, float, float *, cudaStream_t);
 template cudaError_t launch_denoise_features<float>(const void *, const float *, const DenoiseFeatures &, int, int, int, int,
                                                     float, float *, cudaStream_t);
 template cudaError_t launch_denoise_features<double>(const void *, const float *, const DenoiseFeatures &, int, int, int,
                                                      int, float, float *, cudaStream_t);
+template cudaError_t launch_denoise_rows<float>(const void *, const float *, int, int, int, int, int, int, float, float *,
+                                                cudaStream_t);
+template cudaError_t launch_denoise_rows<double>(const void *, const float *, int, int, int, int, int, int, float, float *,
+                                                 cudaStream_t);
+template cudaError_t launch_denoise_features_rows<float>(const void *, const float *, const DenoiseFeatures &, int, int, int,
+                                                         int, int, int, float, float *, cudaStream_t);
+template cudaError_t launch_denoise_features_rows<double>(const void *, const float *, const DenoiseFeatures &, int, int,
+                                                          int, int, int, int, float, float *, cudaStream_t);
 
 }  // namespace rt

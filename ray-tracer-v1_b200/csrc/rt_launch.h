@@ -244,6 +244,19 @@ inline float square_to_float(float k) {
 template <typename T>
 cudaError_t launch_denoise_features(const void *accum, const float *var, const DenoiseFeatures &feat, int W, int H, int r,
                                     int f, float k, float *image, cudaStream_t st);
+// halo depth of the filters (rt_denoise_halo): an output row reads rows within r + f of its own; the feature gradient
+// reads y +- 1 whatever r and f are
+inline int denoise_halo(int r, int f, bool features) {
+    return features && r + f < 1 ? 1 : r + f;
+}
+// the same filters for the output rows [y0, y1) of the frame only (rt_denoise_rows, rt_denoise_features_rows): buffers
+// stay [H,W,.]; the kernels read rows [max(0, y0 - h), min(H, y1 + h)) and write rows [y0, y1), 0 <= y0 < y1 <= H
+template <typename T>
+cudaError_t launch_denoise_rows(const void *accum, const float *var, int W, int H, int y0, int y1, int r, int f, float k,
+                                float *image, cudaStream_t st);
+template <typename T>
+cudaError_t launch_denoise_features_rows(const void *accum, const float *var, const DenoiseFeatures &feat, int W, int H,
+                                         int y0, int y1, int r, int f, float k, float *image, cudaStream_t st);
 
 // FFMA issue-rate micro-benchmark (rt_f32.cu): `iters` trips of 16 independent FFMA per thread
 cudaError_t launch_fp32_peak(int blocks, int threads, int iters, float *sink, cudaStream_t st);

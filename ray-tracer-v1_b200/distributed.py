@@ -11,6 +11,11 @@ The path shards three ways (SURVEY.md section 8e); each needs at most ONE collec
               2^53: exact), so the variance image is bit-identical too.
 * env      -- environment slices (C5): no collective at all, see ray_tracer_env.BatchedRayTracerEnv.shard.
 
+A denoised frame (``render(..., denoise=True)``, DESIGN §4.8e) is filtered in the same row bands: every rank forms the
+final sums of its band (``reduce_row_bands`` in samples mode), receives the ``h`` rows of its neighbours' sums and
+variance its filter reads (``halo_plan`` / ``exchange_halos``, one batched point-to-point exchange) and filters its band
+with ``rt_denoise_rows``, which reads no row outside that window; rank 0 gathers the bands.
+
 Because the Philox stream is keyed by the GLOBAL (pixel, sample, bounce), a sharded frame equals the unsharded frame
 bit for bit for any world size.  The partition/collective helpers take the band renderer as a callable so the
 world_size-2 ``gloo`` tests on CPU exercise exactly this code with a stand-in renderer.
@@ -18,7 +23,7 @@ world_size-2 ``gloo`` tests on CPU exercise exactly this code with a stand-in re
 import numpy as np
 
 __all__ = ["row_bands", "sample_ranges", "env_slices", "tile_stripes", "gather_row_bands", "reduce_sample_sums",
-           "PeerFabric", "ShardedPathRenderer"]
+           "halo_windows", "halo_plan", "exchange_halos", "reduce_row_bands", "PeerFabric", "ShardedPathRenderer"]
 
 
 def _split(total, world):
@@ -103,6 +108,61 @@ def reduce_sample_sums(accum, group=None, dst=0):
     dst_global = dist.get_global_rank(group, dst) if group is not None else dst
     dist.reduce(accum, dst=dst_global, op=dist.ReduceOp.SUM, group=group)
     return accum
+
+
+def halo_windows(height, world, halo):
+    """Each rank's window [y_lo, y_hi) = [max(0, y0 - halo), min(H, y1 + halo)) around its band [y0, y1) of
+    ``row_bands``: the rows a stencil of depth ``halo`` reads to compute the band.  An empty band has an empty window."""
+    H, h = int(height), int(halo)
+    return [(a, a) if a == b else (max(0, a - h), min(H, b + h)) for a, b in row_bands(H, world)]
+
+
+def halo_plan(height, world, halo):
+    """The row copies that give every rank the rows of its ``halo_windows`` window it does not own: a list of
+    (src, dst, a, b), rank ``src`` sends rows [a, b) of its band to rank ``dst``.  Every such row is covered exactly
+    once, from the rank whose band holds it, so a halo deeper than a neighbour's band takes rows from several ranks."""
+    bands = row_bands(height, world)
+    plan = []
+    for dst, (lo, hi) in enumerate(halo_windows(height, world, halo)):
+        for src, (a, b) in enumerate(bands):
+            a, b = max(a, lo), min(b, hi)
+            if src != dst and a < b:
+                plan.append((src, dst, a, b))
+    return plan
+
+
+def exchange_halos(tensors, plan, group=None):
+    """Carry out ``halo_plan`` for every [H, ...] tensor of ``tensors`` (each rank's own band already final), with one
+    batched point-to-point exchange (``batch_isend_irecv``).  Row slices of a contiguous tensor are contiguous, so the
+    rows are sent from and received into the tensors themselves."""
+    dist = _dist()
+    rank, world = _world(group)
+    glob = (lambda r: dist.get_global_rank(group, r)) if group is not None else (lambda r: r)
+    ops = []
+    for src, dst, a, b in plan:
+        if rank == src:
+            ops += [dist.P2POp(dist.isend, t[a:b], glob(dst), group) for t in tensors]
+        elif rank == dst:
+            ops += [dist.P2POp(dist.irecv, t[a:b], glob(src), group) for t in tensors]
+    if world > 1 and ops:
+        for req in dist.batch_isend_irecv(ops):
+            req.wait()
+    return tensors
+
+
+def reduce_row_bands(t, bands, group=None):
+    """Sum the per-rank [H, ...] tensors ``t`` so that each rank holds the final sums of its own band ``bands[rank]``:
+    one in-place reduce per non-empty band, sent to the band's owner.  The bands do not overlap, so every row is reduced
+    once (in all, the traffic of a reduce-scatter); rows outside a rank's own band are left undefined."""
+    dist = _dist()
+    rank, world = _world(group)
+    if world == 1:
+        return t
+    for owner, (a, b) in enumerate(bands):
+        if a < b:
+            dst = dist.get_global_rank(group, owner) if group is not None else owner
+            dist.reduce(t[a:b], dst=dst, op=dist.ReduceOp.SUM, group=group)
+    return t
 
 
 class _DevArray:
@@ -274,6 +334,16 @@ class ShardedPathRenderer:
             self._var_key = (W, H)
         self._ensure_host_vars(W, H)
 
+    def _ensure_features(self, W, H):
+        """First-hit feature buffers (albedo [H,W,3], normal [H,W,3], depth [H,W], fvar [H,W,3] float32), allocated by
+        the first feature frame."""
+        torch = self.torch
+        if getattr(self, "_feat_key", None) != (W, H):
+            dev = torch.device("cuda", self.device)
+            self.features = tuple(torch.zeros(s, dtype=torch.float32, device=dev)
+                                  for s in ((H, W, 3), (H, W, 3), (H, W), (H, W, 3)))
+            self._feat_key = (W, H)
+
     def _to_host(self, src, slot, release=None, var=None):
         """Queue the device->host copy of ``src`` (and of the variance image ``var``, if given) on the copy stream (after
         everything the current stream has queued) into pinned slot ``slot``; ``release`` (optional) runs on the copy
@@ -307,7 +377,7 @@ class ShardedPathRenderer:
         return pi.result(), (None if pv is None else pv.result())
 
     def render(self, cam, W, H, spp, max_bounces, mirror_threshold, seed=0, fov=60.0, mode="tiles", to_host=False,
-               variance=False):
+               variance=False, denoise=False, features=False, denoise_params=None):
         """Render one frame cooperatively.  Returns (image, stats) on rank 0 -- image a CUDA tensor [H,W,3] float32, a
         numpy view of pinned host memory when ``to_host`` is True, or a ``PendingFrame`` when ``to_host == "async"``
         (the copy runs on a second stream while the next frame renders) -- and (None, stats) elsewhere.  stats = this
@@ -316,16 +386,33 @@ class ShardedPathRenderer:
         ``variance=True`` (the same on every rank of a frame): also the variance of each pixel's mean in colour
         levels^2, [H,W,3] float32, bit-identical to ``render_path(..., variance=True)`` of the unsharded frame.  The
         call then returns (image, stats, var) on rank 0, var of the same kind as image, and (None, stats, None)
-        elsewhere."""
+        elsewhere.
+
+        ``denoise=True`` (DESIGN §4.8e): the image is the frame filtered by the variance-guided non-local-means filter,
+        bit-identical to ``FrameContext.render_path(..., denoise=True)``.  Every rank forms the final sums of its row
+        band (samples mode: ``reduce_row_bands`` of the sums and moments in place of the reduce to rank 0), resolves
+        its band's variance, exchanges the halo rows of both with its neighbours and filters its band
+        (``DeviceScene.denoise(rows=)``); rank 0 gathers the bands.  ``features=True`` (needs ``denoise``): the
+        feature-guided filter, each rank rendering the first-hit features of its window rows over the samples
+        [0, min(spp, FrameContext.FEATURE_SPP)).  ``denoise_params``: a dict of ``DeviceScene.denoise``'s keywords
+        (radius, patch_radius, k, k_f, tau); None: the library defaults.  The return shape does not change."""
         torch, nat, sc = self.torch, self.nat, self.scene
+        if features and not denoise:
+            raise ValueError("features=True needs denoise=True: the sharded renderer does not gather the feature buffers")
+        dparams = dict(denoise_params or {})
+        if denoise:
+            # the halo depth, from the library; also rejects a bad radius / patch_radius before any collective
+            halo = nat.denoise_halo(features=features, **{k: dparams[k] for k in ("radius", "patch_radius") if k in dparams})
         self._ensure(W, H)
-        if variance:
+        if variance or denoise:
             self._ensure_variance(W, H)
+        if features:
+            self._ensure_features(W, H)
         self._frame += 1
         slot = self._frame & 1
         self.image = self.images[slot]
-        var = self.vars[slot] if variance else None
-        moments = self.moments if variance else None
+        var = self.vars[slot] if (variance or denoise) else None
+        moments = self.moments if (variance or denoise) else None
         torch.cuda.current_stream().wait_event(self._copied[slot])         # slot's previous copy-out has finished
         rows = (0, H)
         samples = (0, spp)
@@ -339,12 +426,19 @@ class ShardedPathRenderer:
         self.stats.zero_()
         if mode == "samples" and samples[0] == samples[1]:
             self.accum.zero_()
-            if variance:
+            if moments is not None:
                 moments.zero_()
         p = sc.path_params(cam, W, H, spp, max_bounces, mirror_threshold, seed=seed, fov=fov, rows=rows, samples=samples)
         sc.render_path(p, self.accum, self.precision, stats=self.stats, moments=moments)
         self.launches = 1
-        if mode == "tiles":
+        if denoise:
+            self._denoise_bands(cam, W, H, spp, seed, fov, mode, var, halo, features, dparams)
+            gather_row_bands(self.image, row_bands(H, self.world), self.group)
+            if variance:
+                gather_row_bands(var, row_bands(H, self.world), self.group)
+            else:
+                var = None
+        elif mode == "tiles":
             sc.resolve(self.accum, W, H, spp, self.image, self.precision, rows=rows)
             self.launches += 1
             if variance:
@@ -367,6 +461,32 @@ class ShardedPathRenderer:
             return (None, self.stats, None) if variance else (None, self.stats)
         image, var = self._deliver(self.image, var, slot, to_host)
         return (image, self.stats, var) if variance else (image, self.stats)
+
+    def _denoise_bands(self, cam, W, H, spp, seed, fov, mode, var, halo, features, dparams):
+        """The denoised frame's steps after the render: this rank's band sums and variance, the halo exchange, its
+        window's features and the band filter into ``self.image``."""
+        sc, prec = self.scene, self.precision
+        bands = row_bands(H, self.world)
+        y0, y1 = bands[self.rank]
+        if mode == "samples":
+            reduce_row_bands(self.accum, bands, self.group)
+            reduce_row_bands(self.moments, bands, self.group)
+        if y1 > y0:
+            sc.resolve_variance(self.accum, self.moments, W, H, var, prec, rows=(y0, y1))
+            self.launches += 1
+        exchange_halos([self.accum, var], halo_plan(H, self.world, halo), self.group)
+        lo, hi = halo_windows(H, self.world, halo)[self.rank]
+        if features and hi > lo:
+            # the feature kernel is per pixel: rendering the window rows here equals exchanging them
+            from .frames import FrameContext
+            p = sc.path_params(cam, W, H, spp, 1, 0.0, seed=seed, fov=fov, rows=(lo, hi),
+                               samples=(0, min(int(spp), FrameContext.FEATURE_SPP)))
+            sc.render_features(p, *self.features, precision=prec)
+            self.launches += 1
+        if y1 > y0:
+            sc.denoise(self.accum, var, W, H, self.image, prec, rows=(y0, y1),
+                       features=self.features if features else None, **dparams)
+            self.launches += 1
 
     # ---- fused sinks over NVLink peer memory ------------------------------------------------------------------
     def _ensure_fabric(self, W, H):
